@@ -1,6 +1,6 @@
 """bench.py -- clouds/sec of the Point-DAE geometry chain on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic ShapeNet-shaped clouds
 (headline shape B=128 clouds per GPU, N=2048 points, G=64 groups, M=32 neighbours):
@@ -34,7 +34,6 @@ POOL = 48                        # distinct resident batches cycled through: 48 
 METRIC = "clouds/sec (FPS+Group+Chamfer fwd/bwd, B=128 N=2048)"
 UNIT = "clouds/s"
 REF_BUDGET_S = 170.0             # wall-clock budget of the CPU reference arm (it does ~50 clouds/s on 16 cores)
-MIN_TIMED_MS = 60.0              # the timed region is repeated until it is at least this long
 
 
 def workload_name():
@@ -413,12 +412,13 @@ def run_ours(args):
             graphs.append((g, out))
 
     def run_step(i):
+        """one step of the timed path; returns its outputs (StepBuffers, or the (loss, neighborhood, gpred) tuple)"""
         if step_bufs is not None:
-            ops.hot_step(clouds_d[i % POOL], preds_d[i % POOL], G, M, gone, buffers=step_bufs[i % 2])
-        elif graphs:
+            return ops.hot_step(clouds_d[i % POOL], preds_d[i % POOL], G, M, gone, buffers=step_bufs[i % 2])
+        if graphs:
             graphs[i % POOL][0].replay()
-        else:
-            step_device(i)
+            return graphs[i % POOL][1]
+        return step_device(i)
 
     grouper = group.Group(G, M)
     cd_l2 = chamfer_dist.ChamferDistanceL2()
@@ -528,32 +528,25 @@ def run_ours(args):
         return float(t.item())
 
     # ---- device-resident timing ----------------------------------------------------------------------
-    for i in range(max(args.warmup, 100)):  # at least 100 untimed steps (~30 ms) so clocks are at their loaded state
-        run_step(i)
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
         time.sleep(0.3)
-    # K steps are ~5 ms at the driver's --steps 20: the K-step region is repeated back to back until the timed region is
-    # at least MIN_TIMED_MS long (same count on every rank), and ms_per_step is the mean over all timed steps
+    # at least 100 untimed steps (~15 ms) right before the timed ones, so clocks are at their loaded state when timing starts
+    for i in range(max(args.warmup, 100)):
+        run_step(i)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    # exactly --steps timed steps; ms_per_step is their mean
     barrier()
     e0.record(stream)
     for i in range(args.steps):
-        run_step(args.warmup + i)
+        outputs = run_step(args.warmup + i)
     e1.record(stream)
     barrier()
-    probe_ms = max_over_ranks(e0.elapsed_time(e1))
-    inner = max(1, int(MIN_TIMED_MS / max(probe_ms, 1e-3)) + 1)
-    barrier()
-    e0.record(stream)
-    for rep in range(inner):
-        for i in range(args.steps):
-            run_step(args.warmup + rep * args.steps + i)
-    e1.record(stream)
-    barrier()
+    if args.dump_outputs and rank == 0:  # before any later call reuses the step's buffers
+        dump_outputs(args.dump_outputs, outputs)
     total_ms = max_over_ranks(e0.elapsed_time(e1))
-    ms_per_step = total_ms / (args.steps * inner)
+    ms_per_step = total_ms / args.steps
     value = world * B / (ms_per_step * 1e-3)
     # dominant kernel, timed live with CUDA events on its launching stream: the Chamfer forward alone (no co-running
     # branch), once per timed step over the same rotating pool.  Launched from Python each forward is three kernels
@@ -617,9 +610,9 @@ def run_ours(args):
     t0 = time.perf_counter()
     e0.record(stream)
     e2e_first = max(args.warmup, 100)
-    e2e_steps = args.steps * inner
-    for i in range(e2e_steps):
-        step_e2e(e2e_first + i, first=(i == 0))
+    e2e_steps = args.steps
+    for i in range(e2e_steps):  # the warm-up left the next batch prefetched: the timed steps continue its pipeline
+        step_e2e(e2e_first + i, first=False)
     e1.record(stream)
     barrier()
     e2e_ms = max_over_ranks(max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3)) / e2e_steps
@@ -667,7 +660,7 @@ def run_ours(args):
         t0 = time.perf_counter()
         e0.record(stream)
         for i in range(e2e_steps):
-            step_e2e_native(e2e_first + i, first=(i == 0))
+            step_e2e_native(e2e_first + i, first=False)
         e1.record(stream)
         barrier()
         e2e_native_ms = max_over_ranks(max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3)) / e2e_steps
@@ -802,9 +795,7 @@ def run_ours(args):
                 "overlap": ": FPS+Group || Chamfer forward -> (loss || backward)"}[args.patchifier] + (
                 "; kNN gated behind the Chamfer scan" if args.knn_gate == "scan" else "") + (
                 "; FPS+Group = one launch (FPS warps + kNN consumer warps per cloud)" if fused_patchifier else ""),
-            "timed_steps": args.steps * inner, "timed_region_ms": total_ms,
-            "timed_region_note": "the K-step region repeated %d times back to back (>= %.0f ms); ms_per_step = mean over "
-                                 "all timed steps" % (inner, MIN_TIMED_MS),
+            "timed_steps": args.steps, "timed_region_ms": total_ms,
             "e2e": {"value": world * B / ((e2e_native_ms or e2e_ms) * 1e-3), "unit": UNIT,
                     "h2d_bytes_per_step": (2 if args.e2e_upload == "both" else 1) * B * N * 12,
                     "h2d_only_ms_per_step": h2d_only_ms,
@@ -824,7 +815,7 @@ def run_ours(args):
                            "copies the next batch from pinned host memory and the loss back to the host (a training step: "
                            "patches and gradients stay on the device)" + (
                                "" if args.no_graphs else "; the step is replayed as a CUDA graph")},
-            "gpu_launches": launches_per_step * args.steps * inner,
+            "gpu_launches": launches_per_step * args.steps,
             "roofline": roofline,
             "other_kernels": others,
             "configs": configs,
@@ -1170,6 +1161,24 @@ def other_kernels(dev, clouds_d, preds_d, peaks, props):
     return out
 
 
+STEP_OUTPUTS = ("neighborhood", "center", "fps_idx", "dist1", "dist2", "idx1", "idx2", "loss3", "gpred", "gcloud")
+
+
+def dump_outputs(out_dir, out):
+    """Writes the outputs of one timed step as out_dir/<name>.npy so that two builds can be compared array for array:
+    the StepBuffers of the native step call, or (loss, neighborhood, gpred) of the graph / eager arms.  Floating
+    arrays are stored as float32, index arrays as float64 (exact).  At the headline shape this is about 16 MB."""
+    import numpy as np
+    if isinstance(out, tuple):
+        arrays = dict(zip(("loss", "neighborhood", "gpred"), out))
+    else:
+        arrays = {name: getattr(out, name) for name in STEP_OUTPUTS}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -1216,7 +1225,14 @@ def main():
                     help="what the end-to-end arm copies from pinned host memory every step: the cloud (default; the "
                          "prediction is produced on the device by the model) or cloud + prediction")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config (C2..C5) and sharded-C5 evidence blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0; the inputs "
+                         "depend only on the arguments, so two builds run with the same arguments can be compared)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (the CPU reference arm sizes its batch by wall-clock time)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

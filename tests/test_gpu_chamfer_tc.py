@@ -1,8 +1,9 @@
 """Chamfer forward through the tensor-core filter (csrc/chamfer_tc.cu) -- the default for clouds of 512..2048 points --
-against the CPU oracle (extensions/chamfer_dist/chamfer.cu:15-145 restated), the reference's own CUDA kernel rebuilt for
-sm_100a, and the FP32-pipe kernels of csrc/chamfer.cu.  Bar: dist and idx bit-exact, for every input: the filter only
+against the CPU oracle (extensions/chamfer_dist/chamfer.cu:15-145 restated), stored outputs of the reference's own CUDA
+kernel, and the FP32-pipe kernels of csrc/chamfer.cu.  Bar: dist and idx bit-exact, for every input: the filter only
 decides which 32-column groups are evaluated exactly, never the result."""
 import ctypes
+import os
 
 import numpy as np
 import pytest
@@ -10,10 +11,10 @@ import torch
 
 from oracle import cpu as oracle
 from pointdae_b200 import _native, chamfer_dist, ops, synth
-import _refmods
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
+CHAMFER_GOLD = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "chamfer.npz"))
 
 
 def cu(a):
@@ -152,21 +153,17 @@ def test_reference_set_sharded_share_through_the_tensor_cores(tc_mode, mode, n, 
     assert torch.equal(sd, d1) and torch.equal(si, i1)
 
 
-@pytest.mark.parametrize("b,n,m", [(8, 1024, 1024), (128, 2048, 2048), (6, 2000, 1500)])
-def test_fp32_pipe_kernels_still_match_reference_cuda(tc_mode, b, n, m):
-    """the tensor-core path is the default for these shapes; the FP32-pipe kernels (every other shape, the sharded entry
-    points) stay pinned to the reference's kernel at the same shapes"""
-    ref = _refmods.ref_chamfer()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    a, c = clouds_pair("prediction", min(b, 8), n, m, seed=n)
-    x1, x2 = cu(np.tile(a, (-(-b // a.shape[0]), 1, 1))[:b]), cu(np.tile(c, (-(-b // c.shape[0]), 1, 1))[:b])
-    want = ref.forward(x1, x2)
+@pytest.mark.parametrize("case", sorted({k.split("/")[0] for k in CHAMFER_GOLD.files if "/" in k} - {"transposed"}))
+def test_fp32_pipe_kernels_still_match_reference_cuda(tc_mode, case):
+    """the FP32-pipe kernels (mode 0: every shape outside the tensor-core range, the sharded entry points) and both
+    tensor-core modes give what the reference's own chamfer.forward returned on a B200 (chamfer.npz), bit for bit"""
+    z = CHAMFER_GOLD
+    x1, x2 = cu(z[case + "/xyz1"]), cu(z[case + "/xyz2"])
     for mode in (0, 2, 3):
         tc_mode(mode)
         got = ops.chamfer_forward(x1, x2)
-        assert torch.equal(got[0], want[0]) and torch.equal(got[1], want[1]), mode
-        assert torch.equal(got[2], want[2]) and torch.equal(got[3], want[3]), mode
+        for g, key in zip(got, ("dist1", "dist2", "idx1", "idx2")):
+            np.testing.assert_array_equal(g.cpu().numpy(), z[case + "/" + key], err_msg="mode %d %s" % (mode, key))
 
 
 @pytest.mark.parametrize("mode", [2, 3])

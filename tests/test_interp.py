@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 import torch
 
+import _golden_sample
 import _interp_cases
 import _refmods
 from oracle import cpu as oracle
@@ -24,15 +25,14 @@ def _gold():
 def test_oracle_matches_reference_cuda(name):
     z = _gold()
     unknown, known = CASES[name]
-    assert np.array_equal(z[name + "/unknown"], unknown) and np.array_equal(z[name + "/known"], known)
     d2, idx = oracle.three_nn(unknown, known)
     np.testing.assert_array_equal(idx, z[name + "/idx"])
     np.testing.assert_array_equal(d2, z[name + "/dist2"])
     for c in (5, 16):
-        feats, weight, gout = (z["%s/c%d/%s" % (name, c, k)] for k in ("feats", "weight", "gout"))
-        np.testing.assert_array_equal(oracle.three_interpolate(feats, idx, weight), z["%s/c%d/out" % (name, c)])
-        want = z["%s/c%d/gfeats" % (name, c)]
-        got = oracle.three_interpolate_grad(gout, idx, weight, known.shape[1])
+        feats, weight, gout = _interp_cases.interp_inputs(synth, name, unknown, known, z[name + "/idx"], z[name + "/dist2"], c)
+        np.testing.assert_array_equal(*_golden_sample.expect(z, "%s/c%d/out" % (name, c), oracle.three_interpolate(feats, idx, weight)))
+        got, want = _golden_sample.expect(z, "%s/c%d/gfeats" % (name, c),
+                                          oracle.three_interpolate_grad(gout, idx, weight, known.shape[1]))
         np.testing.assert_allclose(got, want, rtol=1e-5, atol=1e-5 * np.abs(want).max())
 
 
@@ -61,14 +61,14 @@ def test_gpu_three_nn_interpolate_match_golden_and_oracle(name):
     dist, idx_b = pointnet2_utils.three_nn(u, k)  # public name: Euclidean distances
     np.testing.assert_array_equal(dist.cpu().numpy(), np.sqrt(z[name + "/dist2"]))
     for c in (5, 16):
-        feats, weight, gout = (z["%s/c%d/%s" % (name, c, kk)] for kk in ("feats", "weight", "gout"))
+        feats, weight, gout = _interp_cases.interp_inputs(synth, name, unknown, known, z[name + "/idx"], z[name + "/dist2"], c)
         f = torch.from_numpy(feats).to(dev).requires_grad_(True)
         w, g = torch.from_numpy(weight).to(dev), torch.from_numpy(gout).to(dev)
         out = pointnet2_utils.three_interpolate(f, idx, w)
-        np.testing.assert_array_equal(out.detach().cpu().numpy(), z["%s/c%d/out" % (name, c)])
+        np.testing.assert_array_equal(*_golden_sample.expect(z, "%s/c%d/out" % (name, c), out.detach().cpu().numpy()))
         out.backward(g)
-        want = z["%s/c%d/gfeats" % (name, c)]
-        np.testing.assert_allclose(f.grad.cpu().numpy(), want, rtol=1e-5, atol=1e-5 * np.abs(want).max())
+        got, want = _golden_sample.expect(z, "%s/c%d/gfeats" % (name, c), f.grad.cpu().numpy())
+        np.testing.assert_allclose(got, want, rtol=1e-5, atol=1e-5 * np.abs(want).max())
 
 
 @pytest.mark.gpu
