@@ -398,6 +398,67 @@ int pdae_edge_gather_extremum_f32(const float *p, const float *q, const int64_t 
                                   const float *shift, float slope, int b, int n, int k, int co, float *out,
                                   pdae_stream_t stream);
 
+/* ---- deterministic gradients -------------------------------------------------------------------------------------
+ * Twins of the scatter-add gradients whose result is a pure function of the inputs (independent of grid, batch
+ * composition, stream and concurrent load): every gradient element starts from its own term (+0 where the op has none)
+ * and adds the scattered contributions one by one in ascending order of the source slot's linear index within the
+ * cloud, each contribution formed by the same expression as the atomic form, with rounded fp32 products and adds.
+ * Each takes a workspace of its own *_workspace_bytes query, builds ordered reverse maps there and writes every
+ * target once; no float atomics, no allocation, no host synchronisation (capturable).  Same argument rules and
+ * outputs as the atomic forms.  Orders:
+ *   chamfer (both forms)  point i of cloud 1: g_i (a_i - b[idx1[i]]), then -v_j for every j of cloud 2 with
+ *                         idx2[j] == i, j ascending; cloud 2 symmetric
+ *   pair loss             the own term, then the matched rows' terms, source ascending
+ *   gather grad           source j ascending
+ *   group_points grad     source slot q * nsample + k ascending
+ *   three_interpolate     slot i * 3 + s ascending (terms rn(gout * weight))
+ *   graph feature grad    the centre term of row j (p ascending), then G[i][p][0:c] for every edge with
+ *                         idx[i][p] == j, slot i * k + p ascending                                                   */
+size_t pdae_chamfer_bwd_det_workspace_bytes(int b, int n, int m); /* both Chamfer forms */
+int pdae_chamfer_bwd_det_f32(const float *xyz1, const float *xyz2, const int *idx1, const int *idx2, const float *gd1,
+                             const float *gd2, int b, int n, int m, float *gx1, float *gx2, void *workspace,
+                             size_t workspace_bytes, pdae_stream_t stream);
+int pdae_chamfer_loss_bwd_det_f32(const float *xyz1, const float *xyz2, const int *idx1, const int *idx2, const float *dist1,
+                                  const float *dist2, const float *gloss, float w1, float w2, int b, int n, int m, int l1,
+                                  float *gx1, float *gx2, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_pair_loss_bwd_det_workspace_bytes(int bs, int n, int m);
+int pdae_pair_loss_bwd_det_f32(const float *a, const float *b, const int *idx1, const int *idx2, const float *gloss, float w1,
+                               float w2, int bs, int n, int m, int d, int metric, float *ga, float *gb, void *workspace,
+                               size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_gather_grad_det_workspace_bytes(int b, int n, int m);
+int pdae_gather_grad_det_f32(const float *gout, const int *idx, int b, int c, int n, int m, float *gfeat, void *workspace,
+                             size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_group_points_grad_det_workspace_bytes(int b, int n, int npoints, int nsample);
+int pdae_group_points_grad_det_f32(const float *gout, const int *idx, int b, int c, int n, int npoints, int nsample,
+                                   float *gpoints, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_three_interpolate_grad_det_workspace_bytes(int b, int n, int m);
+int pdae_three_interpolate_grad_det_f32(const float *gout, const int *idx, const float *weight, int b, int c, int n, int m,
+                                        float *gpoints, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_graph_feature_grad_det_workspace_bytes(int b, int c, int n, int k);
+int pdae_graph_feature_grad_det_f32(const float *gout, const int64_t *idx, int b, int c, int n, int k, float *gx,
+                                    void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+
+/* The reverse index those gradients gather through, on its own: idx (b,s) int32 or int64 with targets in [0,t) ->
+ * ptr (b,t+1) bucket offsets within the cloud, slot (b,s) the source slots of each bucket in ascending order, i.e. a
+ * stable argsort of each cloud's targets.  Sources outside [0,t) are left out (ptr[t] counts the others; slot entries
+ * past it are not written).  Buckets are sorted by one thread up to 32 slots, by one CTA in shared memory up to 8192,
+ * by one CTA's ordered compaction of the cloud beyond.  Workspace: pdae_reverse_index_workspace_bytes.              */
+size_t pdae_reverse_index_workspace_bytes(int b, int s, int t);
+int pdae_reverse_index_i32(const int32_t *idx, int b, int s, int t, int *ptr, int *slot, void *workspace,
+                           size_t workspace_bytes, pdae_stream_t stream);
+int pdae_reverse_index_i64(const int64_t *idx, int b, int s, int t, int *ptr, int *slot, void *workspace,
+                           size_t workspace_bytes, pdae_stream_t stream);
+
+/* pdae_step_f32 with a flags word (pdae_step_f32 is this call with flags = 0).  PDAE_STEP_DETERMINISTIC: the backward on
+ * the side stream is pdae_chamfer_loss_bwd_det_f32; everything else is unchanged.  Workspace:
+ * pdae_step_ex_workspace_bytes with the same flags.                                                                  */
+#define PDAE_STEP_DETERMINISTIC 1u
+size_t pdae_step_ex_workspace_bytes(int b, int n, int g, int m, unsigned flags);
+int pdae_step_ex_f32(const float *cloud, const float *pred, int b, int n, int g, int m, int *fps_idx, float *center,
+                     float *neighborhood, float *dist1, float *dist2, int *idx1, int *idx2, float *loss3, const float *gloss,
+                     float *gpred, float *gcloud, void *workspace, size_t workspace_bytes, unsigned flags,
+                     pdae_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

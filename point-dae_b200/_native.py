@@ -89,6 +89,25 @@ SIGNATURES = {
     "pdae_affine_points_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pdae_group_affine_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "pdae_edge_gather_extremum_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _i, _i, _i, _i, _vp, _vp]),
+    "pdae_chamfer_bwd_det_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_chamfer_bwd_det_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_chamfer_loss_bwd_det_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _f, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_pair_loss_bwd_det_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_pair_loss_bwd_det_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_gather_grad_det_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_gather_grad_det_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "pdae_group_points_grad_det_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "pdae_group_points_grad_det_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "pdae_three_interpolate_grad_det_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_three_interpolate_grad_det_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "pdae_graph_feature_grad_det_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "pdae_graph_feature_grad_det_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "pdae_reverse_index_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_reverse_index_i32": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_reverse_index_i64": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_step_ex_workspace_bytes": (_sz, [_i, _i, _i, _i, ctypes.c_uint]),
+    "pdae_step_ex_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                              ctypes.c_uint, _vp]),
 }
 
 _lib = None

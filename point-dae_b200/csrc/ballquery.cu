@@ -9,6 +9,7 @@
 // serially; here a warp owns a query and scans 32 points per step (ballot + prefix popcount keep
 // the index order), so a 20 000-point scene uses the whole GPU and stops as soon as a ball is full.
 #include "common.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -118,4 +119,27 @@ extern "C" int pdae_group_points_grad_f32(const float *gout, const int *idx, int
                                                                        gpoints);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
+}
+
+// deterministic form: gpoints[b][l][p] = +0 (+) gout[b][l][j] over the slots j = q * nsample + k with idx == p, ascending
+extern "C" size_t pdae_group_points_grad_det_workspace_bytes(int b, int n, int npoints, int nsample) {
+  if (b <= 0 || n < 0 || npoints < 0 || nsample < 0) return 0;
+  const long long ps = static_cast<long long>(npoints) * nsample;
+  if (ps > 0x7fffffffLL) return 0;
+  return rev_map_bytes(b, static_cast<int>(ps), n);
+}
+
+extern "C" int pdae_group_points_grad_det_f32(const float *gout, const int *idx, int b, int c, int n, int npoints, int nsample,
+                                              float *gpoints, void *workspace, size_t workspace_bytes, pdae_stream_t stream) {
+  if (b < 0 || c < 0 || n < 0 || npoints < 0 || nsample < 0) return PDAE_E_INVALID;
+  const size_t gsz = static_cast<size_t>(b) * c * n;
+  if (gsz == 0) return 0;
+  const long long ps = static_cast<long long>(npoints) * nsample;
+  if (!gpoints || ps > 0x7fffffffLL || (ps && (!gout || !idx))) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_group_points_grad_det_workspace_bytes(b, n, npoints, nsample)) return PDAE_E_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  RevMap map;
+  const int rc = rev_map_build(idx, b, static_cast<int>(ps), n, workspace, &map, st);
+  if (rc) return rc;
+  return rev_gather_channel_major(gout, nullptr, b, c, static_cast<int>(ps), n, 1, map, gpoints, st);
 }

@@ -21,6 +21,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -471,6 +472,154 @@ static int launch_chamfer_bwd(const float *xyz1, const float *xyz2, const int *i
   return 0;
 }
 
+// ---- deterministic backward: the same terms gathered per point in a defined order, no float atomics ------------------
+// Point i of cloud 1 gets its own term g_i (a_i - b_idx1[i]), then -v_j for every point j of cloud 2 with idx2[j] == i,
+// j ascending, with rounded fp32 adds (cloud 2 symmetric).  rev1 lists, per point of cloud 1, the points of cloud 2
+// that chose it (the ordered reverse map of idx2), rev2 the converse.
+template <typename GradSrc>
+__global__ void __launch_bounds__(256) chamfer_bwd_det_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2,
+                                                              const int *__restrict__ idx1, const int *__restrict__ idx2,
+                                                              const GradSrc gs, int n, int m, int blocks_per_cloud, RevMap rev1,
+                                                              RevMap rev2, float *__restrict__ gx1, float *__restrict__ gx2) {
+  const unsigned cloud_u = blockIdx.x / blocks_per_cloud;
+  int i = (blockIdx.x - cloud_u * blocks_per_cloud) * blockDim.x + threadIdx.x;
+  const size_t cloud = cloud_u;
+  const bool second = i >= n;
+  const float *A, *Bp;
+  const int *idx, *rp, *rs;
+  float *ga;
+  size_t o, so;
+  if (!second) {
+    A = xyz1 + cloud * n * 3; Bp = xyz2 + cloud * m * 3; idx = idx1 + cloud * n; o = cloud * n + i;
+    ga = gx1 + cloud * n * 3; so = cloud * m;
+    rp = rev1.ptr + cloud * (n + 1); rs = rev1.slot + cloud * m;
+  } else {
+    i -= n;
+    if (i >= m) return;
+    A = xyz2 + cloud * m * 3; Bp = xyz1 + cloud * n * 3; idx = idx2 + cloud * m; o = cloud * m + i;
+    ga = gx2 + cloud * m * 3; so = cloud * n;
+    rp = rev2.ptr + cloud * (m + 1); rs = rev2.slot + cloud * n;
+  }
+  const int j2 = __ldg(idx + i);
+  const float g = __fmul_rn(gs.at(second, o), 2.0f);
+  float a[3], acc[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) a[c] = __ldg(A + 3 * i + c);
+#pragma unroll
+  for (int c = 0; c < 3; ++c) acc[c] = __fmul_rn(g, __fsub_rn(a[c], __ldg(Bp + 3 * j2 + c)));
+  // the sources live in the other cloud: their own points are Bp, their match (this point) is a
+  // buckets longer than REV_SHORT (up to a whole cloud for a collapsed prediction) are written by the warp walk below
+  const int lo = __ldg(rp + i), hi = __ldg(rp + i + 1);
+  if (hi - lo > REV_SHORT) return;
+  for (int q = lo; q < hi; ++q) {
+    const int j = __ldg(rs + q);
+    const float gj = __fmul_rn(gs.at(!second, so + j), 2.0f);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) acc[c] = __fadd_rn(acc[c], -__fmul_rn(gj, __fsub_rn(__ldg(Bp + 3 * j + c), a[c])));
+  }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) ga[3 * i + c] = acc[c];
+}
+
+// The long buckets (the maps' queues): one warp per target point.  The lanes load 32 sources at a time and form their terms
+// in parallel; every lane then adds the 32 terms in source order from the shuffles, so the sum is the one the point kernel
+// forms and a bucket of a whole cloud costs its serial adds, not a load latency per source.
+template <typename GradSrc>
+__global__ void __launch_bounds__(256) chamfer_bwd_det_long_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2,
+                                                                   const int *__restrict__ idx1, const int *__restrict__ idx2,
+                                                                   const GradSrc gs, int n, int m, RevMap rev1, RevMap rev2,
+                                                                   float *__restrict__ gx1, float *__restrict__ gx2) {
+  const int lane = threadIdx.x & 31;
+  const int n1 = __ldg(rev1.longq), n2 = __ldg(rev2.longq);
+  const int stride = static_cast<int>((gridDim.x * blockDim.x) >> 5);
+  for (int w = static_cast<int>((blockIdx.x * blockDim.x + threadIdx.x) >> 5); w < n1 + n2; w += stride) {
+    const bool second = w >= n1;
+    const int u = second ? __ldg(rev2.longq + 1 + (w - n1)) : __ldg(rev1.longq + 1 + w);
+    const int t = second ? m : n;
+    const size_t cloud = static_cast<size_t>(u / t);
+    const int i = u - static_cast<int>(cloud) * t;
+    const float *A, *Bp;
+    const int *idx, *rp, *rs;
+    float *ga;
+    size_t o, so;
+    if (!second) {
+      A = xyz1 + cloud * n * 3; Bp = xyz2 + cloud * m * 3; idx = idx1 + cloud * n; o = cloud * n + i;
+      ga = gx1 + cloud * n * 3; so = cloud * m;
+      rp = rev1.ptr + cloud * (n + 1); rs = rev1.slot + cloud * m;
+    } else {
+      A = xyz2 + cloud * m * 3; Bp = xyz1 + cloud * n * 3; idx = idx2 + cloud * m; o = cloud * m + i;
+      ga = gx2 + cloud * m * 3; so = cloud * n;
+      rp = rev2.ptr + cloud * (m + 1); rs = rev2.slot + cloud * n;
+    }
+    const int j2 = __ldg(idx + i);
+    const float g = __fmul_rn(gs.at(second, o), 2.0f);
+    float a[3], acc[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) a[c] = __ldg(A + 3 * i + c);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) acc[c] = __fmul_rn(g, __fsub_rn(a[c], __ldg(Bp + 3 * j2 + c)));
+    // LW_ROUNDS x 32 sources per pass: their loads are all issued before the first add of the pass
+    constexpr int LW_ROUNDS = 4;
+    const int lo = __ldg(rp + i), hi = __ldg(rp + i + 1);
+    for (int q0 = lo; q0 < hi; q0 += 32 * LW_ROUNDS) {
+      int j[LW_ROUNDS];
+      float v[LW_ROUNDS][3];
+#pragma unroll
+      for (int r = 0; r < LW_ROUNDS; ++r) j[r] = q0 + r * 32 + lane < hi ? __ldg(rs + q0 + r * 32 + lane) : -1;
+#pragma unroll
+      for (int r = 0; r < LW_ROUNDS; ++r) {
+        v[r][0] = v[r][1] = v[r][2] = 0.f;
+        if (j[r] >= 0) {
+          const float gj = __fmul_rn(gs.at(!second, so + j[r]), 2.0f);
+#pragma unroll
+          for (int c = 0; c < 3; ++c) v[r][c] = -__fmul_rn(gj, __fsub_rn(__ldg(Bp + 3 * j[r] + c), a[c]));
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < LW_ROUNDS; ++r) {
+        const int cnt = min(32, hi - (q0 + r * 32));
+        for (int l = 0; l < cnt; ++l) {
+#pragma unroll
+          for (int c = 0; c < 3; ++c) acc[c] = __fadd_rn(acc[c], __shfl_sync(0xffffffffu, v[r][c], l));
+        }
+      }
+    }
+    if (lane == 0) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) ga[3 * i + c] = acc[c];
+    }
+  }
+}
+
+static size_t chamfer_bwd_det_bytes(int b, int n, int m) {
+  return (rev_map_bytes(b, m, n) + 255) / 256 * 256 + rev_map_bytes(b, n, m);
+}
+
+template <typename GradSrc>
+static int launch_chamfer_bwd_det(const float *xyz1, const float *xyz2, const int *idx1, const int *idx2, const GradSrc &gs,
+                                  int b, int n, int m, float *gx1, float *gx2, void *ws, cudaStream_t st) {
+  const long long bpc = (static_cast<long long>(n) + m + 255) / 256;
+  if (bpc * b > 0x7fffffffLL) return PDAE_E_UNSUPPORTED;
+  RevMap rev1, rev2;
+  unsigned char *w = static_cast<unsigned char *>(ws);
+  int rc = rev_map_build(idx2, b, m, n, w, &rev1, st);
+  if (rc) return rc;
+  rc = rev_map_build(idx1, b, n, m, w + (rev_map_bytes(b, m, n) + 255) / 256 * 256, &rev2, st);
+  if (rc) return rc;
+  chamfer_bwd_det_kernel<GradSrc><<<static_cast<unsigned>(bpc * b), 256, 0, st>>>(xyz1, xyz2, idx1, idx2, gs, n, m,
+                                                                                  static_cast<int>(bpc), rev1, rev2, gx1, gx2);
+  PDAE_RETURN_IF_LAUNCH_FAILED();
+  if (n > REV_SHORT || m > REV_SHORT) {  // otherwise no bucket can be long
+    const long long most = static_cast<long long>(b) * (n / (REV_SHORT + 1) + m / (REV_SHORT + 1));  // long buckets at most
+    const long long cap = 4LL * sm_count();
+    const long long blocks = (most + 7) / 8 < cap ? (most + 7) / 8 : cap;
+    chamfer_bwd_det_long_kernel<GradSrc><<<static_cast<unsigned>(blocks), 256, 0, st>>>(xyz1, xyz2, idx1, idx2, gs, n, m, rev1,
+                                                                                        rev2, gx1, gx2);
+    PDAE_RETURN_IF_LAUNCH_FAILED();
+  }
+  return 0;
+}
+
 // ---- fused mean losses: (mean f(dist1), mean f(dist2)) with f = identity (L2) or sqrt (L1) ------------------
 // reference: extensions/chamfer_dist/__init__.py:43 (L2: mean + mean) and :413-417 (L1: (mean sqrt + mean sqrt) / 2),
 // there two or four torch kernels plus the add.  Deterministic: fixed-size partial sums in fp32 per CTA (fp64 across
@@ -534,17 +683,6 @@ __global__ void __launch_bounds__(256) unpack_keys_kernel(const uint64_t *__rest
 }
 
 // tuning hook: PDAE_CHAMFER_CFG selects the CTA shape of the large-cloud kernel
-// SMs of the current device (cached per device index; the grid of the balanced kernel is two CTAs per SM)
-static int sm_count() {
-  static int cached[64];
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
-  if (cached[dev] == 0) {
-    int n = 0;
-    cached[dev] = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : 148;
-  }
-  return cached[dev];
-}
 
 static int g_chamfer_variant = -1;
 static int chamfer_variant() {
@@ -1268,4 +1406,46 @@ extern "C" int pdae_chamfer_loss_bwd_f32(const float *xyz1, const float *xyz2, c
   const float n1 = static_cast<float>(t1), n2 = static_cast<float>(t2);
   return launch_chamfer_bwd(xyz1, xyz2, idx1, idx2, GradMean{gloss, dist1, dist2, w1 / n1, w2 / n2, l1 ? 1 : 0}, b, n, m, gx1,
                             gx2, st);
+}
+
+extern "C" size_t pdae_chamfer_bwd_det_workspace_bytes(int b, int n, int m) {
+  if (b <= 0 || n <= 0 || m <= 0) return 0;
+  return chamfer_bwd_det_bytes(b, n, m);
+}
+
+extern "C" int pdae_chamfer_bwd_det_f32(const float *xyz1, const float *xyz2, const int *idx1, const int *idx2,
+                                        const float *gd1, const float *gd2, int b, int n, int m, float *gx1, float *gx2,
+                                        void *workspace, size_t workspace_bytes, pdae_stream_t stream) {
+  if (b < 0 || n < 0 || m < 0) return PDAE_E_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long t1 = static_cast<long long>(b) * n, t2 = static_cast<long long>(b) * m;
+  if ((t1 && (!xyz1 || !gx1)) || (t2 && (!xyz2 || !gx2))) return PDAE_E_INVALID;
+  if (n == 0 || m == 0 || b == 0) {
+    if (t1) PDAE_CUDA_TRY(cudaMemsetAsync(gx1, 0, static_cast<size_t>(t1) * 3 * sizeof(float), st));
+    if (t2) PDAE_CUDA_TRY(cudaMemsetAsync(gx2, 0, static_cast<size_t>(t2) * 3 * sizeof(float), st));
+    return 0;
+  }
+  if (!idx1 || !idx2 || !gd1 || !gd2) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_chamfer_bwd_det_workspace_bytes(b, n, m)) return PDAE_E_WORKSPACE;
+  return launch_chamfer_bwd_det(xyz1, xyz2, idx1, idx2, GradArrays{gd1, gd2}, b, n, m, gx1, gx2, workspace, st);
+}
+
+extern "C" int pdae_chamfer_loss_bwd_det_f32(const float *xyz1, const float *xyz2, const int *idx1, const int *idx2,
+                                             const float *dist1, const float *dist2, const float *gloss, float w1, float w2,
+                                             int b, int n, int m, int l1, float *gx1, float *gx2, void *workspace,
+                                             size_t workspace_bytes, pdae_stream_t stream) {
+  if (b < 0 || n < 0 || m < 0) return PDAE_E_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long t1 = static_cast<long long>(b) * n, t2 = static_cast<long long>(b) * m;
+  if ((t1 && (!xyz1 || !gx1)) || (t2 && (!xyz2 || !gx2))) return PDAE_E_INVALID;
+  if (n == 0 || m == 0 || b == 0) {
+    if (t1) PDAE_CUDA_TRY(cudaMemsetAsync(gx1, 0, static_cast<size_t>(t1) * 3 * sizeof(float), st));
+    if (t2) PDAE_CUDA_TRY(cudaMemsetAsync(gx2, 0, static_cast<size_t>(t2) * 3 * sizeof(float), st));
+    return 0;
+  }
+  if (!idx1 || !idx2 || !gloss || (l1 && (!dist1 || !dist2))) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_chamfer_bwd_det_workspace_bytes(b, n, m)) return PDAE_E_WORKSPACE;
+  const float n1 = static_cast<float>(t1), n2 = static_cast<float>(t2);
+  return launch_chamfer_bwd_det(xyz1, xyz2, idx1, idx2, GradMean{gloss, dist1, dist2, w1 / n1, w2 / n2, l1 ? 1 : 0}, b, n, m,
+                                gx1, gx2, workspace, st);
 }

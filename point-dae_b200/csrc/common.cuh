@@ -81,6 +81,19 @@ __device__ __forceinline__ uint64_t pack_key(float d, uint32_t i) {
 }
 
 static inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
+static inline size_t align256(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
+
+// SMs of the current device (cached per device index; 148 if the query fails)
+inline int sm_count() {
+  static int cached[64];
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
+  if (cached[dev] == 0) {
+    int n = 0;
+    cached[dev] = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : 148;
+  }
+  return cached[dev];
+}
 
 // cross-file internals
 // knn.cu: planar-input, any-channel-count DGCNN kNN (warp-select kernel); used directly for small c.

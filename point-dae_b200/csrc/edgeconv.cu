@@ -12,6 +12,7 @@
 // traffic is b*n*k*co*4 bytes of gathered reads instead of writing and re-reading both tensors.
 // Bound: L2 gather bandwidth.  STATUS: bit-exact with its oracle on B200 (tests/test_row4_edgeconv.py); not yet timed.
 #include "common.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -496,53 +497,6 @@ extern "C" int pdae_edge_backward_f32(const float *z, int ld, const int64_t *idx
 // floats: 0.66 ms -> ~0.15 ms at 16 x 2048, k = 20, co = 256.
 namespace pdae {
 
-__global__ void __launch_bounds__(256) edge_rev_count_kernel(const int64_t *__restrict__ idx, int n, int k, long long total,
-                                                             int *__restrict__ cnt) {
-  const long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (e >= total) return;
-  const long long cloud = e / (static_cast<long long>(n) * k);
-  atomicAdd(cnt + cloud * n + static_cast<int>(__ldg(idx + e)), 1);
-}
-
-// one CTA per cloud: ptr[p] = exclusive prefix sum of cnt (n + 1 entries); cnt is zeroed for its second life as cursor
-__global__ void __launch_bounds__(1024) edge_rev_scan_kernel(int *__restrict__ cnt, int n, int *__restrict__ ptr) {
-  __shared__ int part[1024];
-  int *c = cnt + static_cast<size_t>(blockIdx.x) * n;
-  int *p = ptr + static_cast<size_t>(blockIdx.x) * (n + 1);
-  const int per = (n + 1023) / 1024, lo = threadIdx.x * per, hi = min(n, lo + per);
-  int s = 0;
-  for (int t = lo; t < hi; ++t) s += c[t];
-  part[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = 1; o < 1024; o <<= 1) {  // Hillis-Steele inclusive scan of the 1024 partial sums
-    const int v = threadIdx.x >= o ? part[threadIdx.x - o] : 0;
-    __syncthreads();
-    part[threadIdx.x] += v;
-    __syncthreads();
-  }
-  int run = threadIdx.x ? part[threadIdx.x - 1] : 0;
-  for (int t = lo; t < hi; ++t) {
-    const int v = c[t];
-    p[t] = run;
-    run += v;
-    c[t] = 0;
-  }
-  if (threadIdx.x == 1023) p[n] = part[1023];
-}
-
-__global__ void __launch_bounds__(256) edge_rev_fill_kernel(const int64_t *__restrict__ idx, int n, int k, long long total,
-                                                            const int *__restrict__ ptr, int *__restrict__ cursor,
-                                                            int *__restrict__ src) {
-  const long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (e >= total) return;
-  const long long cloud = e / (static_cast<long long>(n) * k);
-  const int within = static_cast<int>(e - cloud * n * k);
-  const int i = within / k;
-  const int tgt = static_cast<int>(__ldg(idx + e));
-  const int pos = atomicAdd(cursor + cloud * n + tgt, 1);
-  src[cloud * n * k + __ldg(ptr + cloud * (n + 1) + tgt) + pos] = i;  // the source point of the edge
-}
-
 __global__ void __launch_bounds__(EC_WARPS * 32) edge_backward_dense_kernel(const EdgeArgs a, const float *__restrict__ s1,
                                                                             const int *__restrict__ ptr, const int *__restrict__ src,
                                                                             const float *__restrict__ mean,
@@ -646,13 +600,9 @@ extern "C" int pdae_edge_backward_dense_f32(const float *z, int ld, const int64_
   int *src = ptr + static_cast<size_t>(b) * (n + 1);     // (b, n * k)
   const long long total = static_cast<long long>(b) * n * k;
   if ((total + 255) / 256 > 0x7fffffffLL) return PDAE_E_UNSUPPORTED;
-  PDAE_CUDA_TRY(cudaMemsetAsync(cnt, 0, static_cast<size_t>(b) * n * sizeof(int), st));
-  edge_rev_count_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(idx, n, k, total, cnt);
-  PDAE_RETURN_IF_LAUNCH_FAILED();
-  edge_rev_scan_kernel<<<b, 1024, 0, st>>>(cnt, n, ptr);
-  PDAE_RETURN_IF_LAUNCH_FAILED();
-  edge_rev_fill_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(idx, n, k, total, ptr, cnt, src);
-  PDAE_RETURN_IF_LAUNCH_FAILED();
+  if (static_cast<long long>(n) * k > 0x7fffffffLL) return PDAE_E_UNSUPPORTED;
+  const int rrc = rev_csr_unordered(idx, b, n * k, n, k, cnt, ptr, src, st);  // src = the source POINT of each edge
+  if (rrc) return rrc;
   const dim3 grid(static_cast<unsigned>((n + EC_POINTS - 1) / EC_POINTS), static_cast<unsigned>(b));
   edge_backward_dense_kernel<<<grid, EC_WARPS * 32, 0, st>>>(EdgeArgs{z, idx, ld, n, k, co}, s1, ptr, src, mean, invstd, ca, cb, dz);
   PDAE_RETURN_IF_LAUNCH_FAILED();

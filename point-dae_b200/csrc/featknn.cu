@@ -11,6 +11,7 @@
 #include <stdlib.h>
 
 #include "knn_select.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -146,6 +147,28 @@ __global__ void __launch_bounds__(256) graph_feature_grad_center_kernel(const fl
   float s = 0.f;
   for (int p = 0; p < k; ++p) s += __ldg(g + static_cast<size_t>(p) * 2 * c + c + ch) - __ldg(g + static_cast<size_t>(p) * 2 * c + ch);
   atomicAdd(gxt + e, s);
+}
+
+// backward, deterministic: gxt[b, j, ch] = centre term of row j (p ascending), then (+) G[b, i, p, ch] for every edge
+// with idx[b][i][p] == j, slot i * k + p ascending (the ordered reverse map of idx)       (thread per (b,j,ch))
+__global__ void __launch_bounds__(256) graph_feature_grad_det_kernel(const float *__restrict__ gout, int c, int n, int k,
+                                                                     long long total, RevMap map, float *__restrict__ gxt) {
+  const long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (e >= total) return;
+  const long long bj = e / c;
+  const int ch = static_cast<int>(e - bj * c);
+  const long long bb = bj / n;
+  const int j = static_cast<int>(bj - bb * n);
+  const float *g = gout + bj * k * 2 * c;
+  float s = 0.f;
+  for (int p = 0; p < k; ++p)
+    s = __fadd_rn(s, __fsub_rn(__ldg(g + static_cast<size_t>(p) * 2 * c + c + ch), __ldg(g + static_cast<size_t>(p) * 2 * c + ch)));
+  const int *rp = map.ptr + bb * (n + 1);
+  const int *rs = map.slot + bb * n * k;
+  const float *gc = gout + bb * n * k * 2 * c + ch;
+  const int lo = __ldg(rp + j), hi = __ldg(rp + j + 1);
+  for (int q = lo; q < hi; ++q) s = __fadd_rn(s, __ldg(gc + static_cast<size_t>(__ldg(rs + q)) * 2 * c));
+  gxt[e] = s;
 }
 
 // backward, fused and vectorised (c % 4 == 0): one thread per (point, 4 channels) walks its k neighbour rows once:
@@ -917,6 +940,35 @@ extern "C" int pdae_graph_feature_grad_f32(const float *gout, const int64_t *idx
   PDAE_RETURN_IF_LAUNCH_FAILED();
   graph_feature_grad_scatter_kernel<<<static_cast<unsigned>((ts + 255) / 256), 256, 0, st>>>(gout, idx, c, n, k, ts,
                                                                                           gxt);
+  PDAE_RETURN_IF_LAUNCH_FAILED();
+  return launch_transpose(gxt, gx, b, n, c, st);  // (b,n,c) -> (b,c,n)
+}
+
+extern "C" size_t pdae_graph_feature_grad_det_workspace_bytes(int b, int c, int n, int k) {
+  if (b <= 0 || c <= 0 || n <= 0 || k < 0 || static_cast<long long>(n) * k > 0x7fffffffLL) return 0;
+  return align256(rev_map_bytes(b, n * k, n)) + static_cast<size_t>(b) * c * n * sizeof(float);
+}
+
+extern "C" int pdae_graph_feature_grad_det_f32(const float *gout, const int64_t *idx, int b, int c, int n, int k, float *gx,
+                                               void *workspace, size_t workspace_bytes, pdae_stream_t stream) {
+  if (b < 0 || c <= 0 || n < 0 || k < 0) return PDAE_E_INVALID;
+  const size_t gsz = static_cast<size_t>(b) * c * n;
+  if (gsz == 0) return 0;
+  if (!gx) return PDAE_E_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (k == 0) {
+    PDAE_CUDA_TRY(cudaMemsetAsync(gx, 0, gsz * sizeof(float), st));
+    return 0;
+  }
+  if (!gout || !idx || static_cast<long long>(n) * k > 0x7fffffffLL) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_graph_feature_grad_det_workspace_bytes(b, c, n, k)) return PDAE_E_WORKSPACE;
+  RevMap map;
+  int rc = rev_map_build(idx, b, n * k, n, workspace, &map, st);
+  if (rc) return rc;
+  float *gxt = reinterpret_cast<float *>(static_cast<unsigned char *>(workspace) + align256(rev_map_bytes(b, n * k, n)));
+  const long long tc = static_cast<long long>(b) * n * c;
+  if ((tc + 255) / 256 > 0x7fffffffLL) return PDAE_E_UNSUPPORTED;
+  graph_feature_grad_det_kernel<<<static_cast<unsigned>((tc + 255) / 256), 256, 0, st>>>(gout, c, n, k, tc, map, gxt);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return launch_transpose(gxt, gx, b, n, c, st);  // (b,n,c) -> (b,c,n)
 }

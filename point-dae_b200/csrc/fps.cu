@@ -25,6 +25,7 @@
 #include <cooperative_groups.h>
 
 #include "common.cuh"
+#include "reverse.cuh"
 #include "fps_rank.cuh"
 
 namespace cg = cooperative_groups;
@@ -564,4 +565,24 @@ extern "C" int pdae_gather_grad_f32(const float *gout, const int *idx, int b, in
   gather_grad_kernel<<<static_cast<unsigned>(grid), 256, 0, st>>>(gout, idx, c, n, m, total, gfeat);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
+}
+
+// deterministic form: gfeat[b][l][p] = +0 (+) gout[b][l][j] for every j with idx[b][j] == p, j ascending (reverse.cuh)
+extern "C" size_t pdae_gather_grad_det_workspace_bytes(int b, int n, int m) {
+  if (b <= 0 || n < 0 || m < 0) return 0;
+  return rev_map_bytes(b, m, n);
+}
+
+extern "C" int pdae_gather_grad_det_f32(const float *gout, const int *idx, int b, int c, int n, int m, float *gfeat,
+                                        void *workspace, size_t workspace_bytes, pdae_stream_t stream) {
+  if (b < 0 || c < 0 || n < 0 || m < 0) return PDAE_E_INVALID;
+  const size_t gsz = static_cast<size_t>(b) * c * n;
+  if (gsz == 0) return 0;
+  if (!gfeat || (m && (!gout || !idx))) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_gather_grad_det_workspace_bytes(b, n, m)) return PDAE_E_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  RevMap map;
+  const int rc = rev_map_build(idx, b, m, n, workspace, &map, st);
+  if (rc) return rc;
+  return rev_gather_channel_major(gout, nullptr, b, c, m, n, 1, map, gfeat, st);
 }

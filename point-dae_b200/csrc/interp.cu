@@ -14,6 +14,7 @@
 // the grid, the known cloud streams through shared memory as planes (one LDS.128 feeds four candidates) and the
 // three best stay in registers behind a single "beats the third" test.
 #include "common.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -173,4 +174,26 @@ extern "C" int pdae_three_interpolate_grad_f32(const float *gout, const int *idx
   three_interpolate_grad_kernel<<<grid, 256, 0, st>>>(gout, idx, weight, c, m, n, gpoints);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
+}
+
+// deterministic form: gpoints[b][l][p] = +0 (+) rn(gout[b][l][i] * weight[b][i][s]) over the slots i * 3 + s with
+// idx == p, ascending
+extern "C" size_t pdae_three_interpolate_grad_det_workspace_bytes(int b, int n, int m) {
+  if (b <= 0 || n < 0 || m < 0 || 3LL * n > 0x7fffffffLL) return 0;
+  return rev_map_bytes(b, 3 * n, m);
+}
+
+extern "C" int pdae_three_interpolate_grad_det_f32(const float *gout, const int *idx, const float *weight, int b, int c, int n,
+                                                   int m, float *gpoints, void *workspace, size_t workspace_bytes,
+                                                   pdae_stream_t stream) {
+  if (b < 0 || c < 0 || m < 0 || n < 0 || 3LL * n > 0x7fffffffLL) return PDAE_E_INVALID;
+  const size_t gsz = static_cast<size_t>(b) * c * m;
+  if (gsz == 0) return 0;
+  if (!gpoints || (n && (!gout || !idx || !weight))) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_three_interpolate_grad_det_workspace_bytes(b, n, m)) return PDAE_E_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  RevMap map;
+  const int rc = rev_map_build(idx, b, 3 * n, m, workspace, &map, st);
+  if (rc) return rc;
+  return rev_gather_channel_major(gout, weight, b, c, 3 * n, m, 3, map, gpoints, st);
 }

@@ -11,6 +11,7 @@
 //     metric 3  dis_normalized_l2_strict  |u - w|^2
 // (torch semantics: F.normalize's eps clamp, torch.min's tie splitting the gradient, sign(0) = 0 for |.|).
 #include "common.cuh"
+#include "reverse.cuh"
 
 namespace pdae {
 
@@ -151,6 +152,42 @@ __global__ void __launch_bounds__(256) pair_loss_bwd_kernel(const PairArgs x, co
   }
 }
 
+// deterministic form: a point's own term, then the matched rows' terms (the points of the other cloud that chose it,
+// ascending), rounded fp32 products and adds.  rev1 lists per point of a the points of b with idx2 == it, rev2 the converse.
+__global__ void __launch_bounds__(256) pair_loss_bwd_det_kernel(const PairArgs x, const float *__restrict__ gloss, float w1,
+                                                                float w2, RevMap rev1, RevMap rev2, float *__restrict__ ga,
+                                                                float *__restrict__ gb) {
+  const int cloud = blockIdx.y, t = blockIdx.x * 256 + threadIdx.x;
+  const int n = x.n, m = x.m, d = x.d;
+  if (t >= n + m) return;
+  const bool side1 = t < n;
+  const int j = side1 ? t : t - n;
+  const size_t own_o = side1 ? (static_cast<size_t>(cloud) * n + j) * d : (static_cast<size_t>(cloud) * m + j) * d;
+  const int k = side1 ? __ldg(x.idx1 + static_cast<size_t>(cloud) * n + j) : __ldg(x.idx2 + static_cast<size_t>(cloud) * m + j);
+  const size_t oth_o = side1 ? (static_cast<size_t>(cloud) * m + k) * d : (static_cast<size_t>(cloud) * n + k) * d;
+  const float *own = (side1 ? x.a : x.b) + own_o, *oth = (side1 ? x.b : x.a) + oth_o;
+  float p[PL_MAXD], q[PL_MAXD], acc[PL_MAXD];
+  for (int e = 0; e < d; ++e) p[e] = __ldg(own + e), q[e] = __ldg(oth + e);
+  PairVal o;
+  pair_metric<true>(p, q, d, x.metric, o);
+  const float g = __ldg(gloss) * (side1 ? w1 : w2), gs = __ldg(gloss) * (side1 ? w2 : w1);
+  for (int e = 0; e < d; ++e) acc[e] = __fmul_rn(g, o.gp[e]);
+  // sources: points of the other cloud (rows `src`) whose match is this point (row p)
+  const int ns = side1 ? m : n, nt = side1 ? n : m;
+  const int *rp = (side1 ? rev1.ptr : rev2.ptr) + static_cast<size_t>(cloud) * (nt + 1);
+  const int *rs = (side1 ? rev1.slot : rev2.slot) + static_cast<size_t>(cloud) * ns;
+  const float *src = (side1 ? x.b : x.a) + static_cast<size_t>(cloud) * ns * d;
+  const int lo = __ldg(rp + j), hi = __ldg(rp + j + 1);
+  for (int qq = lo; qq < hi; ++qq) {
+    const int i = __ldg(rs + qq);
+    for (int e = 0; e < d; ++e) q[e] = __ldg(src + static_cast<size_t>(i) * d + e);
+    pair_metric<true>(q, p, d, x.metric, o);
+    for (int e = 0; e < d; ++e) acc[e] = __fadd_rn(acc[e], __fmul_rn(gs, o.gt[e]));
+  }
+  float *gown = (side1 ? ga : gb) + own_o;
+  for (int e = 0; e < d; ++e) gown[e] = acc[e];
+}
+
 }  // namespace pdae
 
 using namespace pdae;
@@ -191,6 +228,36 @@ extern "C" int pdae_pair_loss_bwd_f32(const float *a, const float *b, const int 
   pair_loss_bwd_kernel<false><<<grid, 256, 0, st>>>(x, gloss, w1, w2, ga, gb);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   pair_loss_bwd_kernel<true><<<grid, 256, 0, st>>>(x, gloss, w1, w2, ga, gb);
+  PDAE_RETURN_IF_LAUNCH_FAILED();
+  return 0;
+}
+
+static size_t pair_det_bytes(int bs, int n, int m) {
+  return (rev_map_bytes(bs, m, n) + 255) / 256 * 256 + rev_map_bytes(bs, n, m);
+}
+
+extern "C" size_t pdae_pair_loss_bwd_det_workspace_bytes(int bs, int n, int m) {
+  if (bs <= 0 || n <= 0 || m <= 0) return 0;
+  return pair_det_bytes(bs, n, m);
+}
+
+extern "C" int pdae_pair_loss_bwd_det_f32(const float *a, const float *b, const int *idx1, const int *idx2, const float *gloss,
+                                          float w1, float w2, int bs, int n, int m, int d, int metric, float *ga, float *gb,
+                                          void *workspace, size_t workspace_bytes, pdae_stream_t stream) {
+  const int rc = pair_check(a, b, idx1, idx2, bs, n, m, d, metric);
+  if (rc) return rc;
+  if (bs == 0 || n + m == 0) return 0;
+  if (!gloss || !ga || !gb || n == 0 || m == 0) return PDAE_E_INVALID;
+  if (!workspace || workspace_bytes < pdae_pair_loss_bwd_det_workspace_bytes(bs, n, m)) return PDAE_E_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  unsigned char *w = static_cast<unsigned char *>(workspace);
+  RevMap rev1, rev2;
+  int r = rev_map_build(idx2, bs, m, n, w, &rev1, st);
+  if (r) return r;
+  r = rev_map_build(idx1, bs, n, m, w + (rev_map_bytes(bs, m, n) + 255) / 256 * 256, &rev2, st);
+  if (r) return r;
+  const dim3 grid((n + m + 255) / 256, bs);
+  pair_loss_bwd_det_kernel<<<grid, 256, 0, st>>>(PairArgs{a, b, idx1, idx2, n, m, d, metric}, gloss, w1, w2, rev1, rev2, ga, gb);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
 }

@@ -7,6 +7,7 @@
 //            patchifier's CTAs start where and when a forward CTA exits
 //   aux:     fused mean loss (two launches)            } both wait for the forward only and run beside the patchifier;
 //   side:    backward from the loss scalar (two launches) } `stream` waits for both before the call returns
+//            (PDAE_STEP_DETERMINISTIC: the deterministic backward, which builds its reverse maps there first)
 //
 // From Python every launch costs 20-30 us of host time, so a step was replayed as a CUDA graph -- and consecutive graph
 // launches on one stream leave ~10 us between them (measured: 166.7 us per step replayed, 156.7 us with the same launches
@@ -48,24 +49,34 @@ int step_streams(StepStreams **out) {
   return 0;
 }
 
-size_t align256(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
-
 }  // namespace
 }  // namespace pdae
 
 using namespace pdae;
 
-extern "C" size_t pdae_step_workspace_bytes(int b, int n, int g, int m) {
+extern "C" size_t pdae_step_workspace_bytes(int b, int n, int g, int m) { return pdae_step_ex_workspace_bytes(b, n, g, m, 0u); }
+
+// PDAE_STEP_DETERMINISTIC adds the ordered reverse maps of the deterministic backward after the other regions
+extern "C" size_t pdae_step_ex_workspace_bytes(int b, int n, int g, int m, unsigned flags) {
   if (b <= 0 || n <= 0) return 0;
+  const size_t det = (flags & PDAE_STEP_DETERMINISTIC) ? align256(pdae_chamfer_bwd_det_workspace_bytes(b, n, n)) : 0;
   return align256(pdae_chamfer_fwd_workspace_bytes(b, n, n)) + align256(pdae_chamfer_loss_workspace_bytes()) +
-         align256(pdae_fps_group_workspace_bytes(b, n, g, m));
+         align256(pdae_fps_group_workspace_bytes(b, n, g, m)) + det;
 }
 
 extern "C" int pdae_step_f32(const float *cloud, const float *pred, int b, int n, int g, int m, int *fps_idx, float *center,
                              float *neighborhood, float *dist1, float *dist2, int *idx1, int *idx2, float *loss3,
                              const float *gloss, float *gpred, float *gcloud, void *workspace, size_t workspace_bytes,
                              pdae_stream_t stream) {
-  if (b < 0 || n < 0 || g < 0 || m <= 0) return PDAE_E_INVALID;
+  return pdae_step_ex_f32(cloud, pred, b, n, g, m, fps_idx, center, neighborhood, dist1, dist2, idx1, idx2, loss3, gloss, gpred,
+                          gcloud, workspace, workspace_bytes, 0u, stream);
+}
+
+extern "C" int pdae_step_ex_f32(const float *cloud, const float *pred, int b, int n, int g, int m, int *fps_idx, float *center,
+                                float *neighborhood, float *dist1, float *dist2, int *idx1, int *idx2, float *loss3,
+                                const float *gloss, float *gpred, float *gcloud, void *workspace, size_t workspace_bytes,
+                                unsigned flags, pdae_stream_t stream) {
+  if (b < 0 || n < 0 || g < 0 || m <= 0 || (flags & ~static_cast<unsigned>(PDAE_STEP_DETERMINISTIC))) return PDAE_E_INVALID;
   if (b == 0) return 0;
   if (n == 0 || m > n) return PDAE_E_INVALID;
   if (!cloud || !pred || !dist1 || !dist2 || !idx1 || !idx2 || !loss3 || !gloss || !gpred || !gcloud) return PDAE_E_INVALID;
@@ -73,7 +84,10 @@ extern "C" int pdae_step_f32(const float *cloud, const float *pred, int b, int n
   const size_t w_fwd = align256(pdae_chamfer_fwd_workspace_bytes(b, n, n));
   const size_t w_loss = align256(pdae_chamfer_loss_workspace_bytes());
   const size_t w_patch = align256(pdae_fps_group_workspace_bytes(b, n, g, m));
-  if (w_fwd + w_loss + w_patch > 0 && (!workspace || workspace_bytes < w_fwd + w_loss + w_patch)) return PDAE_E_WORKSPACE;
+  const bool det = (flags & PDAE_STEP_DETERMINISTIC) != 0;
+  const size_t w_det = det ? align256(pdae_chamfer_bwd_det_workspace_bytes(b, n, n)) : 0;
+  if (w_fwd + w_loss + w_patch + w_det > 0 && (!workspace || workspace_bytes < w_fwd + w_loss + w_patch + w_det))
+    return PDAE_E_WORKSPACE;
   unsigned char *ws = static_cast<unsigned char *>(workspace);
   StepStreams *s = nullptr;
   int rc = step_streams(&s);
@@ -100,7 +114,11 @@ extern "C" int pdae_step_f32(const float *cloud, const float *pred, int b, int n
   if (rc) return rc;
   PDAE_CUDA_TRY(cudaEventRecord(s->loss_done, s->aux));
   PDAE_CUDA_TRY(cudaStreamWaitEvent(s->side, s->fwd_done, 0));
-  rc = pdae_chamfer_loss_bwd_f32(pred, cloud, idx1, idx2, dist1, dist2, gloss, 1.0f, 1.0f, b, n, n, 0, gpred, gcloud, s->side);
+  if (det)
+    rc = pdae_chamfer_loss_bwd_det_f32(pred, cloud, idx1, idx2, dist1, dist2, gloss, 1.0f, 1.0f, b, n, n, 0, gpred, gcloud,
+                                       ws + w_fwd + w_loss + w_patch, w_det, s->side);
+  else
+    rc = pdae_chamfer_loss_bwd_f32(pred, cloud, idx1, idx2, dist1, dist2, gloss, 1.0f, 1.0f, b, n, n, 0, gpred, gcloud, s->side);
   if (rc) return rc;
   PDAE_CUDA_TRY(cudaEventRecord(s->bwd_done, s->side));
   PDAE_CUDA_TRY(cudaStreamWaitEvent(st, s->loss_done, 0));

@@ -52,7 +52,10 @@ def _fusable(block):
             and tuple(conv.stride) == (1, 1) and conv.groups == 1 and isinstance(bn, torch.nn.BatchNorm2d)
             and isinstance(act, torch.nn.LeakyReLU) and len(block) == 3
             and (bn.training or bn.running_mean is not None)  # eval mode needs running statistics
-            and not torch.is_autocast_enabled())
+            and not torch.is_autocast_enabled()
+            # the fused kernels accumulate their statistics and gradients with float atomics; under
+            # torch.use_deterministic_algorithms(True) the reference composition runs, whose backward is deterministic
+            and not torch.are_deterministic_algorithms_enabled())
 
 
 def edge_conv(x, block, k=20, idx=None):

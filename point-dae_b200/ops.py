@@ -71,6 +71,15 @@ def _dense_storage(t):
 
 
 # ------------------------------------------------------------------------------------------ FPS
+def _deterministic():
+    """torch.use_deterministic_algorithms(True) selects the gradients without float atomics (the *_det entry points)."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _workspace(nbytes, dev):
+    return torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=dev)
+
+
 def fps_block_size(n):
     return int(_native.lib().pdae_fps_block_size(int(n)))
 
@@ -141,8 +150,14 @@ def gather_points_grad(grad_out, idx, n):
     b, c, m = grad_out.shape
     with _on(grad_out.device):
         out = torch.empty((b, c, int(n)), dtype=torch.float32, device=grad_out.device)
-        rc = _native.lib().pdae_gather_grad_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), m, out.data_ptr(),
-                                                _stream())
+        L = _native.lib()
+        if _deterministic():
+            nbytes = L.pdae_gather_grad_det_workspace_bytes(b, int(n), m)
+            ws = _workspace(nbytes, grad_out.device)
+            rc = L.pdae_gather_grad_det_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), m, out.data_ptr(), ws.data_ptr(),
+                                            nbytes, _stream())
+        else:
+            rc = L.pdae_gather_grad_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), m, out.data_ptr(), _stream())
     _native.check(rc, "pdae_gather_grad_f32")
     return out
 
@@ -277,10 +292,14 @@ def fps_group(xyz, num_group, group_size, want_idx=False, overlap_previous=False
 
 
 class StepBuffers:
-    """Outputs and workspace of `hot_step`, allocated once per shape (a training loop reuses them every step)."""
+    """Outputs and workspace of `hot_step`, allocated once per shape (a training loop reuses them every step).
+    deterministic (default: torch.are_deterministic_algorithms_enabled()) sizes the workspace for the deterministic
+    backward as well; `hot_step` grows it in place when a step needs it and the buffers were built without it."""
 
-    def __init__(self, b, n, g, m, device):
-        L = _native.lib()
+    def __init__(self, b, n, g, m, device, deterministic=None):
+        if deterministic is None:
+            deterministic = _deterministic()
+        self.shape = (b, n, g, m)
         f32, i32 = torch.float32, torch.int32
         with _on(device):
             self.fps_idx = torch.empty((b, g), dtype=i32, device=device)
@@ -293,17 +312,30 @@ class StepBuffers:
             self.loss3 = torch.empty(3, dtype=f32, device=device)
             self.gpred = torch.empty((b, n, 3), dtype=f32, device=device)
             self.gcloud = torch.empty((b, n, 3), dtype=f32, device=device)
-            self.ws_bytes = int(L.pdae_step_workspace_bytes(b, n, g, m))
-            self.ws = torch.empty(max(self.ws_bytes, 1), dtype=torch.uint8, device=device)
-        self.shape = (b, n, g, m)
+            self.flags = 0
+            self.ws_bytes = 0
+            self.ws = None
+            self.reserve(deterministic)
+
+    def reserve(self, deterministic):
+        """make the workspace large enough for the deterministic (or default) step; only `ws` changes, the outputs stay"""
+        flags = 1 if deterministic else 0  # PDAE_STEP_DETERMINISTIC
+        if self.ws is not None and flags <= self.flags:
+            return
+        device = self.loss3.device
+        with _on(device):
+            nbytes = int(_native.lib().pdae_step_ex_workspace_bytes(*self.shape, flags))
+            self.ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=device)
+        self.ws_bytes, self.flags = nbytes, flags
 
 
-def hot_step(cloud, pred, num_group, group_size, gloss, buffers=None):
+def hot_step(cloud, pred, num_group, group_size, gloss, buffers=None, deterministic=None):
     """One step of the hot path in ONE native call (csrc/step.cu): Chamfer forward of `pred` against `cloud`, the patchifier
     of `cloud` as a programmatic dependent launch, the fused mean loss and the gradients of that loss scaled by the device
     scalar `gloss`, on the current stream + two library-owned helper streams.  -> StepBuffers (neighborhood, center,
     fps_idx, dist1/2, idx1/2, loss3 = [loss, mean1, mean2], gpred, gcloud); the values of fps_group + chamfer_forward +
-    chamfer_mean_loss + chamfer_loss_backward bit for bit."""
+    chamfer_mean_loss + chamfer_loss_backward bit for bit.  deterministic (default: torch.are_deterministic_algorithms_enabled())
+    selects the backward without float atomics, as chamfer_loss_backward does under that flag."""
     _require_cuda(cloud, "hot_step")
     _require_f32_contig(cloud, "cloud")
     _require_f32_contig(pred, "pred")
@@ -314,14 +346,19 @@ def hot_step(cloud, pred, num_group, group_size, gloss, buffers=None):
     g, m = int(num_group), int(group_size)
     if n < 1 or not (1 <= m <= n):
         raise RuntimeError("group_size=%d must satisfy 1 <= group_size <= %d points" % (m, n))
+    det = _deterministic() if deterministic is None else bool(deterministic)
     if buffers is None or buffers.shape != (b, n, g, m) or buffers.loss3.device != cloud.device:
-        buffers = StepBuffers(b, n, g, m, cloud.device)
+        buffers = StepBuffers(b, n, g, m, cloud.device, deterministic=det)
+    buffers.reserve(det)  # the caller's outputs are kept: only a too-small workspace is replaced
     o = buffers
     with _on(cloud.device):
-        rc = _native.lib().pdae_step_f32(cloud.data_ptr(), pred.data_ptr(), b, n, g, m, o.fps_idx.data_ptr(), o.center.data_ptr(),
-                                         o.neighborhood.data_ptr(), o.dist1.data_ptr(), o.dist2.data_ptr(), o.idx1.data_ptr(),
-                                         o.idx2.data_ptr(), o.loss3.data_ptr(), gloss.data_ptr(), o.gpred.data_ptr(),
-                                         o.gcloud.data_ptr(), o.ws.data_ptr(), o.ws_bytes, _stream())
+        args = (cloud.data_ptr(), pred.data_ptr(), b, n, g, m, o.fps_idx.data_ptr(), o.center.data_ptr(), o.neighborhood.data_ptr(),
+                o.dist1.data_ptr(), o.dist2.data_ptr(), o.idx1.data_ptr(), o.idx2.data_ptr(), o.loss3.data_ptr(), gloss.data_ptr(),
+                o.gpred.data_ptr(), o.gcloud.data_ptr(), o.ws.data_ptr(), o.ws_bytes)
+        if det:
+            rc = _native.lib().pdae_step_ex_f32(*args, 1, _stream())  # PDAE_STEP_DETERMINISTIC
+        else:
+            rc = _native.lib().pdae_step_f32(*args, _stream())
     _native.check(rc, "pdae_step_f32")
     return o
 
@@ -560,9 +597,15 @@ def chamfer_backward(xyz1, xyz2, idx1, idx2, grad_dist1, grad_dist2):
         # preserve_format: dense inputs keep their strides; wider-than-3 rows are only partly written -> zeros
         gx1 = torch.empty_like(xyz1) if xyz1.size(2) == 3 else torch.zeros_like(xyz1)
         gx2 = torch.empty_like(xyz2) if xyz2.size(2) == 3 else torch.zeros_like(xyz2)
-        rc = _native.lib().pdae_chamfer_bwd_f32(xyz1.data_ptr(), xyz2.data_ptr(), idx1.data_ptr(), idx2.data_ptr(),
-                                                grad_dist1.data_ptr(), grad_dist2.data_ptr(), b, n, m, gx1.data_ptr(),
-                                                gx2.data_ptr(), _stream())
+        L = _native.lib()
+        args = (xyz1.data_ptr(), xyz2.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), grad_dist1.data_ptr(),
+                grad_dist2.data_ptr(), b, n, m, gx1.data_ptr(), gx2.data_ptr())
+        if _deterministic():
+            nbytes = L.pdae_chamfer_bwd_det_workspace_bytes(b, n, m)
+            ws = _workspace(nbytes, dev)
+            rc = L.pdae_chamfer_bwd_det_f32(*args, ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_chamfer_bwd_f32(*args, _stream())
     _native.check(rc, "pdae_chamfer_bwd_f32")
     return [gx1, gx2]
 
@@ -609,10 +652,16 @@ def chamfer_loss_backward(xyz1, xyz2, idx1, idx2, dist1, dist2, grad_loss, w1, w
     with _on(dev):
         gx1 = torch.empty_like(xyz1) if xyz1.size(2) == 3 else torch.zeros_like(xyz1)
         gx2 = torch.empty_like(xyz2) if xyz2.size(2) == 3 else torch.zeros_like(xyz2)
-        rc = _native.lib().pdae_chamfer_loss_bwd_f32(
-            xyz1.data_ptr(), xyz2.data_ptr(), idx1.contiguous().data_ptr(), idx2.contiguous().data_ptr(),
-            dist1.contiguous().data_ptr(), dist2.contiguous().data_ptr(), grad_loss.data_ptr(), float(w1), float(w2), b, n,
-            m, 1 if l1 else 0, gx1.data_ptr(), gx2.data_ptr(), _stream())
+        idx1, idx2, dist1, dist2 = idx1.contiguous(), idx2.contiguous(), dist1.contiguous(), dist2.contiguous()
+        L = _native.lib()
+        args = (xyz1.data_ptr(), xyz2.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), dist1.data_ptr(), dist2.data_ptr(),
+                grad_loss.data_ptr(), float(w1), float(w2), b, n, m, 1 if l1 else 0, gx1.data_ptr(), gx2.data_ptr())
+        if _deterministic():
+            nbytes = L.pdae_chamfer_bwd_det_workspace_bytes(b, n, m)
+            ws = _workspace(nbytes, dev)
+            rc = L.pdae_chamfer_loss_bwd_det_f32(*args, ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_chamfer_loss_bwd_f32(*args, _stream())
     _native.check(rc, "pdae_chamfer_loss_bwd_f32")
     return [gx1, gx2]
 
@@ -650,9 +699,15 @@ class MatchedPairLoss(torch.autograd.Function):
         with _on(a.device):
             ga, gb = torch.empty_like(a), torch.empty_like(b)
             gl = g.reshape(1).float().contiguous()
-            rc = _native.lib().pdae_pair_loss_bwd_f32(a.data_ptr(), b.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), gl.data_ptr(),
-                                                      1.0 / (bs * n), 1.0 / (bs * m), bs, n, m, d, ctx.metric, ga.data_ptr(),
-                                                      gb.data_ptr(), _stream())
+            L = _native.lib()
+            args = (a.data_ptr(), b.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), gl.data_ptr(), 1.0 / (bs * n), 1.0 / (bs * m),
+                    bs, n, m, d, ctx.metric, ga.data_ptr(), gb.data_ptr())
+            if _deterministic():
+                nbytes = L.pdae_pair_loss_bwd_det_workspace_bytes(bs, n, m)
+                ws = _workspace(nbytes, a.device)
+                rc = L.pdae_pair_loss_bwd_det_f32(*args, ws.data_ptr(), nbytes, _stream())
+            else:
+                rc = L.pdae_pair_loss_bwd_f32(*args, _stream())
         _native.check(rc, "pdae_pair_loss_bwd_f32")
         return ga, gb, None, None, None
 
@@ -765,10 +820,11 @@ def _graph_feature_bwd(gout_phys, idx, c, n):
     L = _native.lib()
     with _on(gout_phys.device):
         gx = torch.empty((b, c, n), dtype=torch.float32, device=gout_phys.device)
-        nbytes = L.pdae_graph_feature_workspace_bytes(b, c, n)
+        det = _deterministic()
+        nbytes = L.pdae_graph_feature_grad_det_workspace_bytes(b, c, n, k) if det else L.pdae_graph_feature_workspace_bytes(b, c, n)
         ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=gout_phys.device)
-        rc = L.pdae_graph_feature_grad_f32(gout_phys.data_ptr(), idx.data_ptr(), b, c, n, k, gx.data_ptr(),
-                                           ws.data_ptr(), nbytes, _stream())
+        grad = L.pdae_graph_feature_grad_det_f32 if det else L.pdae_graph_feature_grad_f32
+        rc = grad(gout_phys.data_ptr(), idx.data_ptr(), b, c, n, k, gx.data_ptr(), ws.data_ptr(), nbytes, _stream())
     _native.check(rc, "pdae_graph_feature_grad_f32")
     return gx
 
@@ -1112,8 +1168,15 @@ def group_points_grad(grad_out, idx, n):
     b, c, p, s = grad_out.shape
     with _on(grad_out.device):
         out = torch.empty((b, c, int(n)), dtype=torch.float32, device=grad_out.device)
-        rc = _native.lib().pdae_group_points_grad_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), p, s,
-                                                      out.data_ptr(), _stream())
+        L = _native.lib()
+        if _deterministic():
+            nbytes = L.pdae_group_points_grad_det_workspace_bytes(b, int(n), p, s)
+            ws = _workspace(nbytes, grad_out.device)
+            rc = L.pdae_group_points_grad_det_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), p, s, out.data_ptr(),
+                                                  ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_group_points_grad_f32(grad_out.data_ptr(), idx.data_ptr(), b, c, int(n), p, s, out.data_ptr(),
+                                              _stream())
     _native.check(rc, "pdae_group_points_grad_f32")
     return out
 
@@ -1165,7 +1228,14 @@ def three_interpolate_grad(grad_out, idx, weight, m):
     b, c, n = grad_out.shape
     with _on(grad_out.device):
         out = torch.empty((b, c, int(m)), dtype=torch.float32, device=grad_out.device)
-        rc = _native.lib().pdae_three_interpolate_grad_f32(grad_out.data_ptr(), idx.data_ptr(), weight.data_ptr(), b, c,
-                                                           n, int(m), out.data_ptr(), _stream())
+        L = _native.lib()
+        if _deterministic():
+            nbytes = L.pdae_three_interpolate_grad_det_workspace_bytes(b, n, int(m))
+            ws = _workspace(nbytes, grad_out.device)
+            rc = L.pdae_three_interpolate_grad_det_f32(grad_out.data_ptr(), idx.data_ptr(), weight.data_ptr(), b, c, n, int(m),
+                                                       out.data_ptr(), ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_three_interpolate_grad_f32(grad_out.data_ptr(), idx.data_ptr(), weight.data_ptr(), b, c, n, int(m),
+                                                   out.data_ptr(), _stream())
     _native.check(rc, "pdae_three_interpolate_grad_f32")
     return out
