@@ -459,6 +459,39 @@ int pdae_step_ex_f32(const float *cloud, const float *pred, int b, int n, int g,
                      float *gpred, float *gcloud, void *workspace, size_t workspace_bytes, unsigned flags,
                      pdae_stream_t stream);
 
+/* ---- Earth Mover's Distance (approxmatch / matchcost / matchcostgrad) -------------------------------------------
+ * replaces: the reference's extensions/emd (`emd_cuda`: approxmatch_forward, matchcost_forward, matchcost_backward;
+ *           Fan et al. 2017, tf_approxmatch_g.cu), which includes THC and does not build with current torch.
+ * xyz1 (b,n,3), xyz2 (b,m,3) fp32; 1 <= n, m <= 65536 (PDAE_E_UNSUPPORTED beyond).  Per cloud:
+ *   masses     n >= m: remainL = 1, remainR = n / m; else remainL = m / n, remainR = 1 (integer divisions)
+ *   levels     j = 0..9: level = -4^(7-j) for j < 9, 0 for j = 9; c_j = rn(level * 1.44269504f)
+ *   distance   d(k,l) = fma(dz,dz, fma(dy,dy, rn(dx*dx))), dx = x2_l - x1_k (rounded fp32 differences)
+ *   pair term  e = ex2.approx.ftz(rn(c_j * d))
+ *   pass 1     ratioL[k] = remainL[k] / s,  s = fma(e, remainR[l], s) for l ascending from s = 1e-9f
+ *   pass 2     t = fma(e, ratioL[k], t) for k ascending from +0; sumr = rn(t * remainR[l]);
+ *              ratioR[l] = rn(fminf(remainR[l] / (sumr + 1e-9f), 1) * remainR[l]); remainR[l] = fmaxf(0, remainR[l] - sumr)
+ *   pass 3     w(k,l) = rn(rn(e * ratioL[k]) * ratioR[l]); u = u + w for l ascending from +0; remainL[k] = fmaxf(0, remainL[k] - u)
+ *   match      match[l][k] = sum_j w_j(k,l) added in level order from +0, layout (b,m,n)
+ *   cost       rowcost[l] = fma(sqrtf(d), match[l][k], .) for k ascending from +0; then per cloud, thread t < 256 of
+ *              one CTA adds rowcost[t + 256 i] for ascending i from +0 and the 256 partials reduce as
+ *              p[t] = p[t] + p[t + s] for s = 128, 64, ..., 1; cost = p[0] (no normalisation)
+ *   gradient   match held constant: grad1[k] = rn(g_b * a), a = fma(rn(match[l][k] * rsqrtf(fmaxf(d, 1e-20))), x1_k - x2_l, a)
+ *              per coordinate for l ascending from +0; grad2[l] likewise over k ascending with x2_l - x1_k
+ * Every row and column sum is one sequential chain, so the results do not depend on the grid, the batch or the stream
+ * and need no atomics (bit-reproducible with or without torch.use_deterministic_algorithms).
+ * pdae_emd_match_f32 stores the per-level ratios ratio_l (b,10,n) and ratio_r (b,10,m) instead of the (b,m,n) match;
+ * `match` may be null, else the match is also written (one pass from the ratios, 64-bit offsets).  Cost and gradient
+ * read the caller's `match` when it is non-null (the ratios are then ignored and may be null) and rebuild it from the
+ * ratios, bit for bit, otherwise.  Workspace: pdae_emd_workspace_bytes (match and cost; the gradient needs none).     */
+size_t pdae_emd_workspace_bytes(int b, int n, int m);
+int pdae_emd_match_f32(const float *xyz1, const float *xyz2, int b, int n, int m, float *ratio_l, float *ratio_r, float *match,
+                       void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+int pdae_emd_cost_f32(const float *xyz1, const float *xyz2, int b, int n, int m, const float *match, const float *ratio_l,
+                      const float *ratio_r, float *cost, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+int pdae_emd_cost_grad_f32(const float *grad_cost, const float *xyz1, const float *xyz2, int b, int n, int m,
+                           const float *match, const float *ratio_l, const float *ratio_r, float *grad1, float *grad2,
+                           pdae_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -108,6 +108,10 @@ SIGNATURES = {
     "pdae_step_ex_workspace_bytes": (_sz, [_i, _i, _i, _i, ctypes.c_uint]),
     "pdae_step_ex_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
                               ctypes.c_uint, _vp]),
+    "pdae_emd_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_emd_match_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_emd_cost_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_emd_cost_grad_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

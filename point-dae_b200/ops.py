@@ -1239,3 +1239,89 @@ def three_interpolate_grad(grad_out, idx, weight, m):
                                                    out.data_ptr(), _stream())
     _native.check(rc, "pdae_three_interpolate_grad_f32")
     return out
+
+
+# ------------------------------------------------------------------- Earth Mover's Distance (approxmatch)
+EMD_LEVELS = 10
+
+
+def _emd_clouds(xyz1, xyz2, name):
+    for t, nm in ((xyz1, "xyz1"), (xyz2, "xyz2")):
+        _require_cuda(t, name)
+        _require_f32_contig(t, nm)
+        if t.dim() != 3 or t.size(2) != 3:
+            raise RuntimeError("%s must have shape (B, N, 3)" % nm)
+    _same_device(xyz1.device, xyz2=xyz2)
+    if xyz1.size(0) != xyz2.size(0):
+        raise RuntimeError("xyz1 and xyz2 disagree on the batch size")
+    return xyz1.shape[0], xyz1.shape[1], xyz2.shape[1]
+
+
+def _emd_inputs(xyz1, xyz2, name, match, ratio_l, ratio_r):
+    """checks the clouds and the match or ratios; -> (b, n, m, pointers of match / ratio_l / ratio_r or None)"""
+    b, n, m = _emd_clouds(xyz1, xyz2, name)
+    if match is not None:
+        _require_f32_contig(match, "match")
+        _same_device(xyz1.device, match=match)
+        if tuple(match.shape) != (b, m, n):
+            raise RuntimeError("match must have shape (B, m, n) = (%d, %d, %d)" % (b, m, n))
+        return b, n, m, (match.data_ptr(), None, None)
+    if ratio_l is None or ratio_r is None:
+        raise RuntimeError("%s needs either match or both ratios" % name)
+    for t, nm, cnt in ((ratio_l, "ratio_l", n), (ratio_r, "ratio_r", m)):
+        _require_f32_contig(t, nm)
+        _same_device(xyz1.device, **{nm: t})
+        if tuple(t.shape) != (b, EMD_LEVELS, cnt):
+            raise RuntimeError("%s must have shape (B, %d, %d)" % (nm, EMD_LEVELS, cnt))
+    return b, n, m, (None, ratio_l.data_ptr(), ratio_r.data_ptr())
+
+
+def emd_match(xyz1, xyz2, materialize=False):
+    """approxmatch of xyz1 (B,n,3) and xyz2 (B,m,3): -> (ratio_l (B,10,n), ratio_r (B,10,m), match (B,m,n) or None).
+    The per-level ratios determine the match; it is written only with materialize=True."""
+    b, n, m = _emd_clouds(xyz1, xyz2, "emd_match")
+    dev = xyz1.device
+    L = _native.lib()
+    with _on(dev):
+        ratio_l = torch.empty((b, EMD_LEVELS, n), dtype=torch.float32, device=dev)
+        ratio_r = torch.empty((b, EMD_LEVELS, m), dtype=torch.float32, device=dev)
+        match = torch.empty((b, m, n), dtype=torch.float32, device=dev) if materialize else None
+        nbytes = L.pdae_emd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_emd_match_f32(xyz1.data_ptr(), xyz2.data_ptr(), b, n, m, ratio_l.data_ptr(), ratio_r.data_ptr(),
+                                  match.data_ptr() if materialize else None, ws.data_ptr(), nbytes, _stream())
+    _native.check(rc, "pdae_emd_match_f32")
+    return ratio_l, ratio_r, match
+
+
+def emd_cost(xyz1, xyz2, match=None, ratio_l=None, ratio_r=None):
+    """matchcost: (B,) sum over pairs of |x1_k - x2_l| * match[l][k], the match given or rebuilt from the ratios."""
+    b, n, m, (pm, pl, pr) = _emd_inputs(xyz1, xyz2, "emd_cost", match, ratio_l, ratio_r)
+    dev = xyz1.device
+    L = _native.lib()
+    with _on(dev):
+        cost = torch.empty((b,), dtype=torch.float32, device=dev)
+        nbytes = L.pdae_emd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_emd_cost_f32(xyz1.data_ptr(), xyz2.data_ptr(), b, n, m, pm, pl, pr, cost.data_ptr(), ws.data_ptr(),
+                                 nbytes, _stream())
+    _native.check(rc, "pdae_emd_cost_f32")
+    return cost
+
+
+def emd_cost_grad(grad_cost, xyz1, xyz2, match=None, ratio_l=None, ratio_r=None):
+    """matchcost gradient with the match held constant: grad_cost (B,) -> (grad1 (B,n,3), grad2 (B,m,3))."""
+    b, n, m, (pm, pl, pr) = _emd_inputs(xyz1, xyz2, "emd_cost_grad", match, ratio_l, ratio_r)
+    _require_cuda(grad_cost, "emd_cost_grad")
+    _require_f32_contig(grad_cost, "grad_cost")
+    _same_device(xyz1.device, grad_cost=grad_cost)
+    if grad_cost.numel() != b:
+        raise RuntimeError("grad_cost must hold one value per cloud")
+    dev = xyz1.device
+    with _on(dev):
+        grad1 = torch.empty((b, n, 3), dtype=torch.float32, device=dev)
+        grad2 = torch.empty((b, m, 3), dtype=torch.float32, device=dev)
+        rc = _native.lib().pdae_emd_cost_grad_f32(grad_cost.data_ptr(), xyz1.data_ptr(), xyz2.data_ptr(), b, n, m, pm, pl,
+                                                  pr, grad1.data_ptr(), grad2.data_ptr(), _stream())
+    _native.check(rc, "pdae_emd_cost_grad_f32")
+    return grad1, grad2
