@@ -492,6 +492,40 @@ int pdae_emd_cost_grad_f32(const float *grad_cost, const float *xyz1, const floa
                            const float *match, const float *ratio_l, const float *ratio_r, float *grad1, float *grad2,
                            pdae_stream_t stream);
 
+/* ---- variable-size clouds in one batch: segment FPS and segment kNN (parity unpinned) --------------------------
+ * replaces: the reference's extensions/pointops (`pointops_cuda`: furthestsampling_cuda, knnquery_cuda; published
+ *           PointTransformer lib/pointops), which includes THC and does not build with current torch.  The reference
+ *           source is not in this tree: the semantics below restate the published kernels.
+ * Packed layout: xyz (n_total,3) fp32 holds the clouds back to back; offset (b,) int32 holds the cumulative ends,
+ * segment s = [offset[s-1], offset[s]) with offset[-1] = 0; new_offset (b,) likewise for samples / queries.  Offsets
+ * are device pointers and are only read on the device (no call synchronises with the host); they are expected to be
+ * non-decreasing and every value is clamped into [0, n_total] / [0, m_total], so no access leaves the tensors.
+ * Every index written is global (a row of the packed xyz).
+ * FPS (pdae_seg_fps_f32; idx (m_total,) int32, tmp (n_total,) fp32 or null):
+ *   first sample of segment s: idx[start_m] = start_n; sample j folds d = fma(dz,dz, fma(dx,dx, rn(dy*dy))),
+ *   dx = x_k - x_prev, into tmp[k] = fminf(d, tmp[k]) and takes the arg-max over the segment: a point counts when
+ *   tmp[k] > -1 (the reference's `d2 > best` from best = -1; there is no |p|^2 <= 1e-3 skip).  Ties go to the smallest
+ *   bitrev_lg(bs)((k - start_n) mod bs), then to the smaller k, bs = min(1024, 2^floor(log(n)/log(2))) (1 for n = 0).
+ *   `n` (the reference passes the largest segment size) sets the tie rule and the kernel form only: segments larger
+ *   than n are still exact.  tmp starts from the caller's contents (the reference fills 1e10) and on exit holds the
+ *   minima folded with every sample but the last; tmp = null starts from 1e10, writes nothing back and needs
+ *   pdae_seg_fps_workspace_bytes(n_total) of workspace.  A segment without points writes start_n for all of its
+ *   samples; a segment without samples writes nothing.  PDAE_E_UNSUPPORTED when n_total >> log2(bs) >= 2^22.
+ * kNN (pdae_seg_knn_f32; new_xyz (m,3), idx / dist2 (m, nsample) int32 / fp32, 1 <= nsample <= 100):
+ *   query p belongs to the first segment s with p < new_offset[s] and searches the points of that segment only;
+ *   d^2 = fma(dz,dz, fma(dy,dy, rn(dx*dx))), dx = x_k - x_p (the rounding of pdae_knn_f32).  The row holds the
+ *   nsample smallest (d^2, index) pairs with d^2 < 1e10, ascending; the rest of the row is (1e10, start_n).  (The
+ *   reference's heap can resolve exact ties at the k-th distance differently; this order is the definition here.)
+ *   Rows p >= max(new_offset) hold idx -1 and dist2 1e10.  Workspace: pdae_seg_knn_workspace_bytes(b, m).
+ * No atomics: the results depend on the inputs only, not on the launch shape or the stream.                      */
+size_t pdae_seg_fps_workspace_bytes(int n_total);
+int pdae_seg_fps_f32(const float *xyz, int n_total, const int *offset, const int *new_offset, int b, int n, int m_total,
+                     float *tmp, int *idx, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_seg_knn_workspace_bytes(int b, int m);
+int pdae_seg_knn_f32(const float *xyz, int n_total, const float *new_xyz, int m, const int *offset, const int *new_offset,
+                     int b, int nsample, int *idx, float *dist2, void *workspace, size_t workspace_bytes,
+                     pdae_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -112,6 +112,10 @@ SIGNATURES = {
     "pdae_emd_match_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pdae_emd_cost_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pdae_emd_cost_grad_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pdae_seg_fps_workspace_bytes": (_sz, [_i]),
+    "pdae_seg_fps_f32": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_knn_workspace_bytes": (_sz, [_i, _i]),
+    "pdae_seg_knn_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib = None

@@ -32,24 +32,6 @@ namespace cg = cooperative_groups;
 
 namespace pdae {
 
-// block-wide arg-max of (value bits, rank): returns the winning rank in every thread.
-template <int T>
-__device__ __forceinline__ unsigned fps_block_argmax(unsigned vb, unsigned rank, uint2 *slots /*[2][32]*/, int it) {
-  constexpr int W = T / 32;
-  const unsigned full = 0xffffffffu;
-  unsigned m = __reduce_max_sync(full, vb);
-  unsigned r = __reduce_min_sync(full, vb == m ? rank : 0xffffffffu);
-  if (W == 1) return r;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint2 *buf = slots + (it & 1) * 32;
-  if (lane == 0) buf[warp] = make_uint2(m, r);
-  __syncthreads();
-  const uint2 v = lane < W ? buf[lane] : make_uint2(0u, 0xffffffffu);
-  m = __reduce_max_sync(full, v.x);
-  r = __reduce_min_sync(full, v.x == m ? v.y : 0xffffffffu);
-  return r;
-}
-
 // block-wide arg-max for the register-resident kernel: per-warp winners are posted as ONE 64-bit key
 // (value bits << 32 | ~rank: larger value first, then smaller rank) and every thread folds the W keys with a
 // register tree after the barrier -- two broadcast LDS.128 and log2(W) dependent 64-bit max instead of a second pair

@@ -1,5 +1,5 @@
-// fps_rank.cuh -- value / tie-rank encodings of the furthest-point-sampling arg-max, shared by fps.cu and the fused
-// patchifier (patchify.cu).  Reference rule: extensions/pointnet2/_ext_src/src/sampling_gpu.cu:72-176.
+// fps_rank.cuh -- value / tie-rank encodings of the furthest-point-sampling arg-max, shared by fps.cu, the fused
+// patchifier (patchify.cu) and the segment FPS (pointops.cu).  Reference rule: extensions/pointnet2/_ext_src/src/sampling_gpu.cu:72-176.
 #pragma once
 #include "common.cuh"
 
@@ -19,6 +19,24 @@ __device__ __forceinline__ int fps_unrank(unsigned r, int lg_bs) {
   const unsigned rev = r >> 22, hi = r & 0x3fffffu;
   const unsigned slot = lg_bs ? (__brev(rev) >> (32 - lg_bs)) : 0u;
   return static_cast<int>((hi << lg_bs) | slot);
+}
+
+// block-wide arg-max of (value bits, rank): returns the winning rank in every thread.
+template <int T>
+__device__ __forceinline__ unsigned fps_block_argmax(unsigned vb, unsigned rank, uint2 *slots /*[2][32]*/, int it) {
+  constexpr int W = T / 32;
+  const unsigned full = 0xffffffffu;
+  unsigned m = __reduce_max_sync(full, vb);
+  unsigned r = __reduce_min_sync(full, vb == m ? rank : 0xffffffffu);
+  if (W == 1) return r;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  uint2 *buf = slots + (it & 1) * 32;
+  if (lane == 0) buf[warp] = make_uint2(m, r);
+  __syncthreads();
+  const uint2 v = lane < W ? buf[lane] : make_uint2(0u, 0xffffffffu);
+  m = __reduce_max_sync(full, v.x);
+  r = __reduce_min_sync(full, v.x == m ? v.y : 0xffffffffu);
+  return r;
 }
 
 // register i of a thread  ->  which of the thread's points (k = tid + p*T) it holds

@@ -3,7 +3,7 @@ main.py run unchanged:
 
     import pointdae_b200; pointdae_b200.install()
     # now: from pointnet2_ops import pointnet2_utils (and pointnet2_ops.pointnet2_modules) ; from knn_cuda import KNN ; import chamfer ;
-    #      import pointnet2._ext ; import emd_cuda  -> all served by the sm_100a kernels
+    #      import pointnet2._ext ; import emd_cuda ; import pointops_cuda  -> all served by the sm_100a kernels
 
 Only the *compiled / third-party* modules are replaced (the reference's own Python, e.g.
 extensions/chamfer_dist/__init__.py, keeps running on top).  `patch_models()` additionally rebinds
@@ -18,7 +18,7 @@ import types
 def install(loss_modules=False):
     """loss_modules=True additionally serves `extensions.chamfer_dist` (the reference's Python loss classes,
     which import `ipdb` at module level, extensions/chamfer_dist/__init__.py:12) from this package's mirror."""
-    from . import chamfer, emd_cuda, knn_cuda, pointnet2_ext, pointnet2_modules, pointnet2_utils
+    from . import chamfer, emd_cuda, knn_cuda, pointnet2_ext, pointnet2_modules, pointnet2_utils, pointops_cuda
 
     pkg = types.ModuleType("pointnet2_ops")
     pkg.__path__ = []  # mark as package
@@ -32,6 +32,7 @@ def install(loss_modules=False):
     sys.modules["knn_cuda"] = knn_cuda
     sys.modules["chamfer"] = chamfer
     sys.modules["emd_cuda"] = emd_cuda  # extensions/emd's compiled module
+    sys.modules["pointops_cuda"] = pointops_cuda  # extensions/pointops' compiled module
 
     # `import pointnet2._ext as _ext` (extensions/pointnet2/pointnet2_utils.py:23-24)
     p2 = sys.modules.get("pointnet2")

@@ -1325,3 +1325,101 @@ def emd_cost_grad(grad_cost, xyz1, xyz2, match=None, ratio_l=None, ratio_r=None)
                                                   pr, grad1.data_ptr(), grad2.data_ptr(), _stream())
     _native.check(rc, "pdae_emd_cost_grad_f32")
     return grad1, grad2
+
+
+# ------------------------------------------------- variable-size clouds in one batch (the reference's pointops)
+def _segment_inputs(xyz, offset, new_offset, name):
+    _require_cuda(xyz, name)
+    _require_f32_contig(xyz, "xyz")
+    if xyz.dim() != 2 or xyz.size(1) != 3:
+        raise RuntimeError("xyz must have shape (N, 3)")
+    for t, nm in ((offset, "offset"), (new_offset, "new_offset")):
+        _require_i32_contig(t, nm)
+        if t.dim() != 1:
+            raise RuntimeError("%s must have shape (b,)" % nm)
+    _same_device(xyz.device, offset=offset, new_offset=new_offset)
+    if offset.numel() != new_offset.numel():
+        raise RuntimeError("offset and new_offset disagree on the number of segments")
+    return offset.numel()
+
+
+def segment_fps_into(xyz, offset, new_offset, n, idx, tmp=None):
+    """The compiled pointops FPS: writes the global sample indices of every segment into idx (M,) int32 and, when tmp
+    (N,) fp32 is given, starts from and leaves the running minima there.  n (the largest segment size) sets the tie
+    rule; segments larger than n are still exact.  No host synchronisation."""
+    b = _segment_inputs(xyz, offset, new_offset, "furthestsampling")
+    _require_i32_contig(idx, "idx")
+    _same_device(xyz.device, idx=idx, tmp=tmp)
+    if tmp is not None:
+        _require_f32_contig(tmp, "tmp")
+        if tmp.numel() < xyz.size(0):
+            raise RuntimeError("tmp must hold one value per point")
+    n_total = xyz.size(0)
+    L = _native.lib()
+    with _on(xyz.device):
+        nbytes = L.pdae_seg_fps_workspace_bytes(n_total) if tmp is None else 0
+        ws = _workspace(nbytes, xyz.device) if nbytes else None
+        rc = L.pdae_seg_fps_f32(xyz.data_ptr(), n_total, offset.data_ptr(), new_offset.data_ptr(), b, int(n), idx.numel(),
+                                tmp.data_ptr() if tmp is not None else None, idx.data_ptr(),
+                                ws.data_ptr() if ws is not None else None, nbytes, _stream())
+    _native.check(rc, "pdae_seg_fps_f32")
+    return idx
+
+
+def segment_fps(xyz, offset, new_offset, n=None, m=None):
+    """Furthest point sampling of every segment of a packed batch: xyz (N,3) f32, offset / new_offset (b,) int32
+    cumulative ends of the points / samples -> idx (m,) int32 of global indices, m = new_offset[-1].
+
+    n is the largest segment size (it sets the reference's tie rule) and m the number of samples.  Each one left as None
+    is computed from the offsets on the host: this is the one host read of the call (one copy for both).  Pass both to
+    keep the call free of synchronisation, e.g. inside a CUDA graph."""
+    b = _segment_inputs(xyz, offset, new_offset, "segment_fps")
+    if b == 0:
+        return torch.empty((0 if m is None else int(m),), dtype=torch.int32, device=xyz.device)
+    if n is None or m is None:
+        with _on(xyz.device):
+            sizes = torch.diff(offset, prepend=offset.new_zeros(1))
+            n_read, m_read = torch.stack((sizes.max(), new_offset[-1])).tolist()
+        n = n_read if n is None else n
+        m = m_read if m is None else m
+    with _on(xyz.device):
+        idx = torch.empty((max(int(m), 0),), dtype=torch.int32, device=xyz.device)
+    return segment_fps_into(xyz, offset, new_offset, max(int(n), 0), idx)
+
+
+def segment_knn_into(nsample, xyz, new_xyz, offset, new_offset, idx, dist2):
+    """The compiled pointops kNN query: writes idx (m, nsample) int32 and dist2 (m, nsample) fp32 (squared)."""
+    b = _segment_inputs(xyz, offset, new_offset, "knnquery")
+    _require_cuda(new_xyz, "knnquery")
+    _require_f32_contig(new_xyz, "new_xyz")
+    if new_xyz.dim() != 2 or new_xyz.size(1) != 3:
+        raise RuntimeError("new_xyz must have shape (M, 3)")
+    nsample = int(nsample)
+    if not 1 <= nsample <= 100:
+        raise RuntimeError("nsample=%d must satisfy 1 <= nsample <= 100" % nsample)
+    m = new_xyz.size(0)
+    _require_i32_contig(idx, "idx")
+    _require_f32_contig(dist2, "dist2")
+    _same_device(xyz.device, new_xyz=new_xyz, idx=idx, dist2=dist2)
+    if idx.numel() != m * nsample or dist2.numel() != m * nsample:
+        raise RuntimeError("idx and dist2 must hold (M, nsample) = (%d, %d) elements" % (m, nsample))
+    L = _native.lib()
+    with _on(xyz.device):
+        nbytes = L.pdae_seg_knn_workspace_bytes(b, m)
+        ws = _workspace(nbytes, xyz.device)
+        rc = L.pdae_seg_knn_f32(xyz.data_ptr(), xyz.size(0), new_xyz.data_ptr(), m, offset.data_ptr(), new_offset.data_ptr(),
+                                b, nsample, idx.data_ptr(), dist2.data_ptr(), ws.data_ptr(), nbytes, _stream())
+    _native.check(rc, "pdae_seg_knn_f32")
+    return idx, dist2
+
+
+def segment_knn(nsample, xyz, new_xyz, offset, new_offset):
+    """kNN of every query among the points of its own segment: xyz (N,3), new_xyz (M,3) f32, offset / new_offset (b,)
+    int32 cumulative ends -> (idx (M,nsample) int32 global indices, dist2 (M,nsample) f32 squared distances), ascending
+    by (distance, index).  Slots no point fills hold (start of the segment, 1e10); rows past new_offset[-1] hold
+    (-1, 1e10).  1 <= nsample <= 100.  No host synchronisation."""
+    m = new_xyz.size(0)
+    with _on(xyz.device):
+        idx = torch.empty((m, int(nsample)), dtype=torch.int32, device=xyz.device)
+        dist2 = torch.empty((m, int(nsample)), dtype=torch.float32, device=xyz.device)
+    return segment_knn_into(nsample, xyz, new_xyz, offset, new_offset, idx, dist2)
