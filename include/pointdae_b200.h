@@ -221,10 +221,18 @@ int pdae_conv1x1_tf32x3_f32(const float *x, const float *w, const float *bias, i
  *   pdae_edge_backward_f32  partial != NULL: per-CTA partial sums of dbeta / dgamma from g (b,n,co), the upstream
  *                           gradient point-major.  dz != NULL: dz (b,n,ld) = [dP | dQ], zero-filled by the caller
  *                           (dP is scatter-added); train = 1 adds the two per-channel terms training-mode BatchNorm
- *                           spreads over every edge (ca, cb = gamma dbeta / M, gamma dgamma / M, M = b n k).      */
+ *                           spreads over every edge (ca, cb = gamma dbeta / M, gamma dgamma / M, M = b n k).
+ *                           LeakyReLU's derivative is 1 where the BatchNorm output is > 0 and the slope elsewhere, at 0
+ *                           too (torch's convention); the same in the two-phase backward below.                    */
 size_t pdae_edge_partial_count(int b, int n);
 int pdae_edge_stats_f64(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co, double *partial, float *s1,
                         pdae_stream_t stream);  /* s1 (b,n,co) or NULL: sum_j P[idx(i,j)], kept for the backward */
+/* The same sums of v = y - c_o instead of y, c_o = P[0][o] + Q[0][o] of cloud 0 rounded to fp32 (one sample of the
+ * channel); s1 unchanged.  sum y^2 / M - mean^2 loses the digits a channel's mean has above its spread; the shifted sums
+ * keep the statistics at the accuracy of P and Q themselves (what ops.edge_conv uses; finish with
+ * pdae_edge_bn_prepare_shifted_f32 on the same z).                                                                    */
+int pdae_edge_stats_shifted_f64(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co, double *partial,
+                                float *s1, pdae_stream_t stream);
 int pdae_edge_forward_f32(const float *z, int ld, const int64_t *idx, const float *scale, const float *shift, float slope,
                           int b, int n, int k, int co, float *out, unsigned char *jstar, pdae_stream_t stream);
 int pdae_edge_backward_f32(const float *z, int ld, const int64_t *idx, const unsigned char *jstar, const float *g,
@@ -325,6 +333,11 @@ int pdae_edge_backward_dense_f32(const float *z, int ld, const int64_t *idx, con
 int pdae_edge_bn_prepare_f32(const double *partial, int np, int co, double m, const float *gamma, const float *beta,
                              float *running_mean, float *running_var, float momentum, float eps, int train, float *mean,
                              float *invstd, float *scale, float *shift, pdae_stream_t stream);
+/* partial sums of pdae_edge_stats_shifted_f64: mean = c_o + sum v / M with c_o read from z (b,n,ld), variance
+ * sum v^2 / M - (sum v / M)^2.  z may be NULL when train = 0.                                                         */
+int pdae_edge_bn_prepare_shifted_f32(const double *partial, int np, int co, double m, const float *z, int ld, const float *gamma,
+                                     const float *beta, float *running_mean, float *running_var, float momentum, float eps,
+                                     int train, float *mean, float *invstd, float *scale, float *shift, pdae_stream_t stream);
 int pdae_edge_bn_backward_f32(const double *partial, int np, int co, double m, const float *gamma, float *dgamma, float *dbeta,
                               float *ca, float *cb, pdae_stream_t stream);
 

@@ -59,6 +59,9 @@ SIGNATURES = {
     "pdae_edge_partial_count": (_sz, [_i, _i]),
     "pdae_edge_stats_f64": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pdae_edge_bn_prepare_f32": (_i, [_vp, _i, _i, ctypes.c_double, _vp, _vp, _vp, _vp, _f, _f, _i, _vp, _vp, _vp, _vp, _vp]),
+    "pdae_edge_stats_shifted_f64": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "pdae_edge_bn_prepare_shifted_f32": (_i, [_vp, _i, _i, ctypes.c_double, _vp, _i, _vp, _vp, _vp, _vp, _f, _f, _i, _vp, _vp, _vp,
+                                              _vp, _vp]),
     "pdae_edge_bn_backward_f32": (_i, [_vp, _i, _i, ctypes.c_double, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pdae_edge_reverse_workspace_ints": (_sz, [_i, _i, _i]),
     "pdae_edge_backward_select_f32": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp]),

@@ -141,6 +141,12 @@ __device__ __forceinline__ void edge_block_sums_to_global(double (&a)[EC_CHUNK /
   __syncthreads();
 }
 
+// SHIFTED: the sums are of v = y - c_o instead of y, c_o = P[0][o] + Q[0][o] of cloud 0 (fp32, one sample of the
+// channel).  sum y^2 / M - mean^2 cancels most significant digits when a channel's mean is large against its spread
+// (5.4e-5 relative error of invstd for a unit cloud shifted by 20, measured on B200); the shifted sums keep that error
+// at the rounding of P and Q themselves.  Per point the kernel forms q_i - c_o once; sum_j v = s1 + k (q_i - c_o),
+// sum_j v^2 costs one more FADD per edge and channel.
+template <bool SHIFTED>
 __global__ void __launch_bounds__(EC_WARPS * 32) edge_stats_kernel(const EdgeArgs a, double *__restrict__ partial,
                                                                    float *__restrict__ s1_out /*(b, n, co) or NULL*/) {
   __shared__ double sm[2 * EC_CHUNK];
@@ -155,18 +161,25 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_stats_kernel(const EdgeArg
     for (int e = threadIdx.x; e < 2 * EC_CHUNK; e += EC_WARPS * 32) sm[e] = 0.0;
     __syncthreads();
     double t1[PER_LANE], t2[PER_LANE];
+    float cz[PER_LANE];  // c_o of the shifted form, read once per channel pass
 #pragma unroll
-    for (int u = 0; u < PER_LANE; ++u) t1[u] = 0.0, t2[u] = 0.0;
+    for (int u = 0; u < PER_LANE; ++u) {
+      t1[u] = 0.0, t2[u] = 0.0;
+      const int o = c0 + u * 32 + lane, oc = o < co ? o : co - 1;
+      cz[u] = SHIFTED ? __fadd_rn(__ldg(a.z + oc), __ldg(a.z + co + oc)) : 0.f;
+    }
     for (int pw = 0; pw < PER_WARP; ++pw) {
       const int i = i0 + warp * PER_WARP + pw;
       if (i >= n) continue;  // warp-uniform
       float s1[PER_LANE], s2[PER_LANE];
       int oc[PER_LANE];
+      float qs[PER_LANE];  // q_i - c_o (shifted) or 0: v = p + qs
 #pragma unroll
       for (int u = 0; u < PER_LANE; ++u) {
         s1[u] = 0.f, s2[u] = 0.f;
         const int o = c0 + u * 32 + lane;
         oc[u] = o < co ? o : co - 1;
+        qs[u] = SHIFTED ? __fsub_rn(__ldg(Z + static_cast<size_t>(i) * ld + co + oc[u]), cz[u]) : 0.f;
       }
       const int64_t *ip = Ic + static_cast<size_t>(i) * k;
       int j = 0;
@@ -184,7 +197,8 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_stats_kernel(const EdgeArg
 #pragma unroll
           for (int u = 0; u < PER_LANE; ++u) {
             s1[u] += pv[t][u];
-            s2[u] = fmaf(pv[t][u], pv[t][u], s2[u]);
+            const float v = SHIFTED ? __fadd_rn(pv[t][u], qs[u]) : pv[t][u];
+            s2[u] = fmaf(v, v, s2[u]);
           }
       }
       for (; j < k; ++j) {
@@ -193,7 +207,8 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_stats_kernel(const EdgeArg
         for (int u = 0; u < PER_LANE; ++u) {
           const float p = __ldg(Z + row + oc[u]);
           s1[u] += p;
-          s2[u] = fmaf(p, p, s2[u]);
+          const float v = SHIFTED ? __fadd_rn(p, qs[u]) : p;
+          s2[u] = fmaf(v, v, s2[u]);
         }
       }
 #pragma unroll
@@ -201,9 +216,14 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_stats_kernel(const EdgeArg
         const int o = c0 + u * 32 + lane;
         if (o < co) {
           if (s1_out) s1_out[(cloud * n + i) * co + o] = s1[u];  // sum_j P[idx(i,j)]: the backward's dQ needs it
-          const double q = static_cast<double>(__ldg(Z + static_cast<size_t>(i) * ld + co + o));
-          t1[u] += static_cast<double>(s1[u]) + kf * q;
-          t2[u] += static_cast<double>(s2[u]) + 2.0 * q * static_cast<double>(s1[u]) + kf * q * q;
+          if (SHIFTED) {
+            t1[u] += static_cast<double>(s1[u]) + kf * static_cast<double>(qs[u]);
+            t2[u] += static_cast<double>(s2[u]);
+          } else {
+            const double q = static_cast<double>(__ldg(Z + static_cast<size_t>(i) * ld + co + o));
+            t1[u] += static_cast<double>(s1[u]) + kf * q;
+            t2[u] += static_cast<double>(s2[u]) + 2.0 * q * static_cast<double>(s1[u]) + kf * q * q;
+          }
         }
       }
     }
@@ -338,7 +358,7 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_backward_reduce_kernel(con
           const size_t row = static_cast<size_t>(__ldg(Ic + static_cast<size_t>(i) * k + js)) * ld;
           const float y = __fadd_rn(__ldg(Z + row + o), __ldg(Z + static_cast<size_t>(i) * ld + co + o));
           const float bn = __fmaf_rn(__ldg(w.scale + o), y, __ldg(w.shift + o));
-          const float dbn = __ldg(w.g + e) * (bn >= 0.0f ? 1.0f : w.slope);
+          const float dbn = __ldg(w.g + e) * (bn > 0.0f ? 1.0f : w.slope);
           const float yhat = (y - __ldg(w.mean + o)) * __ldg(w.invstd + o);
           t1[u] += static_cast<double>(dbn);
           t2[u] += static_cast<double>(dbn) * static_cast<double>(yhat);
@@ -390,7 +410,7 @@ __global__ void __launch_bounds__(EC_WARPS * 32) edge_backward_kernel(const Edge
           const size_t row = static_cast<size_t>(__ldg(Ic + static_cast<size_t>(i) * k + js[u])) * ld;
           const float y = __fadd_rn(__ldg(Z + row + o), q[u]);
           const float bn = __fmaf_rn(sc[u], y, sh[u]);
-          dsel[u] = ga[u] * (__ldg(w.g + e) * (bn >= 0.0f ? 1.0f : w.slope));  // gamma * dbn on the selected edge
+          dsel[u] = ga[u] * (__ldg(w.g + e) * (bn > 0.0f ? 1.0f : w.slope));  // gamma * dbn on the selected edge
         }
       }
       if (w.train) {
@@ -440,16 +460,30 @@ extern "C" size_t pdae_edge_partial_count(int b, int n) {
   return b <= 0 || n <= 0 ? 0 : static_cast<size_t>(b) * ((n + EC_POINTS - 1) / EC_POINTS);
 }
 
-extern "C" int pdae_edge_stats_f64(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co, double *partial,
-                                   float *s1, pdae_stream_t stream) {
+static int edge_stats_launch(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co, int shifted,
+                             double *partial, float *s1, pdae_stream_t stream) {
   const int rc = edge_check(z, idx, b, n, k, co, ld);
   if (rc) return rc;
   if (b == 0 || n == 0) return 0;
   if (!partial) return PDAE_E_INVALID;
   const dim3 grid(static_cast<unsigned>((n + EC_POINTS - 1) / EC_POINTS), static_cast<unsigned>(b));
-  edge_stats_kernel<<<grid, EC_WARPS * 32, 0, static_cast<cudaStream_t>(stream)>>>(EdgeArgs{z, idx, ld, n, k, co}, partial, s1);
+  const EdgeArgs a{z, idx, ld, n, k, co};
+  if (shifted)
+    edge_stats_kernel<true><<<grid, EC_WARPS * 32, 0, static_cast<cudaStream_t>(stream)>>>(a, partial, s1);
+  else
+    edge_stats_kernel<false><<<grid, EC_WARPS * 32, 0, static_cast<cudaStream_t>(stream)>>>(a, partial, s1);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
+}
+
+extern "C" int pdae_edge_stats_f64(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co, double *partial,
+                                   float *s1, pdae_stream_t stream) {
+  return edge_stats_launch(z, ld, idx, b, n, k, co, 0, partial, s1, stream);
+}
+
+extern "C" int pdae_edge_stats_shifted_f64(const float *z, int ld, const int64_t *idx, int b, int n, int k, int co,
+                                           double *partial, float *s1, pdae_stream_t stream) {
+  return edge_stats_launch(z, ld, idx, b, n, k, co, 1, partial, s1, stream);
 }
 
 extern "C" int pdae_edge_forward_f32(const float *z, int ld, const int64_t *idx, const float *scale, const float *shift,
@@ -614,7 +648,9 @@ namespace pdae {
 
 // partial (np, co, 2) fp64 -> batch mean / biased variance -> invstd, folded scale / shift; running buffers updated like
 // nn.BatchNorm2d (momentum, unbiased variance).  train = 0: the statistics are the running buffers.
+// zc != NULL: the partial sums are of y - c_o (pdae_edge_stats_shifted_f64), c_o = zc[o] + zc[co + o] in fp32.
 __global__ void __launch_bounds__(128) edge_bn_prepare_kernel(const double *__restrict__ partial, int np, int co, double m,
+                                                              const float *__restrict__ zc,
                                                               const float *__restrict__ gamma, const float *__restrict__ beta,
                                                               float *running_mean, float *running_var, float momentum, float eps,
                                                               int train, float *__restrict__ mean, float *__restrict__ invstd,
@@ -628,9 +664,10 @@ __global__ void __launch_bounds__(128) edge_bn_prepare_kernel(const double *__re
       s1 += partial[(static_cast<size_t>(p) * co + o) * 2];
       s2 += partial[(static_cast<size_t>(p) * co + o) * 2 + 1];
     }
-    const double mean64 = s1 / m;
-    double var64 = s2 / m - mean64 * mean64;
+    const double d64 = s1 / m;  // mean of the summed values
+    double var64 = s2 / m - d64 * d64;
     var64 = var64 > 0.0 ? var64 : 0.0;
+    const double mean64 = zc ? static_cast<double>(__fadd_rn(zc[o], zc[co + o])) + d64 : d64;
     if (running_mean) {
       running_mean[o] = (1.0f - momentum) * running_mean[o] + momentum * static_cast<float>(mean64);
       running_var[o] = (1.0f - momentum) * running_var[o] + momentum * static_cast<float>(var64 * (m / (m > 1.0 ? m - 1.0 : 1.0)));
@@ -665,17 +702,34 @@ __global__ void __launch_bounds__(128) edge_bn_backward_kernel(const double *__r
 
 }  // namespace pdae
 
-extern "C" int pdae_edge_bn_prepare_f32(const double *partial, int np, int co, double m, const float *gamma, const float *beta,
-                                        float *running_mean, float *running_var, float momentum, float eps, int train,
-                                        float *mean, float *invstd, float *scale, float *shift, pdae_stream_t stream) {
+static int edge_bn_prepare_launch(const double *partial, int np, int co, double m, const float *zc, const float *gamma,
+                                  const float *beta, float *running_mean, float *running_var, float momentum, float eps, int train,
+                                  float *mean, float *invstd, float *scale, float *shift, pdae_stream_t stream) {
   if (co <= 0 || np < 0 || !mean || !invstd || !scale || !shift) return PDAE_E_INVALID;
   if (train && (!partial || np == 0 || m <= 0)) return PDAE_E_INVALID;
   if (!train && (!running_mean || !running_var)) return PDAE_E_INVALID;
-  edge_bn_prepare_kernel<<<(co + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(partial, np, co, m, gamma, beta, running_mean,
-                                                                                        running_var, momentum, eps, train, mean,
-                                                                                        invstd, scale, shift);
+  edge_bn_prepare_kernel<<<(co + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(partial, np, co, m, train ? zc : nullptr,
+                                                                                        gamma, beta, running_mean, running_var,
+                                                                                        momentum, eps, train, mean, invstd,
+                                                                                        scale, shift);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
+}
+
+extern "C" int pdae_edge_bn_prepare_f32(const double *partial, int np, int co, double m, const float *gamma, const float *beta,
+                                        float *running_mean, float *running_var, float momentum, float eps, int train,
+                                        float *mean, float *invstd, float *scale, float *shift, pdae_stream_t stream) {
+  return edge_bn_prepare_launch(partial, np, co, m, nullptr, gamma, beta, running_mean, running_var, momentum, eps, train, mean,
+                                invstd, scale, shift, stream);
+}
+
+extern "C" int pdae_edge_bn_prepare_shifted_f32(const double *partial, int np, int co, double m, const float *z, int ld,
+                                                const float *gamma, const float *beta, float *running_mean, float *running_var,
+                                                float momentum, float eps, int train, float *mean, float *invstd, float *scale,
+                                                float *shift, pdae_stream_t stream) {
+  if (train && (!z || ld < 2 * co)) return PDAE_E_INVALID;
+  return edge_bn_prepare_launch(partial, np, co, m, z, gamma, beta, running_mean, running_var, momentum, eps, train, mean, invstd,
+                                scale, shift, stream);
 }
 
 extern "C" int pdae_edge_bn_backward_f32(const double *partial, int np, int co, double m, const float *gamma, float *dgamma,

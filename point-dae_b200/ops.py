@@ -919,18 +919,17 @@ def _edge_dims(z, idx, co):
 
 
 def edge_stats(z, idx, co, want_s1=False):
-    """Sum and sum of squares per output channel of y[i][j] = P[idx(i,j)] + Q[i] over all edges of the batch, from the
-    point-major product z = [P | Q] (B,N,2*co): float64 (co, 2) (+ s1 (B,N,co) = sum_j P[idx(i,j)] for the backward)."""
+    """Batch mean and biased variance per output channel of y[i][j] = P[idx(i,j)] + Q[i] over all edges of the batch,
+    from the point-major product z = [P | Q] (B,N,2*co): float64 (co, 2) = [mean | var] (+ s1 (B,N,co) =
+    sum_j P[idx(i,j)] for the backward).  The kernel sums y - c_o, c_o = P[0][0] + Q[0][0] (fp32), so a mean far from 0
+    costs no accuracy."""
     b, n, ld, k = _edge_dims(z, idx, co)
-    L = _native.lib()
     with _on(z.device):
-        partial = torch.empty((int(L.pdae_edge_partial_count(b, n)), co, 2), dtype=torch.float64, device=z.device)
-        s1 = torch.empty((b, n, co), dtype=torch.float32, device=z.device) if want_s1 else None
-        rc = L.pdae_edge_stats_f64(z.data_ptr(), ld, idx.data_ptr(), b, n, k, co, partial.data_ptr(),
-                                   s1.data_ptr() if want_s1 else None, _stream())
-    _native.check(rc, "pdae_edge_stats_f64")
-    sums = partial.sum(dim=0)  # fixed order: deterministic
-    return (sums, s1) if want_s1 else sums
+        partial, s1 = _edge_partials(z, idx, co, want_s1)
+        sums = partial.sum(dim=0) / (float(b) * n * k)  # fixed order: deterministic
+        centre = (z[0, 0, :co] + z[0, 0, co:2 * co]).double()
+        stats = torch.stack([centre + sums[:, 0], (sums[:, 1] - sums[:, 0] ** 2).clamp_min(0.0)], dim=1)
+    return (stats, s1) if want_s1 else stats
 
 
 def edge_forward(z, idx, co, scale, shift, slope=0.2, want_jstar=False):
@@ -990,14 +989,15 @@ def edge_backward(z, idx, co, jstar, g_pm, scale, shift, mean, invstd, gamma, sl
 
 
 def _edge_partials(z, idx, co, want_s1):
-    """raw per-CTA partial sums of the statistics kernel (summed inside pdae_edge_bn_prepare_f32)"""
+    """raw per-CTA partial sums of y - c_o from the shifted statistics kernel (summed inside
+    pdae_edge_bn_prepare_shifted_f32)"""
     b, n, ld, k = _edge_dims(z, idx, co)
     L = _native.lib()
     partial = torch.empty((int(L.pdae_edge_partial_count(b, n)), co, 2), dtype=torch.float64, device=z.device)
     s1 = torch.empty((b, n, co), dtype=torch.float32, device=z.device) if want_s1 else None
-    rc = L.pdae_edge_stats_f64(z.data_ptr(), ld, idx.data_ptr(), b, n, k, co, partial.data_ptr(),
-                               s1.data_ptr() if want_s1 else None, _stream())
-    _native.check(rc, "pdae_edge_stats_f64")
+    rc = L.pdae_edge_stats_shifted_f64(z.data_ptr(), ld, idx.data_ptr(), b, n, k, co, partial.data_ptr(),
+                                       s1.data_ptr() if want_s1 else None, _stream())
+    _native.check(rc, "pdae_edge_stats_shifted_f64")
     return partial, s1
 
 
@@ -1023,13 +1023,14 @@ class EdgeConvFunction(torch.autograd.Function):
                 partial, s1 = _edge_partials(z, idx, co, need_grad)
             stats = torch.empty((4, co), dtype=torch.float32, device=x.device)  # mean | invstd | scale | shift
             gamma_c, beta_c = gamma.contiguous(), beta.contiguous()
-            rc = L.pdae_edge_bn_prepare_f32(partial.data_ptr() if training else None, partial.size(0) if training else 0, co,
-                                            float(b) * n * k, gamma_c.data_ptr(), beta_c.data_ptr(),
-                                            running_mean.data_ptr() if running_mean is not None else None,
-                                            running_var.data_ptr() if running_var is not None else None, float(momentum),
-                                            float(eps), 1 if training else 0, stats[0].data_ptr(), stats[1].data_ptr(),
-                                            stats[2].data_ptr(), stats[3].data_ptr(), _stream())
-            _native.check(rc, "pdae_edge_bn_prepare_f32")
+            rc = L.pdae_edge_bn_prepare_shifted_f32(partial.data_ptr() if training else None, partial.size(0) if training else 0,
+                                                    co, float(b) * n * k, z.data_ptr(), z.size(2), gamma_c.data_ptr(),
+                                                    beta_c.data_ptr(),
+                                                    running_mean.data_ptr() if running_mean is not None else None,
+                                                    running_var.data_ptr() if running_var is not None else None,
+                                                    float(momentum), float(eps), 1 if training else 0, stats[0].data_ptr(),
+                                                    stats[1].data_ptr(), stats[2].data_ptr(), stats[3].data_ptr(), _stream())
+            _native.check(rc, "pdae_edge_bn_prepare_shifted_f32")
             out, jstar = edge_forward(z, idx, co, stats[2], stats[3], slope, want_jstar=need_grad)
         if need_grad:
             ctx.save_for_backward(x, idx, wz, z, jstar, stats, gamma_c, s1)

@@ -155,10 +155,9 @@ def test_both_training_backward_forms_agree():
     idx = dgcnn_util.knn(x, k)
     wz = torch.randn(2 * co, c, device=DEV) / c ** 0.5
     z = ops.conv1x1(x, wz, out_point_major=True)
-    sums, s1 = ops.edge_stats(z, idx, co, want_s1=True)
-    m = float(b * n * k)
-    mean = (sums[:, 0] / m).float()
-    invstd = torch.rsqrt((sums[:, 1] / m - (sums[:, 0] / m) ** 2).float() + 1e-5)
+    stats, s1 = ops.edge_stats(z, idx, co, want_s1=True)
+    mean = stats[:, 0].float()
+    invstd = torch.rsqrt(stats[:, 1].float() + 1e-5)
     gamma, beta = torch.randn(co, device=DEV), torch.randn(co, device=DEV)
     scale = (gamma * invstd).contiguous()
     shift = (beta - scale * mean).contiguous()
