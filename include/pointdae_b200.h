@@ -539,6 +539,55 @@ int pdae_seg_knn_f32(const float *xyz, int n_total, const float *new_xyz, int m,
                      int b, int nsample, int *idx, float *dist2, void *workspace, size_t workspace_bytes,
                      pdae_stream_t stream);
 
+/* ---- Chamfer distance over variable-size clouds in one batch (segment forward, gradients, mean losses) -----------
+ * xyz1 (n_total,3), xyz2 (m_total,3) fp32 packed as above; offset1 / offset2 (b,) int32 cumulative ends (device).
+ * Segments: row p of xyz1 belongs to the first segment s with p < offset1[s] after clamping into [0, n_total] (the rule
+ * of the segment kNN's queries), i.e. segment s = [end1[s-1], end1[s]) with end1[s] = max(offset1[0..s]) clamped; for
+ * non-decreasing offsets that is [offset1[s-1], offset1[s]).  Likewise xyz2.  Segments never overlap, whatever the
+ * offsets.  Segment s of xyz1 is matched only against segment s of xyz2.
+ * Forward (pdae_seg_chamfer_fwd_f32): dist1 (n_total,) / dist2 (m_total,) fp32 squared distances, idx1 / idx2 int32
+ *   GLOBAL row indices.  d = fma(dz,dz, fma(dx,dx, rn(dy*dy))), d* = b - a, minimum over the opposite segment, ties to
+ *   the lowest index: the rounding and tie rule of pdae_chamfer_fwd_f32, so equal segments give its (b,n,3) result bit
+ *   for bit with idx + s*m.  A point whose opposite segment is empty, or that lies past the last segment, gets dist 0
+ *   and idx -1.  Workspace: pdae_seg_chamfer_fwd_workspace_bytes(b, n_total, m_total).
+ * Backward (pdae_seg_chamfer_bwd_f32 / _det_f32): the equal-size backward at b = 1 over the packed arrays (same terms,
+ *   same orders; _det adds the terms of the points that chose a point in ascending source order); a row with idx -1
+ *   has no own term.  _det workspace: pdae_seg_chamfer_bwd_det_workspace_bytes(n_total, m_total).
+ * Mean losses (pdae_seg_chamfer_loss_f32): S = the segments with both sides non-empty.  loss3 = [loss, term1, term2],
+ *   term1 = (1/|S|) sum_{s in S} mean_s f(dist1), term2 likewise, f = identity (L2) or sqrt (L1); loss = term1 + term2
+ *   (L2) or (term1 + term2) / 2 (L1), sqrt in fp32.  |S| = 0 gives 0 everywhere.  Per-segment sums in float64 in a
+ *   fixed order, then one fixed-order float64 pass over the segments: deterministic.  state (4b + 1,) int32 receives
+ *   [|S|, end1 (b), end2 (b), weight1 (b), weight2 (b)] (weights as fp32 bits, see below) for the backward.
+ *   Workspace: pdae_seg_chamfer_loss_workspace_bytes(b).
+ * Loss backward (pdae_seg_chamfer_loss_bwd_f32 / _det_f32, `state` from the loss): the backward above with
+ *   d(loss)/d(dist) of a point of segment s = rn(gloss * weight_s), weight_s = rn(w / (float)(|S| * size_s)),
+ *   w = 1 (L2) or 0.5 (L1), |S| * size_s formed in 64 bits
+ *   (the rounding of pdae_chamfer_loss_bwd_f32, where it is b * n), divided by 2 sqrt(dist) for L1 (dist 0 gives inf,
+ *   NaN after the multiply by 0, like SqrtBackward).  _det workspace: pdae_seg_chamfer_bwd_det_workspace_bytes.
+ * b = 0: the forward, the loss and the loss backward return 0 and write nothing.  No call synchronises with the host;
+ * the forward and the loss use no float atomics, so their results depend on the inputs only.                      */
+size_t pdae_seg_chamfer_fwd_workspace_bytes(int b, int n_total, int m_total);
+int pdae_seg_chamfer_fwd_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *offset1,
+                             const int *offset2, int b, float *dist1, float *dist2, int *idx1, int *idx2, void *workspace,
+                             size_t workspace_bytes, pdae_stream_t stream);
+int pdae_seg_chamfer_bwd_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *idx1, const int *idx2,
+                             const float *gd1, const float *gd2, float *gx1, float *gx2, pdae_stream_t stream);
+size_t pdae_seg_chamfer_bwd_det_workspace_bytes(int n_total, int m_total);
+int pdae_seg_chamfer_bwd_det_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *idx1,
+                                 const int *idx2, const float *gd1, const float *gd2, float *gx1, float *gx2, void *workspace,
+                                 size_t workspace_bytes, pdae_stream_t stream);
+size_t pdae_seg_chamfer_loss_workspace_bytes(int b);
+int pdae_seg_chamfer_loss_f32(const float *dist1, int n_total, const float *dist2, int m_total, const int *offset1,
+                              const int *offset2, int b, int l1, float *loss3, int *state, void *workspace,
+                              size_t workspace_bytes, pdae_stream_t stream);
+int pdae_seg_chamfer_loss_bwd_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *idx1,
+                                  const int *idx2, const float *dist1, const float *dist2, const int *state, int b,
+                                  const float *gloss, int l1, float *gx1, float *gx2, pdae_stream_t stream);
+int pdae_seg_chamfer_loss_bwd_det_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *idx1,
+                                      const int *idx2, const float *dist1, const float *dist2, const int *state, int b,
+                                      const float *gloss, int l1, float *gx1, float *gx2, void *workspace,
+                                      size_t workspace_bytes, pdae_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -119,6 +119,16 @@ SIGNATURES = {
     "pdae_seg_fps_f32": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "pdae_seg_knn_workspace_bytes": (_sz, [_i, _i]),
     "pdae_seg_knn_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_chamfer_fwd_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_seg_chamfer_fwd_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_chamfer_bwd_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "pdae_seg_chamfer_bwd_det_workspace_bytes": (_sz, [_i, _i]),
+    "pdae_seg_chamfer_bwd_det_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_chamfer_loss_workspace_bytes": (_sz, [_i]),
+    "pdae_seg_chamfer_loss_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_chamfer_loss_bwd_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp]),
+    "pdae_seg_chamfer_loss_bwd_det_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _sz,
+                                               _vp]),
 }
 
 _lib = None

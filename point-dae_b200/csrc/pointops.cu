@@ -19,6 +19,7 @@
 // exact (d^2, index) order whatever the grid.  No atomics anywhere; results do not depend on launch shape or stream.
 #include "fps_rank.cuh"
 #include "knn_select.cuh"
+#include "segment.cuh"
 
 #include <math.h>
 
@@ -182,32 +183,6 @@ static int launch_seg_fps_reg(const SegFpsArgs &a, int b, cudaStream_t st) {
 }
 
 // ---- kNN -----------------------------------------------------------------------------------------------------------
-// inclusive block-wide scan (sum or max) of one int per thread of a 1024-thread CTA; `total` gets the last value
-__device__ __forceinline__ int block_scan_incl(int v, int *warp_tot /*[32]*/, int &total, bool is_max) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const int o = __shfl_up_sync(0xffffffffu, v, d);
-    if (lane >= d) v = is_max ? max(v, o) : v + o;
-  }
-  if (lane == 31) warp_tot[warp] = v;
-  __syncthreads();
-  if (warp == 0) {
-    int w = warp_tot[lane];
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const int o = __shfl_up_sync(0xffffffffu, w, d);
-      if (lane >= d) w = is_max ? max(w, o) : w + o;
-    }
-    warp_tot[lane] = w;
-  }
-  __syncthreads();
-  if (warp > 0) v = is_max ? max(v, warp_tot[warp - 1]) : v + warp_tot[warp - 1];
-  total = warp_tot[31];
-  __syncthreads();
-  return v;
-}
-
 // one CTA of 1024 threads.  Table entry: points [sn, en) of the segment, queries [p0, p1) (at most SEG_KNN_WARPS).
 // Query p belongs to the first segment s with p < new_offset[s] (the reference's
 // get_bt_idx), i.e. to [max(new_offset[0..s-1]), new_offset[s]); rows from max(new_offset) up to m get the padding.

@@ -1424,3 +1424,163 @@ def segment_knn(nsample, xyz, new_xyz, offset, new_offset):
         idx = torch.empty((m, int(nsample)), dtype=torch.int32, device=xyz.device)
         dist2 = torch.empty((m, int(nsample)), dtype=torch.float32, device=xyz.device)
     return segment_knn_into(nsample, xyz, new_xyz, offset, new_offset, idx, dist2)
+
+
+# ------------------------------------------------- Chamfer distance over variable-size clouds in one batch
+def _segment_pair(xyz1, xyz2, offset1, offset2, name):
+    """Input rules of the segment Chamfer calls (those of _segment_inputs, per cloud); -> b."""
+    for x, nm in ((xyz1, "xyz1"), (xyz2, "xyz2")):
+        _require_cuda(x, name)
+        _require_f32_contig(x, nm)
+        if x.dim() != 2 or x.size(1) != 3:
+            raise RuntimeError("%s must have shape (N, 3)" % nm)
+    for o, nm in ((offset1, "offset1"), (offset2, "offset2")):
+        _require_i32_contig(o, nm)
+        if o.dim() != 1:
+            raise RuntimeError("%s must have shape (b,)" % nm)
+    _same_device(xyz1.device, xyz2=xyz2, offset1=offset1, offset2=offset2)
+    if offset1.numel() != offset2.numel():
+        raise RuntimeError("offset1 and offset2 disagree on the number of segments")
+    return offset1.numel()
+
+
+def _segment_match(xyz1, xyz2, idx1, idx2, name, **dists):
+    n, m = xyz1.size(0), xyz2.size(0)
+    for x, nm in ((xyz1, "xyz1"), (xyz2, "xyz2")):
+        _require_cuda(x, name)
+        _require_f32_contig(x, nm)
+        if x.dim() != 2 or x.size(1) != 3:
+            raise RuntimeError("%s must have shape (N, 3)" % nm)
+    _require_i32_contig(idx1, "idx1")
+    _require_i32_contig(idx2, "idx2")
+    if idx1.numel() != n or idx2.numel() != m:
+        raise RuntimeError("idx1 / idx2 must hold one index per point")
+    for nm, d in dists.items():
+        _require_f32_contig(d, nm)
+        if d.numel() != (n if nm.endswith("1") else m):
+            raise RuntimeError("%s must hold one value per point" % nm)
+    _same_device(xyz1.device, xyz2=xyz2, idx1=idx1, idx2=idx2, **dists)
+
+
+def segment_chamfer_forward(xyz1, xyz2, offset1, offset2):
+    """Chamfer forward of every segment of a packed batch against the same segment of the other: xyz1 (N,3), xyz2 (M,3)
+    f32, offset1 / offset2 (b,) int32 cumulative ends -> [dist1 (N,) f32 squared, dist2 (M,), idx1 (N,) int32, idx2 (M,)],
+    indices global.  Same rounding and tie rule as chamfer_forward.  A point whose opposite segment is empty, or that lies
+    past the last segment, gets (0, -1).  No host synchronisation."""
+    b = _segment_pair(xyz1, xyz2, offset1, offset2, "segment_chamfer_forward")
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    L = _native.lib()
+    with _on(dev):
+        dist1 = torch.empty((n,), dtype=torch.float32, device=dev)
+        dist2 = torch.empty((m,), dtype=torch.float32, device=dev)
+        idx1 = torch.empty((n,), dtype=torch.int32, device=dev)
+        idx2 = torch.empty((m,), dtype=torch.int32, device=dev)
+        if b == 0:  # no segment: every point is past the last one
+            dist1.zero_(), dist2.zero_(), idx1.fill_(-1), idx2.fill_(-1)
+            return [dist1, dist2, idx1, idx2]
+        nbytes = L.pdae_seg_chamfer_fwd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_seg_chamfer_fwd_f32(xyz1.data_ptr(), n, xyz2.data_ptr(), m, offset1.data_ptr(), offset2.data_ptr(), b,
+                                        dist1.data_ptr(), dist2.data_ptr(), idx1.data_ptr(), idx2.data_ptr(), ws.data_ptr(),
+                                        nbytes, _stream())
+    _native.check(rc, "pdae_seg_chamfer_fwd_f32")
+    return [dist1, dist2, idx1, idx2]
+
+
+def segment_chamfer_backward(xyz1, xyz2, idx1, idx2, grad_dist1, grad_dist2):
+    """Gradients of segment_chamfer_forward: -> [grad_xyz1 (N,3), grad_xyz2 (M,3)].  The indices are global, so this is
+    chamfer_backward at b = 1 over the packed arrays; points with idx -1 get no own term.  Under
+    torch.use_deterministic_algorithms(True) the gradients are bit-reproducible (no float atomics)."""
+    _segment_match(xyz1, xyz2, idx1, idx2, "segment_chamfer_backward")
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    _same_device(dev, grad_dist1=grad_dist1, grad_dist2=grad_dist2)
+    grad_dist1 = grad_dist1.contiguous().float()
+    grad_dist2 = grad_dist2.contiguous().float()
+    if grad_dist1.numel() != n or grad_dist2.numel() != m:
+        raise RuntimeError("grad_dist1 / grad_dist2 must hold one value per point")
+    with _on(dev):
+        gx1, gx2 = torch.empty_like(xyz1), torch.empty_like(xyz2)
+        L = _native.lib()
+        args = (xyz1.data_ptr(), n, xyz2.data_ptr(), m, idx1.data_ptr(), idx2.data_ptr(), grad_dist1.data_ptr(),
+                grad_dist2.data_ptr(), gx1.data_ptr(), gx2.data_ptr())
+        if _deterministic():
+            nbytes = L.pdae_seg_chamfer_bwd_det_workspace_bytes(n, m)
+            ws = _workspace(nbytes, dev)
+            rc = L.pdae_seg_chamfer_bwd_det_f32(*args, ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_seg_chamfer_bwd_f32(*args, _stream())
+    _native.check(rc, "pdae_seg_chamfer_bwd_f32")
+    return [gx1, gx2]
+
+
+def segment_chamfer_loss(dist1, dist2, offset1, offset2, l1=False, state=None):
+    """Cloud-weighted mean loss over the segments S whose two sides both hold points: -> float32 tensor (3,) =
+    [loss, term1, term2], term_i = (1/|S|) sum_s mean_s f(dist_i), f = identity (L2) or sqrt (L1), loss = term1 + term2
+    (L2) or (term1 + term2) / 2 (L1); all 0 when S is empty.  The same as averaging ChamferDistanceL2 / L1 over the
+    clouds.  state: optional int32 (4b + 1,) tensor that receives what segment_chamfer_loss_backward reads.
+    Deterministic; no host synchronisation."""
+    for d, nm in ((dist1, "dist1"), (dist2, "dist2")):
+        _require_cuda(d, "segment_chamfer_loss")
+        _require_f32_contig(d, nm)
+    for o, nm in ((offset1, "offset1"), (offset2, "offset2")):
+        _require_i32_contig(o, nm)
+        if o.dim() != 1:
+            raise RuntimeError("%s must have shape (b,)" % nm)
+    dev = dist1.device
+    _same_device(dev, dist2=dist2, offset1=offset1, offset2=offset2, state=state)
+    if offset1.numel() != offset2.numel():
+        raise RuntimeError("offset1 and offset2 disagree on the number of segments")
+    b = offset1.numel()
+    L = _native.lib()
+    with _on(dev):
+        if state is None:
+            state = torch.empty((4 * b + 1,), dtype=torch.int32, device=dev)
+        _require_i32_contig(state, "state")
+        if state.numel() != 4 * b + 1:
+            raise RuntimeError("state must hold 4b + 1 = %d int32 values" % (4 * b + 1))
+        out = torch.zeros(3, dtype=torch.float32, device=dev)
+        if b == 0:
+            state.zero_()
+            return out
+        nbytes = L.pdae_seg_chamfer_loss_workspace_bytes(b)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_seg_chamfer_loss_f32(dist1.data_ptr(), dist1.numel(), dist2.data_ptr(), dist2.numel(), offset1.data_ptr(),
+                                         offset2.data_ptr(), b, 1 if l1 else 0, out.data_ptr(), state.data_ptr(), ws.data_ptr(),
+                                         nbytes, _stream())
+    _native.check(rc, "pdae_seg_chamfer_loss_f32")
+    return out
+
+
+def segment_chamfer_loss_backward(xyz1, xyz2, idx1, idx2, dist1, dist2, state, grad_loss, l1=False):
+    """Gradients of segment_chamfer_loss (given the `state` it wrote) times the device scalar grad_loss:
+    -> [grad_xyz1 (N,3), grad_xyz2 (M,3)].  Deterministic form under torch.use_deterministic_algorithms(True)."""
+    _segment_match(xyz1, xyz2, idx1, idx2, "segment_chamfer_loss_backward", dist1=dist1, dist2=dist2)
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    _require_i32_contig(state, "state")
+    _same_device(dev, state=state, grad_loss=grad_loss)
+    if (state.numel() - 1) % 4:
+        raise RuntimeError("state must be the (4b + 1,) tensor written by segment_chamfer_loss")
+    b = (state.numel() - 1) // 4
+    grad_loss = grad_loss.reshape(-1)
+    if grad_loss.numel() != 1:
+        raise RuntimeError("grad_loss must be a one-element CUDA tensor")
+    grad_loss = grad_loss.float().contiguous()
+    with _on(dev):
+        gx1, gx2 = torch.empty_like(xyz1), torch.empty_like(xyz2)
+        if b == 0:
+            gx1.zero_(), gx2.zero_()
+            return [gx1, gx2]
+        L = _native.lib()
+        args = (xyz1.data_ptr(), n, xyz2.data_ptr(), m, idx1.data_ptr(), idx2.data_ptr(), dist1.data_ptr(), dist2.data_ptr(),
+                state.data_ptr(), b, grad_loss.data_ptr(), 1 if l1 else 0, gx1.data_ptr(), gx2.data_ptr())
+        if _deterministic():
+            nbytes = L.pdae_seg_chamfer_bwd_det_workspace_bytes(n, m)
+            ws = _workspace(nbytes, dev)
+            rc = L.pdae_seg_chamfer_loss_bwd_det_f32(*args, ws.data_ptr(), nbytes, _stream())
+        else:
+            rc = L.pdae_seg_chamfer_loss_bwd_f32(*args, _stream())
+    _native.check(rc, "pdae_seg_chamfer_loss_bwd_f32")
+    return [gx1, gx2]
