@@ -253,9 +253,6 @@ int pdae_pair_loss_fwd_f64(const float *a, const float *b, const int *idx1, cons
 int pdae_pair_loss_bwd_f32(const float *a, const float *b, const int *idx1, const int *idx2, const float *gloss, float w1,
                            float w2, int bs, int n, int m, int d, int metric, float *ga, float *gb, pdae_stream_t stream);
 
-/* tuning hook, no reference counterpart: select the CTA shape of the large-cloud forward kernel (ids as the
- * PDAE_CHAMFER_CFG environment variable; v < 0 only queries).  Returns the previous id.  Not thread-safe.      */
-int pdae_tune_chamfer_variant(int v);
 /* tuning hook, no reference counterpart: number of column chunks every 512-row block of the symmetric forward is cut
  * into (ids as the PDAE_CHAMFER_SPLIT environment variable: 0 = automatic, 1 = never split; nc < 0 only queries).
  * Returns the previous setting.  Results do not depend on it.  Not thread-safe.                                 */

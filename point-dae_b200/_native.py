@@ -71,7 +71,6 @@ SIGNATURES = {
     "pdae_pair_loss_partial_count": (_sz, [_i, _i, _i]),
     "pdae_pair_loss_fwd_f64": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "pdae_pair_loss_bwd_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
-    "pdae_tune_chamfer_variant": (_i, [_i]),
     "pdae_tune_chamfer_split": (_i, [_i]),
     "pdae_tune_chamfer_tc": (_i, [_i, _f]),
     "pdae_chamfer_tc_probe": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

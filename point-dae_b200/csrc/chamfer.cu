@@ -7,7 +7,7 @@
 // attaining it; backward g = 2*grad_dist, v = g*(a - b_idx), gx1[j] += v, gx2[idx] -= v.
 //
 // Design (FP32 FMA-pipe bound, see DESIGN.md):
-//   * a CTA owns QT*THREADS query points held in registers (each coordinate duplicated into a
+//   * a CTA owns QT*CH_THREADS query points held in registers (each coordinate duplicated into a
 //     64-bit register pair) and streams the other cloud through shared memory in planar
 //     (SoA) tiles, so one LDS.128 feeds two packed FADD2/FMUL2/FFMA2 evaluations per query;
 //   * the inner loop carries no index: the running minimum is updated with one FMNMX3 per two
@@ -38,12 +38,11 @@ struct ChamferDir {
                     // pre-filled with the MIN identity: the chunks merge their (row minimum, lowest index) with RED.MIN
 };
 
-// chamfer_min_body (the scan of one row block) lives in chamfer_core.cuh
-template <int QT, int THREADS, int MINB, bool SYM, int CH_TILE = 512 /* reference points per shared-memory tile */,
-          int STEP = 8 /* reference points per inner step (4 or 8): QT*STEP distances are live at once */,
-          bool PACKED = true /* fp32x2 arithmetic */>
-__global__ void __launch_bounds__(THREADS, MINB) chamfer_min_kernel(const ChamferDir d0, const ChamferDir d1) {
-  constexpr int W = THREADS / 32;
+// chamfer_min_body (the scan of one row block) lives in chamfer_core.cuh.  QT = 4 queries per thread, or 1 for the
+// two-scan path of clouds up to 256 points (see launch_min).
+template <int QT, bool SYM>
+__global__ void __launch_bounds__(CH_THREADS, 1) chamfer_min_kernel(const ChamferDir d0, const ChamferDir d1) {
+  constexpr int W = CH_THREADS / 32;
   __shared__ __align__(16) float tile[2][3][CH_TILE];
   __shared__ __align__(16) unsigned colmin[SYM ? 2 : 1][W][SYM ? CH_TILE : 4];
 
@@ -64,54 +63,10 @@ __global__ void __launch_bounds__(THREADS, MINB) chamfer_min_kernel(const Chamfe
     tile_end = tile_begin + tpc;
     if (tile_begin >= ntiles) return;  // uniform for the CTA
   }
-  chamfer_min_body<QT, THREADS, SYM, CH_TILE, STEP, false, PACKED>(
+  chamfer_min_body<QT, SYM>(
       d.q + static_cast<size_t>(cloud) * d.nq * 3, d.r + static_cast<size_t>(cloud) * d.nr * 3, d.nq, d.nr,
-      t * (QT * THREADS), static_cast<size_t>(cloud), d.dist, d.idx, d.keys, d.ref_offset, d.colkeys, tile, colmin,
+      t * (QT * CH_THREADS), static_cast<size_t>(cloud), d.dist, d.idx, d.keys, d.ref_offset, d.colkeys, tile, colmin,
       tile_begin, tile_end, nc > 1);
-}
-
-// Balanced variant of the symmetric forward (opt-in, PDAE_CHAMFER_CFG=17; measured NOT faster, kept as the record of
-// the experiment).  The uniform kernel above hands every CTA
-// 128*QT rows; at 128 x 2048^2 that is 512 equal CTAs for 296 resident slots, and since ONE 4-warp CTA already
-// saturates an SM's FMA issue the SMs that receive three CTAs instead of four idle for the last eighth of the kernel
-// (FMA pipe 67 % of active but 57 % of elapsed cycles).  Here the rows of the whole batch are cut into 128-row
-// slices, the slices are dealt out evenly to a persistent grid (two CTAs per SM), and every CTA walks its share in
-// passes of up to four slices of one cloud (QT = 4, 3, 2 or 1 queries per thread): the per-scheduler work differs by
-// at most one slice (7 against 6.92 at the headline shape).  Warps name themselves in the column keys by
-// (first row / 32) << 3 | QT because passes of different QT give 32*QT-row groups.
-// Result on B200 (profiles/r01/probe_chamfer_balanced.csv): 161.9 us against 161.1 us for the uniform kernel under ncu.
-// Cloud boundaries force passes narrower than four slices (at 16 slices per cloud and ~7 per CTA: 352 passes of QT 3,
-// 208 of QT 4, 64 of QT 2, 32 of QT 1), and a narrow pass pays the per-column work (tile reads, column reductions,
-// REDUX, key posts) for fewer rows: the in-loop FMA rate drops from 67 % to 61.5 % and the SMs are no better balanced
-// (active cycles min/avg/max 242k/279k/297k).
-template <int THREADS, int CH_TILE, int STEP>
-__global__ void __launch_bounds__(THREADS, 1) chamfer_min_balanced_kernel(const ChamferDir d, int slices_per_cloud,
-                                                                          long long total_slices) {
-  constexpr int W = THREADS / 32;
-  __shared__ __align__(16) float tile[2][3][CH_TILE];
-  __shared__ __align__(16) unsigned colmin[2][W][CH_TILE];
-  long long cur = static_cast<long long>(blockIdx.x) * total_slices / gridDim.x;
-  const long long end = static_cast<long long>(blockIdx.x + 1) * total_slices / gridDim.x;
-  while (cur < end) {
-    const long long cloud = cur / slices_per_cloud;
-    const int s0 = static_cast<int>(cur - cloud * slices_per_cloud);
-    long long seg = end - cur;  // what is left of this CTA's share inside the current cloud ...
-    if (seg > slices_per_cloud - s0) seg = slices_per_cloud - s0;
-    const long long passes = (seg + 3) / 4;  // ... walked in as few passes as possible, of (nearly) equal width:
-    const long long cnt = (seg + passes - 1) / passes;  // 5 -> 3+2, 6 -> 3+3, 7 -> 4+3 (narrow passes run at a lower FMA rate)
-    const float *Q = d.q + static_cast<size_t>(cloud) * d.nq * 3, *R = d.r + static_cast<size_t>(cloud) * d.nr * 3;
-    const int row_base = s0 * THREADS;
-    __syncthreads();  // the previous pass is done with the shared buffers
-#define PDAE_PASS(QT)                                                                                                   \
-  chamfer_min_body<QT, THREADS, true, CH_TILE, STEP, true>(Q, R, d.nq, d.nr, row_base, static_cast<size_t>(cloud), d.dist, \
-                                                          d.idx, d.keys, d.ref_offset, d.colkeys, tile, colmin)
-    if (cnt == 4) PDAE_PASS(4);
-    else if (cnt == 3) PDAE_PASS(3);
-    else if (cnt == 2) PDAE_PASS(2);
-    else PDAE_PASS(1);
-#undef PDAE_PASS
-    cur += cnt;
-  }
 }
 
 // ---- tiny clouds (both sides <= SMALL_MAX points): one warp per (cloud, direction) -----------
@@ -219,36 +174,8 @@ __global__ void __launch_bounds__(256) unpack_keys_kernel(const uint64_t *__rest
   idx[i] = static_cast<int>(static_cast<uint32_t>(k));
 }
 
-// tuning hook: PDAE_CHAMFER_CFG selects the CTA shape of the large-cloud kernel
-
-static int g_chamfer_variant = -1;
-static int chamfer_variant() {
-  if (g_chamfer_variant < 0) {
-    const char *e = getenv("PDAE_CHAMFER_CFG");
-    g_chamfer_variant = e ? atoi(e) : 0;
-  }
-  return g_chamfer_variant;
-}
-// tuning hook (profiles/tune_kernels.py): switch the kernel shape inside one process; ids as PDAE_CHAMFER_CFG
-extern "C" int pdae_tune_chamfer_variant(int v) {
-  const int old = chamfer_variant();
-  if (v >= 0) g_chamfer_variant = v;
-  return old;
-}
-// queries per CTA of the kernel launch_min / launch_sym will pick (the callers size `qtiles` with it)
-static int chamfer_qpc(int nq_max, bool sym) {
-  if (!sym && nq_max <= 256) return 128;
-  switch (chamfer_variant() % 25) {
-    case 3: return 512;   // <2,256>
-    case 4: return 256;   // <2,128>
-    case 5: case 6: case 7: return 256;   // <4,64>
-    case 8: case 10: return 512;   // <8,64>
-    case 9: case 11: return 256;   // <8,32>
-    case 12: case 13: return 128;  // <4,32>
-    case 14: case 15: return 1024; // <8,128>
-    default: return 512;  // <4,128>
-  }
-}
+// queries per CTA of the kernel launch_min will pick (the callers size `qtiles` with it)
+static int chamfer_qpc(int nq_max, bool sym) { return !sym && nq_max <= 256 ? CH_THREADS : 4 * CH_THREADS; }
 
 template <bool SYM>
 static int launch_min(const ChamferDir &d0, const ChamferDir &d1, int b, cudaStream_t st) {
@@ -258,29 +185,8 @@ static int launch_min(const ChamferDir &d0, const ChamferDir &d1, int b, cudaStr
   if (grid > 0x7fffffffLL) return PDAE_E_UNSUPPORTED;
   const unsigned g = static_cast<unsigned>(grid);
   const int nq_max = d0.nq > d1.nq ? d0.nq : d1.nq;
-  if (!SYM && nq_max <= 256) {
-    chamfer_min_kernel<1, 128, 1, false><<<g, 128, 0, st>>>(d0, d1);
-  } else {
-    switch (chamfer_variant() % 25) {
-      case 1: chamfer_min_kernel<4, 128, 4, SYM><<<g, 128, 0, st>>>(d0, d1); break;
-      case 2: chamfer_min_kernel<4, 128, 3, SYM><<<g, 128, 0, st>>>(d0, d1); break;
-      case 3: chamfer_min_kernel<2, 256, 3, SYM><<<g, 256, 0, st>>>(d0, d1); break;
-      case 4: chamfer_min_kernel<2, 128, 6, SYM><<<g, 128, 0, st>>>(d0, d1); break;
-      case 5: chamfer_min_kernel<4, 64, 4, SYM, 256><<<g, 64, 0, st>>>(d0, d1); break;
-      case 6: chamfer_min_kernel<4, 64, 8, SYM, 256><<<g, 64, 0, st>>>(d0, d1); break;
-      case 7: chamfer_min_kernel<4, 64, 6, SYM, 256><<<g, 64, 0, st>>>(d0, d1); break;
-      case 8: chamfer_min_kernel<8, 64, 4, SYM, 256, 4><<<g, 64, 0, st>>>(d0, d1); break;
-      case 9: chamfer_min_kernel<8, 32, 8, SYM, 128, 4><<<g, 32, 0, st>>>(d0, d1); break;
-      case 10: chamfer_min_kernel<8, 64, 6, SYM, 256, 4><<<g, 64, 0, st>>>(d0, d1); break;
-      case 11: chamfer_min_kernel<8, 32, 12, SYM, 128, 4><<<g, 32, 0, st>>>(d0, d1); break;
-      case 12: chamfer_min_kernel<4, 32, 16, SYM, 128, 8><<<g, 32, 0, st>>>(d0, d1); break;
-      case 13: chamfer_min_kernel<4, 32, 12, SYM, 128, 8><<<g, 32, 0, st>>>(d0, d1); break;
-      case 14: chamfer_min_kernel<8, 128, 1, SYM, 512, 4><<<g, 128, 0, st>>>(d0, d1); break;
-      case 15: chamfer_min_kernel<8, 128, 1, SYM, 512, 8><<<g, 128, 0, st>>>(d0, d1); break;
-      case 18: chamfer_min_kernel<4, 128, 1, SYM, 512, 8, false><<<g, 128, 0, st>>>(d0, d1); break;
-      default: chamfer_min_kernel<4, 128, 1, SYM><<<g, 128, 0, st>>>(d0, d1); break;
-    }
-  }
+  if (chamfer_qpc(nq_max, SYM) == CH_THREADS) chamfer_min_kernel<1, false><<<g, CH_THREADS, 0, st>>>(d0, d1);
+  else chamfer_min_kernel<4, SYM><<<g, CH_THREADS, 0, st>>>(d0, d1);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
 }
@@ -294,14 +200,19 @@ __global__ void __launch_bounds__(256) fill_keys_kernel(uint64_t *__restrict__ k
   if (i < count) keys[i] = CHAMFER_KEY_IDENTITY;
 }
 
-// symmetric mode, second half: one warp per column point b_j.  colkeys[j] = (min_i d(a_i, b_j), id of the
-// QPG-query group holding a minimiser; lowest such group).  Scanning that group in index order and taking
-// the first query whose distance equals the minimum bit for bit yields the lowest index overall.
-// QPG = queries per group (32 * QT of the main kernel).  A group's queries are contiguous, so each lane takes
-// QPG/32 consecutive ones (float4 loads when the cloud base is 16-byte aligned) and the whole group is examined in
-// one step; lanes are in index order, hence ballot + ffs gives the lowest index.  A warp resolves RPW consecutive
-// column points with all their loads issued up front: the kernel is pure load latency (key -> group rows), so the
-// memory-level parallelism per warp is what sets its speed.
+// rows per column-key group: the 32*QT queries of one warp of the symmetric scan, chamfer_min_kernel<4, true>
+constexpr int RECOVER_QPG = 32 * 4;
+// the list recovery serves clouds up to this many row groups, the warp-per-column recovery larger ones
+constexpr int RECOVER_LIST_GROUPS = 128;
+
+// symmetric mode, second half: the column recovery.  colkeys[j] = (min_i d(a_i, b_j), id of the QPG-query group holding
+// a minimiser; lowest such group), QPG = RECOVER_QPG.  Scanning that group in index order and taking the first query
+// whose distance equals the minimum bit for bit yields the lowest index overall.
+// Warp-per-column form, for clouds above RECOVER_LIST_GROUPS groups: one warp per column point b_j.  A group's queries
+// are contiguous, so each lane takes QPG/32 consecutive ones (float4 loads when the cloud base is 16-byte aligned) and
+// the whole group is examined in one step; lanes are in index order, hence ballot + ffs gives the lowest index.  A warp
+// resolves RPW consecutive column points with all their loads issued up front: the kernel is pure load latency
+// (key -> group rows), so the memory-level parallelism per warp is what sets its speed.
 template <int QPG, int RPW>
 __global__ void __launch_bounds__(256) chamfer_col_recover_kernel(const float *__restrict__ rows, const float *__restrict__ cols,
                                                                   const uint64_t *__restrict__ colkeys, int n_rows,
@@ -361,94 +272,13 @@ __global__ void __launch_bounds__(256) chamfer_col_recover_kernel(const float *_
   }
 }
 
-// Group-major variant of the recovery for clouds up to a few thousand points: one CTA per (cloud, QPG-row group).
-// Every lane keeps QPG/32 consecutive rows of the group in registers for the whole CTA; the warps sweep the cloud's
-// column keys (coalesced), and only the columns whose key names this group are resolved, their coordinates and
-// minimum broadcast from the lane that read them.  The warp-per-column kernel above re-reads a whole group
-// (12*QPG bytes) per column -- 400 MB of L2 traffic at 128 x 2048^2; here the traffic is the keys once per group
-// (8*n_cols bytes per CTA), 10x less, and the rows never leave registers.  Traffic grows with n_rows*n_cols/QPG, so
-// the launcher keeps the warp-per-column kernel for large clouds.
-template <int QPG>
-__global__ void __launch_bounds__(256) chamfer_col_recover_grouped_kernel(const float *__restrict__ rows,
-                                                                          const float *__restrict__ cols,
-                                                                          const uint64_t *__restrict__ colkeys,
-                                                                          int n_rows, int n_cols,
-                                                                          float *__restrict__ dist, int *__restrict__ idx) {
-  constexpr int PER = QPG / 32;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const unsigned g = blockIdx.x;
-  const size_t cloud = blockIdx.y;
-  const float *__restrict__ A = rows + cloud * n_rows * 3;
-  const int base = static_cast<int>(g) * QPG + lane * PER;
-  float rx[PER], ry[PER], rz[PER];
-  if ((n_rows & 3) == 0 && PER % 4 == 0 && base + PER <= n_rows) {
-    const float4 *p4 = reinterpret_cast<const float4 *>(A + 3 * static_cast<size_t>(base));
-    float c[3 * PER];
-#pragma unroll
-    for (int t = 0; t < 3 * PER / 4; ++t) {
-      const float4 w = __ldg(p4 + t);
-      c[4 * t] = w.x; c[4 * t + 1] = w.y; c[4 * t + 2] = w.z; c[4 * t + 3] = w.w;
-    }
-#pragma unroll
-    for (int t = 0; t < PER; ++t) rx[t] = c[3 * t], ry[t] = c[3 * t + 1], rz[t] = c[3 * t + 2];
-  } else {
-#pragma unroll
-    for (int t = 0; t < PER; ++t) {
-      const bool in = base + t < n_rows;  // NaN padding never matches
-      rx[t] = in ? __ldg(A + 3 * static_cast<size_t>(base + t)) : __int_as_float(0x7fc00000);
-      ry[t] = in ? __ldg(A + 3 * static_cast<size_t>(base + t) + 1) : 0.0f;
-      rz[t] = in ? __ldg(A + 3 * static_cast<size_t>(base + t) + 2) : 0.0f;
-    }
-  }
-  const uint64_t *__restrict__ K = colkeys + cloud * n_cols;
-  const float *__restrict__ C = cols + cloud * n_cols * 3;
-  constexpr int UNR = 4;  // key sweeps in flight per warp: the loop is pure L2 latency otherwise
-  for (int j0 = warp * 32; j0 < n_cols; j0 += 256 * UNR) {
-    uint64_t key[UNR];
-    float cx[UNR], cy[UNR], cz[UNR];
-#pragma unroll
-    for (int u = 0; u < UNR; ++u) {  // keys and coordinates fetched together (coalesced, no dependent second trip)
-      const int j = j0 + u * 256 + lane;
-      const bool in = j < n_cols;
-      key[u] = in ? K[j] : ~0ull;
-      cx[u] = in ? __ldg(C + 3 * j) : 0.f, cy[u] = in ? __ldg(C + 3 * j + 1) : 0.f, cz[u] = in ? __ldg(C + 3 * j + 2) : 0.f;
-    }
-#pragma unroll
-    for (int u = 0; u < UNR; ++u) {
-      const int j = j0 + u * 256 + lane;
-      const bool match = static_cast<uint32_t>(key[u]) == g && j < n_cols;
-      const float v = __uint_as_float(static_cast<uint32_t>(key[u] >> 32));
-      unsigned mk = __ballot_sync(0xffffffffu, match);
-      int mine = 0;
-      while (mk) {
-        const int src = __ffs(mk) - 1;
-        mk &= mk - 1;
-        const float bx = __shfl_sync(0xffffffffu, cx[u], src), by = __shfl_sync(0xffffffffu, cy[u], src);
-        const float bz = __shfl_sync(0xffffffffu, cz[u], src), want = __shfl_sync(0xffffffffu, v, src);
-        int first = PER;  // first matching row of this lane
-#pragma unroll
-        for (int t = PER - 1; t >= 0; --t) {
-          const float d = dist_yxz(__fsub_rn(bx, rx[t]), __fsub_rn(by, ry[t]), __fsub_rn(bz, rz[t]));
-          first = (d == want) ? t : first;
-        }
-        const unsigned hit = __ballot_sync(0xffffffffu, first < PER);
-        const int found = __shfl_sync(0xffffffffu, base + first, hit ? __ffs(hit) - 1 : 0);
-        if (lane == src) mine = hit ? found : 0;
-      }
-      if (match) {
-        dist[cloud * n_cols + j] = v;
-        idx[cloud * n_cols + j] = mine;
-      }
-    }
-  }
-}
-
-// List variant of the group-major recovery (default for clouds up to 32 groups): the CTA of (cloud, group) stages the
+// List form of the recovery, for clouds up to RECOVER_LIST_GROUPS groups: the CTA of (cloud, group) stages the
 // group's QPG rows in shared memory as planes, every thread tests a strided share of the cloud's column keys and
 // appends the columns won by this group to a shared list, and then ONE THREAD PER LISTED COLUMN walks the group's rows
 // (broadcast LDS.64 of two rows per plane, packed distance, compare with the recorded minimum bit for bit), back to
 // front so that the lowest matching row is the one kept.  No shuffles or ballots in the walk: ~6.5 instructions per
-// (column, row) against ~14 in the warp-cooperative kernel above.
+// (column, row).  The warp-per-column kernel above re-reads a whole group (12*QPG bytes) per column; here the traffic
+// is the keys once per group (8*n_cols bytes per CTA), which grows with n_rows*n_cols/QPG -- hence the size limit.
 constexpr int RECOVER_LIST_MAX = 4096;  // columns examined per pass (list of int in shared memory)
 
 template <int QPG>
@@ -525,116 +355,28 @@ __global__ void __launch_bounds__(256) chamfer_col_recover_list_kernel(const flo
   }
 }
 
-// Recovery for the balanced kernel: its column keys name the winning warp's rows as (first row / 32) << 3 | QT, a
-// 32-aligned range of 32*QT <= 128 rows.  One CTA per (cloud, aligned 128-row block g) stages rows
-// [128 g, 128 g + 224) -- a range that starts in the block ends before that -- collects the columns whose range starts
-// in the block and walks exactly the range, back to front (lowest matching row kept), as the list kernel above.
-__global__ void __launch_bounds__(256) chamfer_col_recover_var_kernel(const float *__restrict__ rows,
-                                                                      const float *__restrict__ cols,
-                                                                      const uint64_t *__restrict__ colkeys, int n_rows,
-                                                                      int n_cols, float *__restrict__ dist,
-                                                                      int *__restrict__ idx) {
-  constexpr int SPAN = 224;
-  __shared__ __align__(16) float sx[SPAN], sy[SPAN], sz[SPAN];
-  __shared__ int list[RECOVER_LIST_MAX];
-  __shared__ int count;
-  const unsigned g = blockIdx.x;
-  const size_t cloud = blockIdx.y;
-  const float *__restrict__ A = rows + cloud * n_rows * 3;
-  const uint64_t *__restrict__ K = colkeys + cloud * n_cols;
-  const float *__restrict__ C = cols + cloud * n_cols * 3;
-  const int tid = threadIdx.x;
-  if (tid == 0) count = 0;
-  for (int e = tid; e < 3 * SPAN; e += 256) {  // NaN padding (rows past the cloud) never matches
-    const int r = e / 3, c = e - 3 * r;
-    const long long row = static_cast<long long>(g) * 128 + r;
-    const float v = row < n_rows ? __ldg(A + row * 3 + c) : __int_as_float(0x7fc00000);
-    (c == 0 ? sx : c == 1 ? sy : sz)[r] = v;
-  }
-  __syncthreads();
-  constexpr int UNR = 8;
-  for (int c0 = 0; c0 < n_cols; c0 += RECOVER_LIST_MAX) {
-    const int c1 = c0 + RECOVER_LIST_MAX < n_cols ? c0 + RECOVER_LIST_MAX : n_cols;
-    for (int j0 = c0 + tid; j0 < c1; j0 += 256 * UNR) {
-      uint32_t who[UNR];
-#pragma unroll
-      for (int u = 0; u < UNR; ++u) {
-        const int j = j0 + u * 256;
-        who[u] = j < c1 ? static_cast<uint32_t>(K[j]) : 0xffffffffu;
-      }
-#pragma unroll
-      for (int u = 0; u < UNR; ++u)
-        if ((who[u] >> 5) == g) list[atomicAdd(&count, 1)] = j0 + u * 256;  // (first row / 32) / 4 == block
-    }
-    __syncthreads();
-    const int total = count;
-    for (int m = tid; m < total; m += 256) {
-      const int j = list[m];
-      const uint64_t key = K[j];
-      const float want = __uint_as_float(static_cast<uint32_t>(key >> 32));
-      const int lo = static_cast<int>((static_cast<uint32_t>(key) >> 3) & 3u) * 32;  // range start inside the block
-      const int len = static_cast<int>(static_cast<uint32_t>(key) & 7u) * 32;
-      const float bx = __ldg(C + 3 * j), by = __ldg(C + 3 * j + 1), bz = __ldg(C + 3 * j + 2);
-      const float2 cx = make_float2(bx, bx), cy = make_float2(by, by), cz = make_float2(bz, bz);
-      int found = lo;
-#pragma unroll 8
-      for (int r = lo + len - 2; r >= lo; r -= 2) {
-        const float2 d = dist_yxz2(sub2(cx, *reinterpret_cast<const float2 *>(sx + r)),
-                                   sub2(cy, *reinterpret_cast<const float2 *>(sy + r)),
-                                   sub2(cz, *reinterpret_cast<const float2 *>(sz + r)));
-        found = (d.y == want) ? r + 1 : found;
-        found = (d.x == want) ? r : found;
-      }
-      dist[cloud * n_cols + j] = want;
-      idx[cloud * n_cols + j] = static_cast<int>(g) * 128 + found;
-    }
-    __syncthreads();
-    if (tid == 0) count = 0;
-    __syncthreads();
-  }
+// true when the list kernel recovers a cloud of n_rows rows.  It visits every row exactly once, so it also unpacks the
+// row keys of an (unphased) column-split forward.
+static bool recover_unpacks_rows(int n_rows) {
+  return (static_cast<long long>(n_rows) + RECOVER_QPG - 1) / RECOVER_QPG <= RECOVER_LIST_GROUPS;
 }
 
-// second half of the symmetric forward: picks the recovery kernel by cloud size (see the comment above)
-template <int QPG>
+// second half of the symmetric forward: picks the recovery kernel by cloud size
 static int launch_col_recover(const float *rows, const float *cols, const uint64_t *ck, int b, int n_rows, int n_cols,
                               float *dcol, int *icol, cudaStream_t st, const uint64_t *rowkeys = nullptr,
                               float *drow = nullptr, int *irow = nullptr) {
-  const long long groups = (static_cast<long long>(n_rows) + QPG - 1) / QPG;
-  // group-major recovery while its key sweeps (8*groups B per column) stay cheaper than re-reading a group per column
-  const int gdefault = chamfer_variant() < 25 ? 128 : 32;
-  const int glimit = chamfer_variant() >= 50 ? 0 : (getenv("PDAE_RECOVER_GROUPS") ? atoi(getenv("PDAE_RECOVER_GROUPS")) : gdefault);
-  if (groups <= glimit) {  // key + coordinate sweeps (20*groups B per column) cheaper than row re-reads (12*QPG B)
-    const dim3 ggrid(static_cast<unsigned>(groups), b);
-    if (chamfer_variant() < 25) {
-      chamfer_col_recover_list_kernel<QPG><<<ggrid, 256, 0, st>>>(rows, cols, ck, n_rows, n_cols, dcol, icol, rowkeys, drow, irow);
-    } else {
-      if (rowkeys) return PDAE_E_INVALID;  // only the list kernel unpacks row keys (recover_unpacks_rows)
-      chamfer_col_recover_grouped_kernel<QPG><<<ggrid, 256, 0, st>>>(rows, cols, ck, n_rows, n_cols, dcol, icol);
-    }
+  if (recover_unpacks_rows(n_rows)) {
+    const dim3 ggrid(static_cast<unsigned>(ceil_div(n_rows, RECOVER_QPG)), b);
+    chamfer_col_recover_list_kernel<RECOVER_QPG><<<ggrid, 256, 0, st>>>(rows, cols, ck, n_rows, n_cols, dcol, icol, rowkeys,
+                                                                        drow, irow);
   } else {
     if (rowkeys) return PDAE_E_INVALID;
     // 4 column points per warp, 8 warps per CTA (splitting a warp across points was measured slower)
     const dim3 rgrid(static_cast<unsigned>((n_cols + 31) / 32), b);
-    chamfer_col_recover_kernel<QPG, 4><<<rgrid, 256, 0, st>>>(rows, cols, ck, n_rows, n_cols, dcol, icol);
+    chamfer_col_recover_kernel<RECOVER_QPG, 4><<<rgrid, 256, 0, st>>>(rows, cols, ck, n_rows, n_cols, dcol, icol);
   }
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
-}
-
-// true when the recovery of an (unphased) column-split forward can unpack the row keys itself: default kernel shape
-// (the only one that splits) and few enough 128-row groups for the list kernel, which visits every row exactly once
-static bool recover_unpacks_rows(int n_rows) {
-  const int glimit = getenv("PDAE_RECOVER_GROUPS") ? atoi(getenv("PDAE_RECOVER_GROUPS")) : 128;
-  return chamfer_variant() == 0 && (static_cast<long long>(n_rows) + 127) / 128 <= glimit;
-}
-
-static int launch_col_recover_for_variant(const float *rows, const float *cols, const uint64_t *ck, int b, int n_rows,
-                                          int n_cols, float *dcol, int *icol, cudaStream_t st,
-                                          const uint64_t *rowkeys = nullptr, float *drow = nullptr, int *irow = nullptr) {
-  const int v = chamfer_variant() % 25;  // queries per warp = 32 * QT of the variant launched
-  if (v == 3 || v == 4) return launch_col_recover<64>(rows, cols, ck, b, n_rows, n_cols, dcol, icol, st);
-  if ((v >= 8 && v <= 11) || v == 14 || v == 15) return launch_col_recover<256>(rows, cols, ck, b, n_rows, n_cols, dcol, icol, st);
-  return launch_col_recover<128>(rows, cols, ck, b, n_rows, n_cols, dcol, icol, st, rowkeys, drow, irow);
 }
 
 }  // namespace pdae
@@ -698,7 +440,7 @@ static int chamfer_fwd_impl(const float *xyz1, const float *xyz2, int b, int n, 
   const int nq_max = n > m ? n : m;
   const size_t need = static_cast<size_t>(b) * (n < m ? n : m) * sizeof(uint64_t);  // column keys (the row keys are optional)
   const bool sym = n > 0 && m > 0 && !(n <= SMALL_MAX && m <= SMALL_MAX) && workspace != nullptr &&
-                   workspace_bytes >= need && nq_max > 256 && chamfer_variant() < 100 &&
+                   workspace_bytes >= need && nq_max > 256 &&
                    b <= 65535;  // the recovery kernels index clouds with gridDim.y; larger batches take the two-scan path
   if (phase == 2 && !sym) return 0;
   if (n == 0 || m == 0) {  // reference: outputs stay at their zero initialisation (chamfer.cu:152-157)
@@ -734,12 +476,9 @@ static int chamfer_fwd_impl(const float *xyz1, const float *xyz2, int b, int n, 
     int *irow = swap ? idx2 : idx1, *icol = swap ? idx1 : idx2;
     uint64_t *ck = static_cast<uint64_t *>(workspace);
     const long long ncol = static_cast<long long>(b) * nr_cols;
-    const long long slices_per_cloud = (static_cast<long long>(nr_rows) + 127) / 128;
-    const bool balanced = chamfer_variant() == 17 && slices_per_cloud <= 128;  // opt-in (measured no faster)
     const long long nrow = static_cast<long long>(b) * nr_rows;
-    // column split: default kernel shape only (512-row blocks, 512-point tiles), and only with room for the row keys
-    const int nsplit = (!balanced && chamfer_variant() == 0 &&
-                        workspace_bytes >= static_cast<size_t>(ncol + nrow) * sizeof(uint64_t))
+    // column split: only with room for the row keys
+    const int nsplit = workspace_bytes >= static_cast<size_t>(ncol + nrow) * sizeof(uint64_t)
                            ? chamfer_csplit(static_cast<long long>(b) * ceil_div(nr_rows, 512), ceil_div(nr_cols, 512))
                            : 1;
     // the whole forward in one call: the list recovery writes the rows' results while it is there
@@ -748,40 +487,25 @@ static int chamfer_fwd_impl(const float *xyz1, const float *xyz2, int b, int n, 
       const long long nfill = nsplit > 1 ? ncol + nrow : ncol;
       fill_keys_kernel<<<static_cast<unsigned>((nfill + 255) / 256), 256, 0, st>>>(ck, nfill);
       PDAE_RETURN_IF_LAUNCH_FAILED();
-      if (balanced) {
-        const long long total = slices_per_cloud * b;
-        const long long slots = 2LL * sm_count();
-        ChamferDir d{rows, cols, drow, irow, nullptr, ck, nr_rows, nr_cols, 0, 0};
-        chamfer_min_balanced_kernel<128, 512, 8><<<static_cast<unsigned>(total < slots ? total : slots), 128, 0, st>>>(
-            d, static_cast<int>(slices_per_cloud), total);
+      const int qpc = chamfer_qpc(nr_rows, true);
+      ChamferDir d0{rows, cols, drow, irow, nullptr, ck, nr_rows, nr_cols, ceil_div(nr_rows, qpc), 0};
+      ChamferDir d1{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
+      if (nsplit > 1) {  // rows leave as merged keys instead of dist / idx
+        d0.csplit = nsplit;
+        d0.keys = ck + ncol;
+        d0.dist = nullptr;
+        d0.idx = nullptr;
+      }
+      const int rc = launch_min<true>(d0, d1, b, st);
+      if (rc) return rc;
+      if (nsplit > 1 && !fused_unpack) {  // merged row keys -> dist / idx of the larger cloud
+        unpack_keys_kernel<<<static_cast<unsigned>((nrow + 255) / 256), 256, 0, st>>>(ck + ncol, nrow, drow, irow);
         PDAE_RETURN_IF_LAUNCH_FAILED();
-      } else {
-        const int qpc = chamfer_qpc(nr_rows, true);
-        ChamferDir d0{rows, cols, drow, irow, nullptr, ck, nr_rows, nr_cols, ceil_div(nr_rows, qpc), 0};
-        ChamferDir d1{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
-        if (nsplit > 1) {  // rows leave as merged keys instead of dist / idx
-          d0.csplit = nsplit;
-          d0.keys = ck + ncol;
-          d0.dist = nullptr;
-          d0.idx = nullptr;
-        }
-        const int rc = launch_min<true>(d0, d1, b, st);
-        if (rc) return rc;
-        if (nsplit > 1 && !fused_unpack) {  // merged row keys -> dist / idx of the larger cloud
-          unpack_keys_kernel<<<static_cast<unsigned>((nrow + 255) / 256), 256, 0, st>>>(ck + ncol, nrow, drow, irow);
-          PDAE_RETURN_IF_LAUNCH_FAILED();
-        }
       }
     }
     if (phase == 1) return 0;
-    if (balanced) {
-      const dim3 vgrid(static_cast<unsigned>(slices_per_cloud), b);
-      chamfer_col_recover_var_kernel<<<vgrid, 256, 0, st>>>(rows, cols, ck, nr_rows, nr_cols, dcol, icol);
-      PDAE_RETURN_IF_LAUNCH_FAILED();
-      return 0;
-    }
-    if (fused_unpack) return launch_col_recover_for_variant(rows, cols, ck, b, nr_rows, nr_cols, dcol, icol, st, ck + ncol, drow, irow);
-    return launch_col_recover_for_variant(rows, cols, ck, b, nr_rows, nr_cols, dcol, icol, st);
+    if (fused_unpack) return launch_col_recover(rows, cols, ck, b, nr_rows, nr_cols, dcol, icol, st, ck + ncol, drow, irow);
+    return launch_col_recover(rows, cols, ck, b, nr_rows, nr_cols, dcol, icol, st);
   }
   const int qpc = chamfer_qpc(nq_max, false);
   ChamferDir d0{xyz1, xyz2, dist1, idx1, nullptr, nullptr, n, m, ceil_div(n, qpc), 0};
@@ -825,7 +549,7 @@ extern "C" int pdae_chamfer_min_keys_u64(const float *queries, const float *refs
   const int qpc = chamfer_qpc(nq, false);
   ChamferDir d0{queries, refs, nullptr, nullptr, keys, nullptr, nq, nr, ceil_div(nq, qpc), ref_offset};
   ChamferDir d1{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
-  const int nsplit = (chamfer_variant() == 0 && nq > 256) ? chamfer_csplit(static_cast<long long>(b) * ceil_div(nq, 512), ceil_div(nr, 512)) : 1;
+  const int nsplit = nq > 256 ? chamfer_csplit(static_cast<long long>(b) * ceil_div(nq, 512), ceil_div(nr, 512)) : 1;
   if (nsplit > 1) {  // column-split units merge into the output keys
     fill_keys_kernel<<<static_cast<unsigned>((bq + 255) / 256), 256, 0, st>>>(keys, static_cast<long long>(bq));
     PDAE_RETURN_IF_LAUNCH_FAILED();
@@ -871,7 +595,7 @@ extern "C" int pdae_chamfer_sharded_f32(const float *xyz1, const float *xyz2_loc
   ChamferDir d1{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
   // a single scene-scale cloud gives few row blocks (100 000 points: 196 for 148 SMs): column-split units, merged
   // through the very keys this call returns
-  const int nsplit = chamfer_variant() == 0 ? chamfer_csplit(static_cast<long long>(b) * ceil_div(n, 512), ceil_div(m_local, 512)) : 1;
+  const int nsplit = chamfer_csplit(static_cast<long long>(b) * ceil_div(n, 512), ceil_div(m_local, 512));
   if (nsplit > 1) {
     fill_keys_kernel<<<static_cast<unsigned>((bn + 255) / 256), 256, 0, st>>>(keys1, static_cast<long long>(bn));
     PDAE_RETURN_IF_LAUNCH_FAILED();
@@ -879,7 +603,7 @@ extern "C" int pdae_chamfer_sharded_f32(const float *xyz1, const float *xyz2_loc
   }
   const int rc = launch_min<true>(d0, d1, b, st);
   if (rc) return rc;
-  return launch_col_recover_for_variant(xyz1, xyz2_local, ck, b, n, m_local, dist2_local, idx2_local, st);
+  return launch_col_recover(xyz1, xyz2_local, ck, b, n, m_local, dist2_local, idx2_local, st);
 }
 
 extern "C" int pdae_chamfer_unpack_keys(const uint64_t *keys, long long count, float *dist, int *idx,

@@ -6,31 +6,34 @@
 
 namespace pdae {
 
-constexpr int CH_GROUP = 16;  // argmin bookkeeping granularity: four LDS.128 steps = 16 reference points
+constexpr int CH_GROUP = 16;    // argmin bookkeeping granularity: four LDS.128 steps = 16 reference points
+constexpr int CH_THREADS = 128; // threads of a scan CTA: one 4-warp CTA already saturates an SM's FMA issue
+constexpr int CH_TILE = 512;    // reference points per shared-memory tile
+constexpr int CH_STEP = 8;      // reference points per inner step: QT*CH_STEP distances are live at once
+static_assert(3 * CH_TILE % CH_THREADS == 0, "tile must split evenly over the CTA");
+static_assert(CH_TILE % CH_GROUP == 0, "tile must hold whole bookkeeping groups");
+static_assert(CH_STEP == 8, "the running-minimum update of chamfer_min_body takes eight distances per query");
 
 // SYM: the squared distance is symmetric bit for bit (the operands of every product only change
 // sign), so one evaluation of pair (a_i, b_j) serves both directions: besides the per-query running
 // minimum the kernel reduces, for every reference point, the minimum over the warp's 32*QT queries
 // (FMNMX3 across the thread's queries, one REDUX.MIN across the lanes) and posts
-// (min bits << 32 | query-group id) with a 64-bit RED.MIN per CTA; chamfer_col_recover_kernel then
+// (min bits << 32 | query-group id) with a 64-bit RED.MIN per CTA; the column recovery of chamfer.cu then
 // finds the lowest query index inside the winning group.  Halves the FMA-pipe work of the forward.
-// One pass of a CTA: rows [row_base, row_base + QT*THREADS) of cloud `Q` (clamped to nq) against all nr points of
-// `R`.  VARGROUP selects how a warp names itself in the column keys: false = id of its 32*QT-row group
-// (row_base / (32*QT) + warp, uniform groups); true = (first row / 32) << 3 | QT, for the balanced kernel whose
-// passes have different QT.  The shared-memory buffers belong to the caller, so several instantiations can share them.
+// One pass of a CTA: rows [row_base, row_base + QT*CH_THREADS) of cloud `Q` (clamped to nq) against all nr points of
+// `R`.  A warp names itself in the column keys by the id of its 32*QT-row group, row_base / (32*QT) + warp.
+// The shared-memory buffers belong to the caller.
 // SEG (segment forward, segchamfer.cu): `R` is a segment of a packed cloud and may start at any row, so the index
 // recovery takes float4 loads only when R itself is 16-byte aligned; idx is written as ref_offset + local index.
-template <int QT, int THREADS, bool SYM, int CH_TILE, int STEP, bool VARGROUP, bool PACKED = true, bool SEG = false>
+template <int QT, bool SYM, bool SEG = false>
 __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, const float *__restrict__ R, int nq, int nr,
                                                  int row_base, size_t cloud, float *dist, int *idx, uint64_t *keys,
                                                  int ref_offset, uint64_t *colkeys, float (*tile)[3][CH_TILE],
-                                                 unsigned (*colmin)[THREADS / 32][SYM ? CH_TILE : 4], int tile_begin = 0,
+                                                 unsigned (*colmin)[CH_THREADS / 32][SYM ? CH_TILE : 4], int tile_begin = 0,
                                                  int tile_end = 0x7fffffff, bool merge = false) {
   constexpr int QPW = 32 * QT;                  // queries per warp
-  constexpr int W = THREADS / 32;
-  constexpr int LD = 3 * CH_TILE / THREADS;     // floats staged per thread per tile
-  static_assert(3 * CH_TILE % THREADS == 0, "tile must split evenly over the CTA");
-  static_assert(CH_TILE % CH_GROUP == 0, "tile must hold whole bookkeeping groups");
+  constexpr int W = CH_THREADS / 32;
+  constexpr int LD = 3 * CH_TILE / CH_THREADS;  // floats staged per thread per tile
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int qbase = row_base + warp * QPW;
@@ -55,7 +58,7 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
   auto fetch = [&](int tile_base) {
 #pragma unroll
     for (int i = 0; i < LD; ++i) {
-      const int f = tid + i * THREADS;
+      const int f = tid + i * CH_THREADS;
       const int g = tile_base * 3 + f;
       // padding: x = +inf makes the padded distance +inf, which never lowers a minimum
       pre[i] = g < nr3 ? __ldg(R + g) : ((f % 3 == 0) ? __int_as_float(0x7f800000) : 0.0f);
@@ -64,7 +67,7 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
   auto stash = [&](int buf) {
 #pragma unroll
     for (int i = 0; i < LD; ++i) {
-      const int f = tid + i * THREADS;
+      const int f = tid + i * CH_THREADS;
       const int p = f / 3, c = f - 3 * p;
       tile[buf][c][p] = pre[i];
     }
@@ -75,7 +78,7 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
     if (!SYM) return;
     uint64_t *ck = colkeys + cloud * nr;
     const int tb = tp * CH_TILE;
-    for (int j = tid; j < CH_TILE && tb + j < nr; j += THREADS) {
+    for (int j = tid; j < CH_TILE && tb + j < nr; j += CH_THREADS) {
       unsigned v = colmin[tp & 1][0][j];
       int wm = 0;
 #pragma unroll
@@ -84,8 +87,7 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
         wm = u < v ? w : wm;
         v = u < v ? u : v;
       }
-      const unsigned who = VARGROUP ? (static_cast<unsigned>((row_base + wm * QPW) >> 5) << 3) | static_cast<unsigned>(QT)
-                                    : static_cast<unsigned>(row_base / QPW + wm);
+      const unsigned who = static_cast<unsigned>(row_base / QPW + wm);
       atomicMin(reinterpret_cast<unsigned long long *>(ck + tb + j), (static_cast<unsigned long long>(v) << 32) | who);
     }
   };
@@ -101,14 +103,14 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
     if (more) fetch((tl + 1) * CH_TILE);
     if (tl > tile_begin) flush_cols(tl - 1);
     const float *sx = tile[tl & 1][0], *sy = tile[tl & 1][1], *sz = tile[tl & 1][2];
-    unsigned pend[STEP];
+    unsigned pend[CH_STEP];
 #pragma unroll
-    for (int r = 0; r < STEP; ++r) pend[r] = 0u;
+    for (int r = 0; r < CH_STEP; ++r) pend[r] = 0u;
     int pend_off = -1;
     auto store_pend = [&]() {  // lane 0 parks the warp's column minima of one step
       uint4 *dst = reinterpret_cast<uint4 *>(&colmin[tl & 1][warp][pend_off]);
 #pragma unroll
-      for (int r = 0; r < STEP; r += 4) dst[r >> 2] = make_uint4(pend[r], pend[r + 1], pend[r + 2], pend[r + 3]);
+      for (int r = 0; r < CH_STEP; r += 4) dst[r >> 2] = make_uint4(pend[r], pend[r + 1], pend[r + 2], pend[r + 3]);
     };
     const int left = nr - tl * CH_TILE;
     const int ngroups = ((left < CH_TILE ? left : CH_TILE) + CH_GROUP - 1) / CH_GROUP;
@@ -120,48 +122,35 @@ __device__ __forceinline__ void chamfer_min_body(const float *__restrict__ Q, co
 #pragma unroll
       for (int s = 0; s < QT; ++s) cur[s] = best[s];
 #pragma unroll
-      for (int h = 0; h < CH_GROUP; h += STEP) {
-        float4 X[STEP / 4], Y[STEP / 4], Z[STEP / 4];
+      for (int h = 0; h < CH_GROUP; h += CH_STEP) {
+        float4 X[CH_STEP / 4], Y[CH_STEP / 4], Z[CH_STEP / 4];
 #pragma unroll
-        for (int v = 0; v < STEP / 4; ++v) {
+        for (int v = 0; v < CH_STEP / 4; ++v) {
           X[v] = *reinterpret_cast<const float4 *>(sx + g * CH_GROUP + h + 4 * v);
           Y[v] = *reinterpret_cast<const float4 *>(sy + g * CH_GROUP + h + 4 * v);
           Z[v] = *reinterpret_cast<const float4 *>(sz + g * CH_GROUP + h + 4 * v);
         }
-        float2 dd[QT][STEP / 2];
+        float2 dd[QT][CH_STEP / 2];
 #pragma unroll
         for (int s = 0; s < QT; ++s) {
 #pragma unroll
-          for (int v = 0; v < STEP / 4; ++v) {
-            if (PACKED) {
-              dd[s][2 * v] = dist_yxz2(sub2(make_float2(X[v].x, X[v].y), qx[s]), sub2(make_float2(Y[v].x, Y[v].y), qy[s]),
-                                       sub2(make_float2(Z[v].x, Z[v].y), qz[s]));
-              dd[s][2 * v + 1] = dist_yxz2(sub2(make_float2(X[v].z, X[v].w), qx[s]), sub2(make_float2(Y[v].z, Y[v].w), qy[s]),
-                                           sub2(make_float2(Z[v].z, Z[v].w), qz[s]));
-            } else {  // scalar FADD/FMUL/FFMA (same values): experiment for the issue-slot model, see DESIGN.md
-              const float ax = qx[s].x, ay = qy[s].x, az = qz[s].x;
-              dd[s][2 * v] = make_float2(dist_yxz(__fsub_rn(X[v].x, ax), __fsub_rn(Y[v].x, ay), __fsub_rn(Z[v].x, az)),
-                                         dist_yxz(__fsub_rn(X[v].y, ax), __fsub_rn(Y[v].y, ay), __fsub_rn(Z[v].y, az)));
-              dd[s][2 * v + 1] = make_float2(dist_yxz(__fsub_rn(X[v].z, ax), __fsub_rn(Y[v].z, ay), __fsub_rn(Z[v].z, az)),
-                                             dist_yxz(__fsub_rn(X[v].w, ax), __fsub_rn(Y[v].w, ay), __fsub_rn(Z[v].w, az)));
-            }
+          for (int v = 0; v < CH_STEP / 4; ++v) {
+            dd[s][2 * v] = dist_yxz2(sub2(make_float2(X[v].x, X[v].y), qx[s]), sub2(make_float2(Y[v].x, Y[v].y), qy[s]),
+                                     sub2(make_float2(Z[v].x, Z[v].y), qz[s]));
+            dd[s][2 * v + 1] = dist_yxz2(sub2(make_float2(X[v].z, X[v].w), qx[s]), sub2(make_float2(Y[v].z, Y[v].w), qy[s]),
+                                         sub2(make_float2(Z[v].z, Z[v].w), qz[s]));
           }
-          if (STEP == 8) {
-            const float t0 = min3(dd[s][0].x, dd[s][0].y, dd[s][1].x);
-            const float t1 = min3(dd[s][1].y, dd[s][2].x, dd[s][2].y);
-            const float t2 = min3(dd[s][STEP / 2 - 1].x, dd[s][STEP / 2 - 1].y, t0);
-            cur[s] = min3(cur[s], t1, t2);
-          } else {
-            const float t0 = min3(dd[s][0].x, dd[s][0].y, dd[s][1].x);
-            cur[s] = min3(cur[s], dd[s][1].y, t0);
-          }
+          const float t0 = min3(dd[s][0].x, dd[s][0].y, dd[s][1].x);
+          const float t1 = min3(dd[s][1].y, dd[s][2].x, dd[s][2].y);
+          const float t2 = min3(dd[s][3].x, dd[s][3].y, t0);
+          cur[s] = min3(cur[s], t1, t2);
         }
-        if (SYM) {  // column minima over this warp's 32*QT queries for the STEP reference points of the step
+        if (SYM) {  // column minima over this warp's 32*QT queries for the CH_STEP reference points of the step
           // the REDUX results of the previous step are stored only now, a full step of FMA work later, so
           // their latency never stalls the warp
           if (pend_off >= 0 && lane == 0) store_pend();
 #pragma unroll
-          for (int r = 0; r < STEP; ++r) {
+          for (int r = 0; r < CH_STEP; ++r) {
             float c = (r & 1) ? dd[0][r >> 1].y : dd[0][r >> 1].x;
 #pragma unroll
             for (int s = 1; s + 1 < QT; s += 2)

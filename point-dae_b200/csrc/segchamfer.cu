@@ -17,8 +17,6 @@
 
 namespace pdae {
 
-constexpr int SEGCH_THREADS = 128;
-constexpr int SEGCH_TILE = 512;
 constexpr int SEG_LOSS_THREADS = 256;
 
 // one CTA of 1024 threads.  table0 entry (rows [r, e) of xyz1, segment [o0, o1) of xyz2); table1 the converse.
@@ -65,14 +63,14 @@ __global__ void __launch_bounds__(1024) seg_chamfer_table_kernel(const int *__re
 }
 
 template <int QT>
-__global__ void __launch_bounds__(SEGCH_THREADS, 1) seg_chamfer_min_kernel(const float *__restrict__ xyz1,
-                                                                           const float *__restrict__ xyz2,
-                                                                           const int4 *__restrict__ table0,
-                                                                           const int4 *__restrict__ table1,
-                                                                           const int *__restrict__ count, float *dist1,
-                                                                           float *dist2, int *idx1, int *idx2) {
-  __shared__ __align__(16) float tile[2][3][SEGCH_TILE];
-  __shared__ __align__(16) unsigned colmin[1][SEGCH_THREADS / 32][4];
+__global__ void __launch_bounds__(CH_THREADS, 1) seg_chamfer_min_kernel(const float *__restrict__ xyz1,
+                                                                        const float *__restrict__ xyz2,
+                                                                        const int4 *__restrict__ table0,
+                                                                        const int4 *__restrict__ table1,
+                                                                        const int *__restrict__ count, float *dist1,
+                                                                        float *dist2, int *idx1, int *idx2) {
+  __shared__ __align__(16) float tile[2][3][CH_TILE];
+  __shared__ __align__(16) unsigned colmin[1][CH_THREADS / 32][4];
   const int n0 = __ldg(count), n1 = __ldg(count + 1);
   int u = blockIdx.x;
   const bool second = u >= n0;
@@ -85,15 +83,14 @@ __global__ void __launch_bounds__(SEGCH_THREADS, 1) seg_chamfer_min_kernel(const
   const float *R = (second ? xyz1 : xyz2) + 3 * static_cast<size_t>(e.z);
   float *dist = (second ? dist2 : dist1) + e.x;
   int *idx = (second ? idx2 : idx1) + e.x;
-  chamfer_min_body<QT, SEGCH_THREADS, false, SEGCH_TILE, 8, false, true, true>(Q, R, e.y - e.x, e.w - e.z, 0, 0, dist, idx,
-                                                                                nullptr, e.z, nullptr, tile, colmin);
+  chamfer_min_body<QT, false, true>(Q, R, e.y - e.x, e.w - e.z, 0, 0, dist, idx, nullptr, e.z, nullptr, tile, colmin);
 }
 
 // rows per unit: 128 (one query per thread) when the segments average at most 256 points, as the equal-size forward
 // does for small clouds, else 512.  Host-known values only.
 static int seg_chamfer_rows(int b, int n_total, int m_total) {
   const long long big = n_total > m_total ? n_total : m_total;
-  return big <= 256LL * b ? SEGCH_THREADS : 4 * SEGCH_THREADS;
+  return big <= 256LL * b ? CH_THREADS : 4 * CH_THREADS;
 }
 static long long seg_chamfer_units0(int b, int n_total, int rows) { return (static_cast<long long>(n_total) + rows - 1) / rows + b; }
 
@@ -238,10 +235,10 @@ extern "C" int pdae_seg_chamfer_fwd_f32(const float *xyz1, int n_total, const fl
                                                dist2, idx1, idx2);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   const unsigned grid = static_cast<unsigned>(u0 + u1);
-  if (rows == SEGCH_THREADS)
-    seg_chamfer_min_kernel<1><<<grid, SEGCH_THREADS, 0, st>>>(xyz1, xyz2, table0, table1, count, dist1, dist2, idx1, idx2);
+  if (rows == CH_THREADS)
+    seg_chamfer_min_kernel<1><<<grid, CH_THREADS, 0, st>>>(xyz1, xyz2, table0, table1, count, dist1, dist2, idx1, idx2);
   else
-    seg_chamfer_min_kernel<4><<<grid, SEGCH_THREADS, 0, st>>>(xyz1, xyz2, table0, table1, count, dist1, dist2, idx1, idx2);
+    seg_chamfer_min_kernel<4><<<grid, CH_THREADS, 0, st>>>(xyz1, xyz2, table0, table1, count, dist1, dist2, idx1, idx2);
   PDAE_RETURN_IF_LAUNCH_FAILED();
   return 0;
 }

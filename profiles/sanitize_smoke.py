@@ -35,7 +35,8 @@ from pointdae_b200 import _native, chamfer_dist
 loss3 = ops.chamfer_mean_loss(d[0], d[1], True)
 ops.chamfer_loss_backward(x, y, d[2], d[3], d[0], d[1], torch.ones(1, device=dev), 0.5, 0.5, True)
 xp = x.clone().requires_grad_(True); chamfer_dist.ChamferDistanceL2()(xp, y).backward()
-_native.lib().pdae_tune_chamfer_variant(50); ops.chamfer_forward(x, y); _native.lib().pdae_tune_chamfer_variant(0)
+tc = _native.lib().pdae_tune_chamfer_tc(0, 0.0)  # FP32-pipe forward; > 128 row groups: warp-per-column recovery
+ops.chamfer_forward(cu(synth.clouds(1, 16500, seed=7)), y[:1].contiguous()); _native.lib().pdae_tune_chamfer_tc(tc, 0.0)
 q300 = cu(synth.clouds(2, 300, seed=8)); knn_cuda.KNN(20, True)(q300, q300)
 # three_nn / three_interpolate
 dist3, idx3 = pointnet2_utils.three_nn(y, cen)
