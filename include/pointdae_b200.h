@@ -275,12 +275,12 @@ int pdae_chamfer_tc_shares(int b, int n, int m, int grid, long long *bounds_out,
  * trace: optional 256 x 6 int64 of clock64 stamps of CTA 0's first tiles (pipeline timeline), or NULL.                     */
 int pdae_chamfer_tc_probe(const float *xyz1, const float *xyz2, int b, int n, int m, float *dist1, float *dist2, int *idx1,
                           int *idx2, unsigned long long *stats4, long long *trace, pdae_stream_t stream);
-/* kNN / Group (dim 3, k <= 64): impl 4 = multi-query warps + TMA tile prefetch (default), 3 = the first-generation
- * kernel (kept for A/B measurements); qw queries per warp (1/2/4), nw warps per CTA (4/8), tile points per shared-memory
- * tile, nz chunks along the reference cloud (needs the workspace), tma 0/1, spec 0/1 (warp-specialised CTAs with a
- * producer warp; 8-warp CTAs only).  -1 = automatic.  Same results for every
- * setting (tests/test_gpu_parity.py).  Environment: PDAE_KNN_IMPL, PDAE_KNN4_{QW,NW,TILE,NZ,TMA}.                    */
-int pdae_tune_knn(int impl, int qw, int nw, int tile, int nz, int tma, int spec);
+/* tuning / test hook of kNN / Group (dim 3, k <= 64): form = (queries per warp, warps per CTA) of the kernel: 0 = (4, 8)
+ * warp-specialised (7 compute warps + a producer warp), 1 = (4, 8), 2 = (4, 4), 3 = (2, 4); tile points per
+ * shared-memory tile, nz chunks along the reference cloud (needs the workspace), tma 0/1.  -1 = automatic.  Same results
+ * for every setting (tests/test_gpu_knn4.py).  Returns 0, or PDAE_E_INVALID for a form outside -1..3 (the setting is
+ * then unchanged).  Not thread-safe.                                                                                 */
+int pdae_tune_knn(int form, int tile, int nz, int tma);
 
 /* reference-set sharding (scene-scale clouds, SURVEY.md 8e; new, no reference counterpart):
  * one direction, queries (b,nq,3) against the local slice refs (b,nr,3) whose first point has

@@ -74,7 +74,7 @@ SIGNATURES = {
     "pdae_tune_chamfer_split": (_i, [_i]),
     "pdae_tune_chamfer_tc": (_i, [_i, _f]),
     "pdae_chamfer_tc_probe": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "pdae_tune_knn": (_i, [_i, _i, _i, _i, _i, _i, _i]),
+    "pdae_tune_knn": (_i, [_i, _i, _i, _i]),
     "pdae_chamfer_tc_shares": (_i, [_i, _i, _i, _i, _vp, _vp]),
     "pdae_chamfer_loss_workspace_bytes": (_sz, []),
     "pdae_chamfer_loss_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),

@@ -66,7 +66,7 @@ __device__ __forceinline__ void affine_seq(const float *__restrict__ mats, int t
   }
 }
 
-// optional second output of the fused Group epilogue (knn3.cu): the corrupted copy of every patch.
+// optional second output of the fused Group epilogue (knn4.cu, patchify.cu): the corrupted copy of every patch.
 struct GroupAffine {
   const float *mats;  // (b, t, 3, 3)
   int t;
@@ -98,13 +98,9 @@ inline int sm_count() {
 // cross-file internals
 // knn.cu: planar-input, any-channel-count DGCNN kNN (warp-select kernel); used directly for small c.
 int feat_knn_generic(const float *x, int b, int c, int n, int k, int64_t *idx, cudaStream_t st);
-// knn3.cu: 3-D fast path (k <= 64): row-major points with optional fused Group output, and planar (b,3,n) self-kNN.
-int knn3_points(const float *ref, const float *query, int b, int r, int q, int k, int out_kq, float *dist, int64_t *idx,
-                float *group, cudaStream_t st, uint64_t *keys = nullptr, uint32_t ref_offset = 0u, int raw_group = 0,
-                const GroupAffine *affine = nullptr);
-int knn3_planar(const float *x, int b, int n, int k, int64_t *idx, cudaStream_t st);
-// knn4.cu: second-generation 3-D fast path (multi-query warps, segment-minima threshold, TMA tile prefetch, chunks along
-// the reference cloud through an optional caller-owned workspace); same contract and results as knn3.cu.
+// knn4.cu: 3-D fast path, k <= 64 (multi-query warps, segment-minima threshold, TMA tile prefetch, chunks along the
+// reference cloud through an optional caller-owned workspace): row-major points with optional fused Group output, and
+// planar (b,3,n) self-kNN; same results as knn.cu.  PDAE_E_UNSUPPORTED when one chunk exceeds its 16-bit step numbers.
 int knn4_points(const float *ref, const float *query, int b, int r, int q, int k, int out_kq, float *dist, int64_t *idx,
                 float *group, cudaStream_t st, uint64_t *keys = nullptr, uint32_t ref_offset = 0u, int raw_group = 0,
                 const GroupAffine *affine = nullptr, void *ws = nullptr, size_t ws_bytes = 0);
@@ -119,8 +115,6 @@ int chamfer_tc_forward(const float *xyz1, const float *xyz2, int b, int n, int m
 bool chamfer_tc_sharded_applies(int b, int n, int m_local);
 int chamfer_tc_sharded(const float *xyz1, const float *xyz2_local, int b, int n, int m_local, int ref_offset, uint64_t *keys1,
                        float *dist2_local, int *idx2_local, void *workspace, size_t workspace_bytes, cudaStream_t st);
-// which generation serves dim-3, k <= 64 searches: 4 (default) or 3 (PDAE_KNN_IMPL=3, kept for A/B measurements)
-int knn3d_impl();
 
 }  // namespace pdae
 

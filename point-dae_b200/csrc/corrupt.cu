@@ -10,7 +10,7 @@
 //   * pdae_affine_points_f32 applies the whole chain to patches and centres in ONE pass (drop-in for
 //     `corrupt_data` on tensors the model already formed), and
 //   * pdae_group_affine_f32 produces the clean and the corrupted, re-centred patches straight from the kNN
-//     epilogue of the patchifier (knn3.cu), so the absolute-coordinate copies never exist in memory.
+//     epilogue of the patchifier (knn4.cu), so the absolute-coordinate copies never exist in memory.
 // Bound: HBM/L2 streaming, 24 B per point (12 in, 12 out); the arithmetic is 9*t FMA-pipe ops per point.
 #include "common.cuh"
 
@@ -89,8 +89,7 @@ extern "C" int pdae_group_affine_f32(const float *xyz, const float *center, cons
   if (m <= 64) {
     // t == 0 still takes the fused branch (identity chain): point at any valid address, never dereferenced
     const GroupAffine aff{mats ? mats : xyz, t, t_neighborhood, t_center};
-    return knn3d_impl() == 3 ? knn3_points(xyz, center, b, n, g, m, 0, nullptr, idx, neighborhood, st, nullptr, 0u, 0, &aff)
-                             : knn4_points(xyz, center, b, n, g, m, 0, nullptr, idx, neighborhood, st, nullptr, 0u, 0, &aff);
+    return knn4_points(xyz, center, b, n, g, m, 0, nullptr, idx, neighborhood, st, nullptr, 0u, 0, &aff);
   }
   const int rc = pdae_group_f32(xyz, center, b, n, g, m, idx, neighborhood, stream);
   if (rc) return rc;

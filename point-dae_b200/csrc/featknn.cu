@@ -359,232 +359,25 @@ __global__ void __launch_bounds__(FT_THREADS, 2) feat_knn_tiled_kernel(const flo
   }
 }
 
-// ---- the same search in two kernels through a materialised distance matrix (default when a workspace is given) ------
+// ---- the same search through a materialised distance matrix (default when a workspace is given) -------------------------
 // ncu on the fused kernel above (C = 64, N = 2048, B = 16): 364 M warp instructions of which only 134 M are the packed
 // FMA work -- the streaming selection (about k ln(N/k) + k insertions per query, a ballot / queue append per candidate,
 // a bitonic flush every 32) costs more issue slots than the distances.  On B200 writing the B x N x N fp32 matrix the
-// reference also materialises is cheap (268 MB at that shape: ~40 us each way at the measured 6.5 TB/s), so:
-//   kernel A (feat_dist_tiled_kernel): the register-tiled distance computation of the kernel above, distances stored
-//     straight to global memory (coalesced 128-bit stores); every thread keeps the two smallest distances it has seen per
-//     query (3 FMNMX per value), and at the end the 32 per-thread minima of a query -- real distances of 32 distinct
-//     points -- are sorted by one warp: their k-th smallest is an upper bound tau0 of the true k-th distance (k <= 32);
-//   kernel B (feat_select_kernel): one warp per query re-reads its row (L2 / HBM stream), appends the ~1.2 k points with
-//     d <= tau0 to lane-private lists with predicated stores, compacts, sorts 64-bit (distance, index) keys and writes
-//     the first k -- the pass 2 of knn3.cu.  Overflow (mass ties) -> exact streaming warp-select over the stored row.
-// Same distances, same (distance, lower index first) order: bit-identical to the fused kernel and the oracle.
-constexpr int FS_LC = 8;  // lane-private candidate slots of kernel B
-
-__global__ void __launch_bounds__(FT_THREADS, 2) feat_dist_tiled_kernel(const float *__restrict__ x, int c, int n, int k,
-                                                                        float *__restrict__ dmat /*(b, n, n)*/,
-                                                                        float *__restrict__ tau /*(b, n)*/) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float *ops0 = reinterpret_cast<float *>(smem_raw);                 // operand stage, 2 buffers
-  float *mins = ops0 + 2 * FT_K * (FT_Q + FT_R);                     // [FT_Q][32] per-thread minima, written at the end
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int ty = tid >> 4, tx = tid & 15;  // 16 x 16 threads: 4 queries x (4 + 4) references each
-  const int cloud = blockIdx.y;
-  const int q0 = blockIdx.x * FT_Q;
-  const float *__restrict__ X = x + static_cast<size_t>(cloud) * c * n;
-  float *__restrict__ D = dmat + static_cast<size_t>(cloud) * n * n;
-  const float INF = __int_as_float(0x7f800000);
-  constexpr int LD = FT_K * (FT_Q + FT_R) / FT_THREADS;
-
-  const int nst = (c + FT_K - 1) / FT_K;
-  const int ntiles = (n + FT_R - 1) / FT_R;
-  const int total = nst * ntiles;
-  float pre[LD];
-  const float *__restrict__ pq = X + static_cast<size_t>(tid >> 6) * n + q0 + (tid & 63);
-  const float *__restrict__ pr = X + static_cast<size_t>(tid >> 7) * n + (tid & 127);
-  const bool q_ok = q0 + (tid & 63) < n;
-  auto fetch = [&](int st) {
-    const int tile_i = st / nst;
-    const int r0 = tile_i * FT_R, c0 = (st - tile_i * nst) * FT_K;
-    const int kc = c - c0;
-    const bool r_ok = r0 + (tid & 127) < n;
-    const float *bq = pq + static_cast<size_t>(c0) * n;
-    const float *br = pr + static_cast<size_t>(c0) * n + r0;
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      pre[i] = (q_ok && (tid >> 6) + 4 * i < kc) ? __ldg(bq + static_cast<size_t>(4 * i) * n) : 0.f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-      pre[4 + i] = (r_ok && (tid >> 7) + 2 * i < kc) ? __ldg(br + static_cast<size_t>(2 * i) * n) : 0.f;
-  };
-  auto stash = [&](int buf) {
-    float *dst = ops0 + buf * FT_K * (FT_Q + FT_R);
-#pragma unroll
-    for (int i = 0; i < LD; ++i) dst[tid + i * FT_THREADS] = pre[i];
-  };
-
-  float m0[4], m1[4];
-#pragma unroll
-  for (int a = 0; a < 4; ++a) m0[a] = m1[a] = INF;
-  const bool vec = (n & 3) == 0;
-
-  fetch(0);
-  stash(0);
-  __syncthreads();
-  float2 acc[4][4];
-  for (int st = 0; st < total; ++st) {
-    const int tile_i = st / nst, si = st - tile_i * nst;
-    const int r0 = tile_i * FT_R, c0 = si * FT_K;
-    if (si == 0) {
-#pragma unroll
-      for (int a = 0; a < 4; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b) acc[a][b] = make_float2(0.f, 0.f);
-    }
-    if (st + 1 < total) fetch(st + 1);
-    const float *qs = ops0 + (st & 1) * FT_K * (FT_Q + FT_R);
-    const float *rs = qs + FT_K * FT_Q;
-    const int kc = (c - c0) < FT_K ? (c - c0) : FT_K;
-#pragma unroll 4
-    for (int cc = 0; cc < kc; ++cc) {
-      const float4 qv = *reinterpret_cast<const float4 *>(qs + cc * FT_Q + ty * 4);
-      const float4 ra = *reinterpret_cast<const float4 *>(rs + cc * FT_R + tx * 4);
-      const float4 rb = *reinterpret_cast<const float4 *>(rs + cc * FT_R + 64 + tx * 4);
-      const float2 rp[4] = {make_float2(ra.x, ra.y), make_float2(ra.z, ra.w), make_float2(rb.x, rb.y), make_float2(rb.z, rb.w)};
-      const float qq[4] = {qv.x, qv.y, qv.z, qv.w};
-#pragma unroll
-      for (int a = 0; a < 4; ++a) {
-        const float2 q2 = make_float2(qq[a], qq[a]);
-#pragma unroll
-        for (int b = 0; b < 4; ++b) {
-          const float2 t = sub2(rp[b], q2);
-          acc[a][b] = fma2(t, t, acc[a][b]);
-        }
-      }
-    }
-    if (st + 1 < total) stash((st + 1) & 1);
-    if (si == nst - 1) {
-      // all channels of this reference tile done: store the thread's 4 x 8 distances and fold them into its minima
-      const int ra0 = r0 + tx * 4, rb0 = r0 + 64 + tx * 4;  // first reference of each half
-#pragma unroll
-      for (int a = 0; a < 4; ++a) {
-        float v[8] = {acc[a][0].x, acc[a][0].y, acc[a][1].x, acc[a][1].y, acc[a][2].x, acc[a][2].y, acc[a][3].x, acc[a][3].y};
-        const int qg = q0 + ty * 4 + a;
-        if (r0 + FT_R > n) {  // last, partial tile: references past the cloud must neither be stored nor compete
-#pragma unroll
-          for (int e = 0; e < 8; ++e) v[e] = ((e < 4 ? ra0 + e : rb0 + e - 4) < n) ? v[e] : INF;
-        }
-        if (qg < n) {
-          float *row = D + static_cast<size_t>(qg) * n;
-          if (vec) {
-            if (ra0 < n) *reinterpret_cast<float4 *>(row + ra0) = make_float4(v[0], v[1], v[2], v[3]);
-            if (rb0 < n) *reinterpret_cast<float4 *>(row + rb0) = make_float4(v[4], v[5], v[6], v[7]);
-          } else {
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              const int r = e < 4 ? ra0 + e : rb0 + e - 4;
-              if (r < n) row[r] = v[e];
-            }
-          }
-        }
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {  // two smallest of everything this thread has seen for query a
-          const float t1 = fmaxf(m0[a], v[e]);
-          m0[a] = fminf(m0[a], v[e]);
-          m1[a] = fminf(m1[a], t1);
-        }
-      }
-    }
-    __syncthreads();
-  }
-  // ---- tau0 per query: k-th smallest of the 32 per-thread minima (16 threads x 2) ------------------------------------
-#pragma unroll
-  for (int a = 0; a < 4; ++a) {
-    mins[(ty * 4 + a) * 32 + 2 * tx] = m0[a];
-    mins[(ty * 4 + a) * 32 + 2 * tx + 1] = m1[a];
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (int i = 0; i < 8; ++i) {
-    const int ql = warp * 8 + i;
-    float sv[1] = {mins[ql * 32 + lane]};
-    warp_sort_multi_f32<1>(sv, lane);
-    const float t = __shfl_sync(0xffffffffu, sv[0], k - 1);
-    if (lane == 0 && q0 + ql < n) tau[static_cast<size_t>(cloud) * n + q0 + ql] = t;
-  }
-}
-
-__global__ void __launch_bounds__(256) feat_select_kernel(const float *__restrict__ dmat, const float *__restrict__ tau,
-                                                          int n, int k, int64_t *__restrict__ idx) {
-  __shared__ uint64_t queue_all[8][64];
-  __shared__ uint64_t lq_all[8][FS_LC * 32];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q = blockIdx.x * 8 + warp;
-  const size_t cloud = blockIdx.y;
-  if (q >= n) return;
-  const float *__restrict__ row = dmat + (cloud * n + q) * n;
-  const float tau0 = __ldg(tau + cloud * n + q);
-  uint64_t *queue = queue_all[warp], *lq = lq_all[warp];
-  const bool degenerate = !(tau0 < __int_as_float(0x7f800000));
-  int cnt = 0;
-  if ((n & 3) == 0) {
-    for (int j0 = 0; j0 < n; j0 += 128) {
-      const int j = j0 + 4 * lane;
-      if (j < n) {
-        const float4 d = __ldcs(reinterpret_cast<const float4 *>(row + j));
-        const float v[4] = {d.x, d.y, d.z, d.w};
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const bool cnd = v[e] <= tau0;
-          if (cnd && cnt < FS_LC) lq[cnt * 32 + lane] = pack_key(v[e], static_cast<uint32_t>(j + e));
-          cnt += cnd;
-        }
-      }
-    }
-  } else {
-    for (int j = lane; j < n; j += 32) {
-      const float v = __ldcs(row + j);
-      const bool cnd = v <= tau0;
-      if (cnd && cnt < FS_LC) lq[cnt * 32 + lane] = pack_key(v, static_cast<uint32_t>(j));
-      cnt += cnd;
-    }
-  }
-  if (degenerate) cnt = FS_LC + 1;
-  int incl = cnt;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int t = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += t;
-  }
-  const int totalc = __shfl_sync(0xffffffffu, incl, 31);
-  const bool overflow = __any_sync(0xffffffffu, cnt > FS_LC) || totalc > 64;
-  uint64_t keys[2];
-  if (!overflow) {
-    const int off = incl - cnt;
-    for (int i = 0; i < cnt; ++i) queue[off + i] = lq[i * 32 + lane];
-    __syncwarp();
-#pragma unroll
-    for (int e = 0; e < 2; ++e) keys[e] = (e * 32 + lane) < totalc ? queue[e * 32 + lane] : KEY_INF;
-    __syncwarp();
-    warp_sort_multi<2>(keys, lane);
-  } else {  // exact fallback: streaming warp-select over the stored row
-    WarpSelect<1> sel;
-    sel.init();
-    for (int j0 = 0; j0 < n; j0 += 32) {
-      const int j = j0 + lane;
-      const bool in = j < n;
-      const uint64_t key = in ? pack_key(__ldg(row + j), static_cast<uint32_t>(j)) : KEY_INF;
-      sel.offer(in && key < sel.tau, key, queue, lane, 0, k - 1);
-    }
-    sel.finish(queue, lane);
-    keys[0] = sel.L[0];
-    keys[1] = KEY_INF;
-  }
-  if (lane < k) idx[(cloud * n + q) * k + lane] = static_cast<int64_t>(static_cast<uint32_t>(keys[0]));
-}
-
-// ---- symmetric form of the matrix path (default) -------------------------------------------------------------------------
+// reference also materialises is cheap (268 MB at that shape: ~40 us each way at the measured 6.5 TB/s), so the distances
+// go to global memory and a warp per query selects from its stored row.
 // The search is a SELF-kNN: d(i,j) and d(j,i) are the same bits (the operands of every subtraction only change sign), so
-// each unordered pair is evaluated once.  A CTA still owns 64 queries but walks only the 128-point reference tiles from
-// its own diagonal tile on; besides its rows it stores the TRANSPOSED block D[r][q] (for every reference four consecutive
+// each unordered pair is evaluated once.  A CTA owns 64 queries and walks only the 128-point reference tiles from its own
+// diagonal tile on; besides its rows it stores the TRANSPOSED block D[r][q] (for every reference four consecutive
 // queries = one 128-bit store; the two 16-row halves of a warp fill whole 32-byte sectors), which is exactly the part of
 // the lower triangle no CTA computes directly.  Executed FMA work: (ntiles + 1) / (2 ntiles) of the full matrix.
-// The threshold tau0 can no longer come from this kernel (a CTA does not see its rows' lower-triangle distances), so the
-// selection kernel takes it from the stored row itself: 64 segment minima per query (one FMNMX3 per two values),
-// k-th smallest by one 32-bit bitonic sort -- the pass 1 of knn4.cu -- then the row is read again (L1 / L2 hit).
+// A CTA does not see its rows' lower-triangle distances, so the selection kernel takes its threshold tau0 from the stored
+// row itself: 64 segment minima per query (one FMNMX3 per two values), k-th smallest by one 32-bit bitonic sort -- the
+// pass 1 of knn4.cu -- then the row is read again (L1 / L2 hit), the ~1.2 k points with d <= tau0 go to lane-private
+// lists (predicated stores), are compacted, sorted as 64-bit (distance, index) keys and the first k written.  Overflow
+// (mass ties) -> exact streaming warp-select over the stored row.  Same distances, same (distance, lower index first)
+// order: bit-identical to the fused kernel and the oracle.
+constexpr int FS_LC = 8;  // lane-private candidate slots of the selection kernel
+
 __global__ void __launch_bounds__(FT_THREADS, 2) feat_dist_sym_kernel(const float *__restrict__ x, int c, int n,
                                                                       float *__restrict__ dmat /*(b, n, n)*/) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -809,26 +602,16 @@ static int launch_feat_knn_matrix(const float *x, int b, int c, int n, int k, in
   long long chunk = static_cast<long long>(workspace_bytes / per);
   if (chunk < 1) return PDAE_E_WORKSPACE;
   if (chunk > 65535) chunk = 65535;
-  const size_t smem = (2 * static_cast<size_t>(FT_K) * (FT_Q + FT_R) + static_cast<size_t>(FT_Q) * 32) * sizeof(float);
+  const size_t smem = 2 * static_cast<size_t>(FT_K) * (FT_Q + FT_R) * sizeof(float);
   for (long long b0 = 0; b0 < b; b0 += chunk) {
     const int nb = static_cast<int>(b - b0 < chunk ? b - b0 : chunk);
     float *dmat = static_cast<float *>(workspace);
-    float *tau = dmat + static_cast<size_t>(nb) * n * n;
-    const dim3 ga(ceil_div(n, FT_Q), nb);
-    const dim3 gb(ceil_div(n, 8), nb);
-    static const bool full_matrix = getenv("PDAE_FEATKNN_FULL") != nullptr;  // A/B hook: the round-1 form (every pair twice)
-    if (full_matrix) {
-      feat_dist_tiled_kernel<<<ga, FT_THREADS, smem, st>>>(x + static_cast<size_t>(b0) * c * n, c, n, k, dmat, tau);
-      PDAE_RETURN_IF_LAUNCH_FAILED();
-      feat_select_kernel<<<gb, 256, 0, st>>>(dmat, tau, n, k, idx + static_cast<size_t>(b0) * n * k);
-      PDAE_RETURN_IF_LAUNCH_FAILED();
-    } else {
-      if (ga.x > 65535) return PDAE_E_UNSUPPORTED;
-      feat_dist_sym_kernel<<<dim3(ga.y, ga.x), FT_THREADS, smem, st>>>(x + static_cast<size_t>(b0) * c * n, c, n, dmat);
-      PDAE_RETURN_IF_LAUNCH_FAILED();
-      feat_select2_kernel<<<gb, 256, 0, st>>>(dmat, n, k, idx + static_cast<size_t>(b0) * n * k);
-      PDAE_RETURN_IF_LAUNCH_FAILED();
-    }
+    const int nqb = ceil_div(n, FT_Q);
+    if (nqb > 65535) return PDAE_E_UNSUPPORTED;
+    feat_dist_sym_kernel<<<dim3(nb, nqb), FT_THREADS, smem, st>>>(x + static_cast<size_t>(b0) * c * n, c, n, dmat);
+    PDAE_RETURN_IF_LAUNCH_FAILED();
+    feat_select2_kernel<<<dim3(ceil_div(n, 8), nb), 256, 0, st>>>(dmat, n, k, idx + static_cast<size_t>(b0) * n * k);
+    PDAE_RETURN_IF_LAUNCH_FAILED();
   }
   return 0;
 }
@@ -852,10 +635,10 @@ using namespace pdae;
 extern "C" int pdae_feat_knn_f32(const float *x, int b, int c, int n, int k, int64_t *idx, pdae_stream_t stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (b > 0 && n > 0 && x && idx && c >= 8 && k >= 1 && k <= 32 && k <= n) return launch_feat_knn_tiled(x, b, c, n, k, idx, st);
-  return feat_knn_generic(x, b, c, n, k, idx, st);  // c == 3 -> knn3 planar fast path; other shapes -> streaming warp-select
+  return feat_knn_generic(x, b, c, n, k, idx, st);  // c == 3 -> knn4 planar fast path; other shapes -> streaming warp-select
 }
 
-// workspace of the matrix path: whole clouds' worth of (n x n distances + n thresholds), capped at 1 GiB (the host
+// workspace of the matrix path: whole clouds' worth of (n x n distances + n spare floats), capped at 1 GiB (the host
 // function walks the batch in chunks); 0 when the shape takes another path or one cloud alone exceeds the cap.
 extern "C" size_t pdae_feat_knn_workspace_bytes(int b, int c, int n, int k) {
   if (b <= 0 || n <= 0 || c < 8 || k < 1 || k > 32 || k > n) return 0;
@@ -870,7 +653,7 @@ extern "C" int pdae_feat_knn_ws_f32(const float *x, int b, int c, int n, int k, 
                                     size_t workspace_bytes, pdae_stream_t stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (b > 0 && n > 0 && x && idx && c >= 8 && k >= 1 && k <= 32 && k <= n && workspace &&
-      workspace_bytes >= feat_matrix_bytes_per_cloud(n) && getenv("PDAE_FEATKNN_FUSED") == nullptr)
+      workspace_bytes >= feat_matrix_bytes_per_cloud(n))
     return launch_feat_knn_matrix(x, b, c, n, k, idx, workspace, workspace_bytes, st);
   return pdae_feat_knn_f32(x, b, c, n, k, idx, stream);
 }

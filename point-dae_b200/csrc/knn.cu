@@ -175,10 +175,13 @@ using namespace pdae;
 
 static int knn_dim3(const float *ref, const float *query, int b, int r, int q, int k, int out_kq, float *dist, int64_t *idx,
                     float *group, cudaStream_t st, uint64_t *keys, uint32_t off, int raw, void *ws, size_t ws_bytes) {
-  if (knn3d_impl() == 3) return knn3_points(ref, query, b, r, q, k, out_kq, dist, idx, group, st, keys, off, raw);
   const int rc = knn4_points(ref, query, b, r, q, k, out_kq, dist, idx, group, st, keys, off, raw, nullptr, ws, ws_bytes);
-  // clouds beyond the 16-bit step numbers of one chunk (> 8 M points without a workspace): first-generation kernel
-  return rc == PDAE_E_UNSUPPORTED ? knn3_points(ref, query, b, r, q, k, out_kq, dist, idx, group, st, keys, off, raw) : rc;
+  if (rc != PDAE_E_UNSUPPORTED) return rc;
+  // clouds beyond the 16-bit step numbers of one chunk (> 8 M points without a workspace): streaming warp-select
+  KnnArgs a{ref, query, dist, idx, group, keys, off, raw, r, q, 3, k, 0, 1, out_kq};
+  const int prc = knn_plan(a, b);
+  if (prc) return prc;
+  return launch_knn<3, false>(a, b, st);
 }
 
 extern "C" size_t pdae_knn_workspace_bytes(int b, int r, int q, int dim, int k) {
@@ -354,7 +357,7 @@ int pdae::feat_knn_generic(const float *x, int b, int c, int n, int k, int64_t *
   if (b == 0 || n == 0) return 0;
   if (k > n || k > KNN_MAX_K) return PDAE_E_INVALID;
   if (!x || !idx) return PDAE_E_INVALID;
-  if (c == 3 && k <= 64) return knn3d_impl() == 3 ? knn3_planar(x, b, n, k, idx, st) : knn4_planar(x, b, n, k, idx, st);
+  if (c == 3 && k <= 64) return knn4_planar(x, b, n, k, idx, st);
   KnnArgs a{x, nullptr, nullptr, idx, nullptr, nullptr, 0u, 0, n, n, c, k, 0, 1, 0};
   const int rc = knn_plan(a, b);
   if (rc) return rc;

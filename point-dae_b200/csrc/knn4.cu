@@ -1,11 +1,11 @@
 // knn4.cu -- 3-D k nearest neighbours, second-generation fast path (knn_cuda.KNN with dim 3, the fused Group tail,
-// the first DGCNN EdgeConv layer).  Same results as knn.cu / knn3.cu bit for bit (ascending by (squared distance,
+// the first DGCNN EdgeConv layer).  Same results as knn.cu bit for bit (ascending by (squared distance,
 // index), distance = fma(dz,dz, fma(dy,dy, dx*dx)) like KNN_CUDA's `ssd += tmp*tmp` loop); the schedule is built around
 // the FP32 FMA pipe instead of the selection logic:
 //
 //   * a warp owns QW queries AT ONCE: every lane loads four adjacent reference points per step (one LDS.128 per plane)
 //     and evaluates them against all QW queries, so the shared-memory traffic and the address arithmetic are paid once
-//     per QW x 128 pair evaluations (knn3: once per 64);
+//     per QW x 128 pair evaluations;
 //   * pass 1 keeps, per lane and query, E running minima over disjoint subsets of the lane's points ("segments":
 //     32*E per query, one FMNMX3 per two pair evaluations).  The minima are distances of distinct points, so their k-th
 //     smallest (one fp32 bitonic sort across the warp) is an upper bound tau of the true k-th distance, and a tight one
@@ -22,8 +22,6 @@
 //     the reference cloud into grid.z chunks; each chunk emits its k best keys and a warp-per-query merge kernel
 //     finishes (the key order makes the merge exact), so every SM has work.
 #include "knn_select.cuh"
-
-#include <cstdlib>
 
 namespace pdae {
 
@@ -641,21 +639,18 @@ struct Knn4Plan {
   int qw, nw, tile, nz, tma, spec, dense_in_stage;
 };
 
-// Tuning hooks (profiles/tune_knn.py): pdae_tune_knn / PDAE_KNN4_{QW,NW,TILE,NZ,TMA,SPEC} override the plan; -1 = automatic.
-struct Knn4Tune {
-  int impl, qw, nw, tile, nz, tma, spec;
+// The (queries per warp, warps per CTA, warp-specialised) forms the plan chooses from, numbered as pdae_tune_knn takes them.
+struct Knn4Form {
+  int qw, nw, spec;
 };
-static int env_int(const char *name, int dflt) {
-  const char *s = std::getenv(name);
-  return s && *s ? std::atoi(s) : dflt;
-}
-static Knn4Tune &knn4_tune() {
-  static Knn4Tune t{env_int("PDAE_KNN_IMPL", 4), env_int("PDAE_KNN4_QW", -1), env_int("PDAE_KNN4_NW", -1),
-                    env_int("PDAE_KNN4_TILE", -1), env_int("PDAE_KNN4_NZ", -1), env_int("PDAE_KNN4_TMA", -1),
-                    env_int("PDAE_KNN4_SPEC", -1)};
-  return t;
-}
-int knn3d_impl() { return knn4_tune().impl == 3 ? 3 : 4; }
+constexpr int KNN4_NFORMS = 4;
+static constexpr Knn4Form KNN4_FORMS[KNN4_NFORMS] = {{4, 8, 1}, {4, 8, 0}, {4, 4, 0}, {2, 4, 0}};
+
+// Tuning hook (profiles/tune_knn.py, tests/test_gpu_knn4.py): pdae_tune_knn overrides the plan; -1 = automatic.
+struct Knn4Tune {
+  int form, tile, nz, tma;
+};
+static Knn4Tune knn4_tune{-1, -1, -1, -1};
 
 static size_t knn4_smem_bytes(int e, const Knn4Plan &p) {
   const size_t per_warp = e == 2 ? Knn4Smem<2>::per_warp(p.qw, p.dense_in_stage) : Knn4Smem<4>::per_warp(p.qw, p.dense_in_stage);
@@ -666,7 +661,7 @@ static size_t knn4_smem_bytes(int e, const Knn4Plan &p) {
 static Knn4Plan knn4_plan(int b, int r, int q, int k, bool aligned, bool have_ws) {
   Knn4Plan p;
   const int e = k <= 32 ? 2 : 4;
-  const Knn4Tune &tn = knn4_tune();
+  const Knn4Tune &tn = knn4_tune;
   // streamed clouds that cannot fill the GPU with CTAs (scene scale: few queries, long cloud): warp-specialised CTAs
   // (7 compute warps + 1 producer, two plane buffers) keep the lone CTA of an SM computing while tiles are converted;
   // with several CTAs per SM the conversions already overlap with other CTAs' scans and the eighth compute warp wins
@@ -674,7 +669,6 @@ static Knn4Plan knn4_plan(int b, int r, int q, int k, bool aligned, bool have_ws
   const bool streamed = r > 2048;
   const long long ctas_plain = static_cast<long long>(b) * ((q + 31) / 32);
   p.spec = streamed && ctas_plain < 148 * 3 ? 1 : 0;
-  if (tn.spec >= 0) p.spec = tn.spec;
   p.tile = tn.tile > 0 ? tn.tile : 2048;
   if (p.tile < 256) p.tile = 256;
   p.tile = (p.tile + 255) & ~255;
@@ -687,14 +681,7 @@ static Knn4Plan knn4_plan(int b, int r, int q, int k, bool aligned, bool have_ws
   p.nw = 4;
   if (q >= 256 && nq >= 148LL * 8 * 4 * 2) p.nw = 8;
   if (streamed) p.qw = 4, p.nw = 8;
-  if (tn.qw > 0) p.qw = tn.qw;
-  if (tn.nw > 0) p.nw = tn.nw;
-  if (p.qw != 1 && p.qw != 2 && p.qw != 4) p.qw = 4;
-  if (p.nw != 4 && p.nw != 8) p.nw = 4;
-  if (p.spec) {  // instantiated shapes
-    p.nw = 8;
-    if (p.qw == 1) p.qw = 2;
-  }
+  if (tn.form >= 0) p.qw = KNN4_FORMS[tn.form].qw, p.nw = KNN4_FORMS[tn.form].nw, p.spec = KNN4_FORMS[tn.form].spec;
   // the TMA landing zone costs a tile of shared memory: worth it only when tiles are streamed
   p.tma = aligned && (r & 3) == 0 && ntiles > 1;
   if (tn.tma >= 0) p.tma = tn.tma;
@@ -720,9 +707,8 @@ static Knn4Plan knn4_plan(int b, int r, int q, int k, bool aligned, bool have_ws
       if (cost < best * 0.97) best = cost, p.nz = nz;
     }
   }
-  const int nz_env = tn.nz;
-  if (nz_env > 0 && have_ws) {
-    const int tpc = (ntiles + nz_env - 1) / nz_env;
+  if (tn.nz > 0 && have_ws) {
+    const int tpc = (ntiles + tn.nz - 1) / tn.nz;
     p.nz = (ntiles + tpc - 1) / tpc;
     if (p.nz > 16) p.nz = 16;
   }
@@ -751,18 +737,11 @@ static int knn4_launch_cfg(Knn4Args a, int b, const Knn4Plan &p, cudaStream_t st
 
 template <bool PLANAR, int E, bool AFF>
 static int knn4_launch_e(const Knn4Args &a, int b, const Knn4Plan &p, cudaStream_t st) {
-  if (p.spec) {
-    if (p.qw == 4) return knn4_launch_cfg<PLANAR, E, 4, 8, AFF, true>(a, b, p, st);
-    return knn4_launch_cfg<PLANAR, E, 2, 8, AFF, true>(a, b, p, st);
-  }
-  if (p.nw == 8) {
-    if (p.qw == 4) return knn4_launch_cfg<PLANAR, E, 4, 8, AFF, false>(a, b, p, st);
-    if (p.qw == 2) return knn4_launch_cfg<PLANAR, E, 2, 8, AFF, false>(a, b, p, st);
-    return knn4_launch_cfg<PLANAR, E, 1, 8, AFF, false>(a, b, p, st);
-  }
+  // the plan yields one of KNN4_FORMS
+  if (p.spec) return knn4_launch_cfg<PLANAR, E, 4, 8, AFF, true>(a, b, p, st);
+  if (p.nw == 8) return knn4_launch_cfg<PLANAR, E, 4, 8, AFF, false>(a, b, p, st);
   if (p.qw == 4) return knn4_launch_cfg<PLANAR, E, 4, 4, AFF, false>(a, b, p, st);
-  if (p.qw == 2) return knn4_launch_cfg<PLANAR, E, 2, 4, AFF, false>(a, b, p, st);
-  return knn4_launch_cfg<PLANAR, E, 1, 4, AFF, false>(a, b, p, st);
+  return knn4_launch_cfg<PLANAR, E, 2, 4, AFF, false>(a, b, p, st);
 }
 
 size_t knn4_workspace_bytes(int b, int r, int q, int k) {
@@ -814,8 +793,8 @@ int knn4_planar(const float *x, int b, int n, int k, int64_t *idx, cudaStream_t 
 
 }  // namespace pdae
 
-extern "C" int pdae_tune_knn(int impl, int qw, int nw, int tile, int nz, int tma, int spec) {
-  pdae::Knn4Tune &t = pdae::knn4_tune();
-  t.impl = impl, t.qw = qw, t.nw = nw, t.tile = tile, t.nz = nz, t.tma = tma, t.spec = spec;
+extern "C" int pdae_tune_knn(int form, int tile, int nz, int tma) {
+  if (form < -1 || form >= pdae::KNN4_NFORMS) return PDAE_E_INVALID;
+  pdae::knn4_tune = pdae::Knn4Tune{form, tile, nz, tma};
   return 0;
 }

@@ -1,5 +1,6 @@
 // knn_select.cuh -- warp-level exact top-k selection primitives shared by knn.cu (streaming
-// warp-select, any dimension) and knn3.cu (3-D fast path with a lane-local threshold pre-pass).
+// warp-select, any dimension), knn4.cu (3-D fast path with a segment-minima threshold pre-pass), featknn.cu,
+// patchify.cu and pointops.cu.
 // Keys are (float bits << 32 | index): the unsigned order is the (distance, lower index) order.
 #pragma once
 #include "common.cuh"
@@ -93,36 +94,6 @@ __device__ __forceinline__ void warp_sort_multi(uint64_t (&v)[E], int lane) {
           const bool up = ((e * 32 + lane) & k) == 0;
           const bool keep_min = ((lane & j) == 0) == up;
           v[e] = keep_min ? umin64(v[e], o) : umax64(v[e], o);
-        }
-      }
-    }
-  }
-}
-// same network on fp32 values (used for the threshold pre-pass; ties are irrelevant there)
-template <int E>
-__device__ __forceinline__ void warp_sort_multi_f32(float (&v)[E], int lane) {
-#pragma unroll
-  for (int k = 2; k <= 32 * E; k <<= 1) {
-#pragma unroll
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      if (j >= 32) {
-#pragma unroll
-        for (int e = 0; e < E; ++e) {
-          const int pe = e ^ (j >> 5);
-          if (pe > e) {
-            const bool up = ((e * 32) & k) == 0;
-            const float lo = fminf(v[e], v[pe]), hi = fmaxf(v[e], v[pe]);
-            v[e] = up ? lo : hi;
-            v[pe] = up ? hi : lo;
-          }
-        }
-      } else {
-#pragma unroll
-        for (int e = 0; e < E; ++e) {
-          const float o = __shfl_xor_sync(0xffffffffu, v[e], j);
-          const bool up = ((e * 32 + lane) & k) == 0;
-          const bool keep_min = ((lane & j) == 0) == up;
-          v[e] = keep_min ? fminf(v[e], o) : fmaxf(v[e], o);
         }
       }
     }

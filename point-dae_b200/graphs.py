@@ -26,7 +26,7 @@ class PriorityGraph:
     `low_priority` lists substrings of kernel names that go to the lowest launch priority; every other kernel node
     gets the highest.  Memset / memcpy nodes have no priority."""
 
-    def __init__(self, low_priority=("fps_", "knn3_", "knn_", "gather_")):
+    def __init__(self, low_priority=("fps_", "knn_", "gather_")):
         self.low = tuple(low_priority)
         self.graph = torch.cuda.CUDAGraph(keep_graph=True)
         self.exec = None

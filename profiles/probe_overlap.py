@@ -70,7 +70,7 @@ out = {
     "both_two_streams_us": time_graphs(both),
     "both_one_stream_us": time_graphs(both_serial),
     "loss_then_patch_one_stream_us": time_graphs(loss_then_patch),
-    "both_prio_patch_low_us": time_graphs(both, prio=("fps_", "knn3_")),
+    "both_prio_patch_low_us": time_graphs(both, prio=("fps_", "knn4_")),
     "both_prio_patch_high_us": time_graphs(both, prio=("chamfer", "fill_keys")),
 }
 print(json.dumps(out))

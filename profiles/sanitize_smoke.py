@@ -14,8 +14,8 @@ pointnet2_utils.furthest_point_sample(cu(synth.clouds(1, 20000, seed=3)), 16)   
 pointnet2_utils.furthest_point_sample(cu(synth.clouds(1, 200000, seed=4)), 4)     # global fallback
 idx, cen = group.fps(x, 33)
 ops.group_points_knn(x, cen, 17)
-knn_cuda.KNN(5, True)(y, cen)                       # knn3, k<=32
-knn_cuda.KNN(40, True)(y, cen)                      # knn3, k<=64
+knn_cuda.KNN(5, True)(y, cen)                       # knn4, k<=32
+knn_cuda.KNN(40, True)(y, cen)                      # knn4, k<=64
 knn_cuda.KNN(100, True)(y, cen)                     # streaming warp-select
 knn_cuda.KNN(8, True)(torch.cat([y, y], 2), torch.cat([cen, cen], 2))  # dim 6
 big = cu(synth.clouds(1, 9000, seed=5)); knn_cuda.KNN(16, True)(big, big[:, :50].contiguous())  # multi-tile
@@ -30,7 +30,7 @@ for c in (3, 7, 64):
 bq = pointnet2_utils.ball_query(0.2, 16, y, cen)
 gp = pointnet2_utils.grouping_operation(y.transpose(1, 2).contiguous().requires_grad_(True), bq); gp.sum().backward()
 go = pointnet2_utils.gather_operation(y.transpose(1, 2).contiguous().requires_grad_(True), idx); go.sum().backward()
-# fused loss epilogue + scalar-gradient backward, both recovery kernels, odd query counts (idle warps in knn3)
+# fused loss epilogue + scalar-gradient backward, both recovery kernels, odd query counts (idle warps in knn4)
 from pointdae_b200 import _native, chamfer_dist
 loss3 = ops.chamfer_mean_loss(d[0], d[1], True)
 ops.chamfer_loss_backward(x, y, d[2], d[3], d[0], d[1], torch.ones(1, device=dev), 0.5, 0.5, True)

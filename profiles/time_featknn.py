@@ -1,9 +1,9 @@
-"""DGCNN feature kNN (16 x 2048 points, k = 20) timing: python profiles/time_featknn.py  (PDAE_FEATKNN_FULL=1: round-1 form)"""
+"""DGCNN feature kNN (16 x 2048 points, k = 20) timing: python profiles/time_featknn.py"""
 import json, os, statistics, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from pointdae_b200 import dgcnn_util, synth
-out = {"form": "full matrix (round 1)" if os.environ.get("PDAE_FEATKNN_FULL") else "symmetric"}
+out = {"form": "symmetric"}
 for C in (64, 128):
     x = torch.from_numpy(synth.features(16, C, 2048, seed=C)).to("cuda:0")
     for _ in range(3):

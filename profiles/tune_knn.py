@@ -2,10 +2,10 @@
 
     python profiles/tune_knn.py [--out gpurun_out/r02/tune_knn.json] [--quick]
 
-For every shape: the first-generation kernel (impl 3) is the timing baseline and the bit-exact comparator; the
-second-generation kernel (impl 4) is run over a grid of (queries per warp, warps per CTA, TMA on/off, chunks along the
-reference cloud) through pdae_tune_knn.  Times are CUDA events around replayed CUDA graphs of `reps` launches on the
-launching stream.  Prints one JSON object; `fma_frac` = pairs x 6 lane-ops / time / (148 x 128 x sm clock)."""
+For every shape: the automatic plan (form -1) is the timing baseline and the bit-exact comparator; the kernel is run
+over a grid of (form, TMA on/off, chunks along the reference cloud, tile) through pdae_tune_knn, where form is one of the
+four (queries per warp, warps per CTA, warp-specialised) shapes the plan chooses from.  Times are CUDA events around
+replayed CUDA graphs of `reps` launches on the launching stream.  Prints one JSON object; `fma_frac` = pairs x 6 lane-ops / time / (148 x 128 x sm clock)."""
 import argparse
 import itertools
 import json
@@ -45,8 +45,11 @@ def timed(fn, reps=10, rounds=5):
     return best * 1e3  # us
 
 
-def tune(impl=4, qw=-1, nw=-1, tile=-1, nz=-1, tma=-1, spec=-1):
-    _native.lib().pdae_tune_knn(impl, qw, nw, tile, nz, tma, spec)
+FORMS = {0: "qw4 nw8 spec", 1: "qw4 nw8", 2: "qw4 nw4", 3: "qw2 nw4"}
+
+
+def tune(form=-1, tile=-1, nz=-1, tma=-1):
+    assert _native.lib().pdae_tune_knn(form, tile, nz, tma) == 0
 
 
 def main():
@@ -74,47 +77,42 @@ def main():
             run = lambda: ops.group_points_knn(xyz, center, k, want_idx=True)
         pairs = b * q * r
         rec = {"pairs": pairs, "fma_floor_us": pairs * 6 / PEAK * 1e6, "runs": []}
-        tune(impl=3)
+        tune()
         want = run()
         torch.cuda.synchronize()
-        t3 = timed(run)
-        rec["impl3_us"] = t3
-        rec["impl3_fma_frac"] = pairs * 6 / (t3 * 1e-6) / PEAK
         ntiles = (r + 2047) // 2048
-        grid = [dict(qw=-1, nw=-1, tma=-1, nz=-1, spec=-1, tile=-1)]
+        grid = [dict(form=-1, tma=-1, nz=-1, tile=-1)]
         if not args.quick:
             nzs = [-1] if ntiles == 1 else sorted({1, 2, 3, 4, 6, 8, 12, 16} & set(range(1, ntiles + 1))) + [-1]
-            for qw, nw, tma, nz in itertools.product((1, 2, 4), (4, 8), (0, 1), nzs):
-                if b * q > 20000 and (qw == 1 or (nz not in (-1, 1))):
+            tiles = (1024, 2048) if ntiles > 1 else (2048,)
+            for form, tma, nz, tile in itertools.product(FORMS, (0, 1), nzs, tiles):
+                if b * q > 20000 and nz not in (-1, 1):
                     continue
-                grid.append(dict(qw=qw, nw=nw, tma=tma, nz=nz, spec=0, tile=2048))
-            if ntiles > 1:  # warp-specialised CTAs (7 compute warps + producer)
-                for qw, tma, nz, tile in itertools.product((2, 4), (0, 1), nzs, (1024, 2048)):
-                    if b * q > 20000 and nz not in (-1, 1):
-                        continue
-                    grid.append(dict(qw=qw, nw=8, tma=tma, nz=nz, spec=1, tile=tile))
+                if form == 0 and ntiles == 1:  # the producer warp only pays off on streamed clouds
+                    continue
+                grid.append(dict(form=form, tma=tma, nz=nz, tile=tile))
         for cfg in grid:
-            tune(impl=4, **cfg)
+            tune(**cfg)
             got = run()
             torch.cuda.synchronize()
             same = all((a is None and bb is None) or torch.equal(a, bb) for a, bb in zip(
                 got if isinstance(got, tuple) else (got,), want if isinstance(want, tuple) else (want,)))
             t = timed(run)
-            rec["runs"].append(dict(cfg, us=t, fma_frac=pairs * 6 / (t * 1e-6) / PEAK, same_as_impl3=bool(same)))
+            rec["runs"].append(dict(cfg, us=t, fma_frac=pairs * 6 / (t * 1e-6) / PEAK, same_as_auto=bool(same)))
         tune()
         best = min(rec["runs"], key=lambda x: x["us"])
         rec["best"] = best
         rec["auto"] = rec["runs"][0]
-        print(name, "impl3 %.1f us | auto %.1f us (%s) | best %.1f us %s" % (
-            t3, rec["auto"]["us"], "same" if rec["auto"]["same_as_impl3"] else "DIFFERENT", best["us"],
-            {kk: best[kk] for kk in ("qw", "nw", "tma", "nz", "spec", "tile")}), flush=True)
-        assert all(x["same_as_impl3"] for x in rec["runs"]), [x for x in rec["runs"] if not x["same_as_impl3"]]
+        print(name, "auto %.1f us | best %.1f us %s (%s)" % (
+            rec["auto"]["us"], best["us"], {kk: best[kk] for kk in ("form", "tma", "nz", "tile")},
+            FORMS.get(best["form"], "automatic")), flush=True)
+        assert all(x["same_as_auto"] for x in rec["runs"]), [x for x in rec["runs"] if not x["same_as_auto"]]
         out[name] = rec
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
             json.dump(out, f, indent=1)
-    print(json.dumps({k: {"impl3_us": v["impl3_us"], "auto_us": v["auto"]["us"], "best": v["best"]} for k, v in out.items()}))
+    print(json.dumps({k: {"auto_us": v["auto"]["us"], "best": v["best"]} for k, v in out.items()}))
 
 
 if __name__ == "__main__":

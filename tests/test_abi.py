@@ -73,6 +73,9 @@ def test_argument_validation_needs_no_gpu():
     assert L.pdae_step_f32(None, None, 0, 2048, 64, 32, *([None] * 11), None, 0, None) == 0
     assert L.pdae_step_f32(None, None, 2, 2048, 64, 32, *([None] * 11), None, 0, None) == -1
     assert L.pdae_step_workspace_bytes(128, 2048, 64, 32) % 256 == 0
+    # kNN tuning hook: form -1 (automatic) or 0..3; anything else is rejected
+    assert L.pdae_tune_knn(4, -1, -1, -1) == -1
+    assert L.pdae_tune_knn(-2, -1, -1, -1) == -1
 
 
 def test_source_is_sm100a_only():
