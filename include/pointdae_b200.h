@@ -585,6 +585,34 @@ int pdae_seg_chamfer_loss_bwd_det_f32(const float *xyz1, int n_total, const floa
                                       const float *gloss, int l1, float *gx1, float *gx2, void *workspace,
                                       size_t workspace_bytes, pdae_stream_t stream);
 
+/* ---- Earth Mover's Distance over variable-size clouds in one batch (segment approxmatch, cost, gradient) --------
+ * xyz1 (n_total,3), xyz2 (m_total,3) fp32 packed; offset1 / offset2 (b,) int32 cumulative ends (device).  Segments:
+ * the rule of the segment Chamfer above (end[s] = max(clamp(offset[0..s]))); segment s of xyz1 is matched only against
+ * segment s of xyz2.  Per segment with n_s, m_s >= 1: exactly the arithmetic and orders of pdae_emd_* above at b = 1
+ * (masses from the integer divisions of n_s and m_s, the ten levels with ex2.approx.ftz, the three passes, the cost as a
+ * per-column chain then 256 strided chains and the fixed pairwise tree, the gradient chains with rsqrtf times
+ * grad_cost[s]), indices relative to the segment start.  So every segment's ratios, cost and gradients equal those of
+ * pdae_emd_* on that segment's slices at b = 1, bit for bit, and equal segments give the batched (b,n,3) results.
+ * Ratios: ratio_l (10, n_total), ratio_r (10, m_total), level-major: level j of point p at j * n_total + p (equal
+ * segments: ratio_l viewed (10,b,n) and transposed to (b,10,n) is the equal-size layout).  There is no match output:
+ * cost and gradient rebuild it from the ratios.
+ * A segment with an empty side has cost 0, and every point of it gets ratios 0 and gradient 0; so do the points past
+ * the last segment.  b = 0: return 0 and write nothing.  No per-segment size cap (the equal-size 65536 stays there):
+ * one segment runs on one cluster of at most 8 CTAs, so its time grows with n_s * m_s.  n_total, m_total above
+ * 2^31 / 10 give PDAE_E_UNSUPPORTED.  Each call runs its own pre-pass over the offsets; none synchronises with the host.
+ * No atomics: the results depend on the inputs only, not on the launch shape, the stream or the deterministic flag.
+ * Workspace (all three calls): pdae_seg_emd_workspace_bytes(b, n_total, m_total).                                */
+size_t pdae_seg_emd_workspace_bytes(int b, int n_total, int m_total);
+int pdae_seg_emd_match_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *offset1,
+                           const int *offset2, int b, float *ratio_l, float *ratio_r, void *workspace, size_t workspace_bytes,
+                           pdae_stream_t stream);
+int pdae_seg_emd_cost_f32(const float *xyz1, int n_total, const float *xyz2, int m_total, const int *offset1,
+                          const int *offset2, int b, const float *ratio_l, const float *ratio_r, float *cost, void *workspace,
+                          size_t workspace_bytes, pdae_stream_t stream);
+int pdae_seg_emd_cost_grad_f32(const float *grad_cost, const float *xyz1, int n_total, const float *xyz2, int m_total,
+                               const int *offset1, const int *offset2, int b, const float *ratio_l, const float *ratio_r,
+                               float *grad1, float *grad2, void *workspace, size_t workspace_bytes, pdae_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -128,6 +128,10 @@ SIGNATURES = {
     "pdae_seg_chamfer_loss_bwd_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp]),
     "pdae_seg_chamfer_loss_bwd_det_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _sz,
                                                _vp]),
+    "pdae_seg_emd_workspace_bytes": (_sz, [_i, _i, _i]),
+    "pdae_seg_emd_match_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_emd_cost_f32": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "pdae_seg_emd_cost_grad_f32": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib = None

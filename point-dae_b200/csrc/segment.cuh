@@ -1,4 +1,4 @@
-// segment.cuh -- device helpers shared by the kernels over packed variable-size clouds (pointops.cu, segchamfer.cu).
+// segment.cuh -- device helpers shared by the kernels over packed variable-size clouds (pointops.cu, segchamfer.cu, segemd.cu).
 #pragma once
 #include "common.cuh"
 

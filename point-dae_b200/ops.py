@@ -1584,3 +1584,83 @@ def segment_chamfer_loss_backward(xyz1, xyz2, idx1, idx2, dist1, dist2, state, g
             rc = L.pdae_seg_chamfer_loss_bwd_f32(*args, _stream())
     _native.check(rc, "pdae_seg_chamfer_loss_bwd_f32")
     return [gx1, gx2]
+
+
+# ------------------------------------------------- Earth Mover's Distance over variable-size clouds in one batch
+def _segment_emd_ratios(ratio_l, ratio_r, n, m, dev):
+    for t, nm, cnt in ((ratio_l, "ratio_l", n), (ratio_r, "ratio_r", m)):
+        _require_f32_contig(t, nm)
+        _same_device(dev, **{nm: t})
+        if tuple(t.shape) != (EMD_LEVELS, cnt):
+            raise RuntimeError("%s must have shape (%d, %d)" % (nm, EMD_LEVELS, cnt))
+
+
+def segment_emd_match(xyz1, xyz2, offset1, offset2):
+    """approxmatch of every segment of a packed batch against the same segment of the other: xyz1 (N,3), xyz2 (M,3) f32,
+    offset1 / offset2 (b,) int32 cumulative ends -> (ratio_l (10,N), ratio_r (10,M)), level-major.  Per segment the
+    arithmetic of emd_match at b = 1; points of a segment with an empty side, or past the last segment, get ratios 0.
+    No host synchronisation."""
+    b = _segment_pair(xyz1, xyz2, offset1, offset2, "segment_emd_match")
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    L = _native.lib()
+    with _on(dev):
+        ratio_l = torch.empty((EMD_LEVELS, n), dtype=torch.float32, device=dev)
+        ratio_r = torch.empty((EMD_LEVELS, m), dtype=torch.float32, device=dev)
+        if b == 0:  # no segment: every point is past the last one
+            ratio_l.zero_(), ratio_r.zero_()
+            return ratio_l, ratio_r
+        nbytes = L.pdae_seg_emd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_seg_emd_match_f32(xyz1.data_ptr(), n, xyz2.data_ptr(), m, offset1.data_ptr(), offset2.data_ptr(), b,
+                                      ratio_l.data_ptr(), ratio_r.data_ptr(), ws.data_ptr(), nbytes, _stream())
+    _native.check(rc, "pdae_seg_emd_match_f32")
+    return ratio_l, ratio_r
+
+
+def segment_emd_cost(xyz1, xyz2, offset1, offset2, ratio_l, ratio_r):
+    """matchcost per segment from the ratios of segment_emd_match: -> (b,); 0 for a segment with an empty side."""
+    b = _segment_pair(xyz1, xyz2, offset1, offset2, "segment_emd_cost")
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    _segment_emd_ratios(ratio_l, ratio_r, n, m, dev)
+    L = _native.lib()
+    with _on(dev):
+        cost = torch.empty((b,), dtype=torch.float32, device=dev)
+        if b == 0:
+            return cost
+        nbytes = L.pdae_seg_emd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_seg_emd_cost_f32(xyz1.data_ptr(), n, xyz2.data_ptr(), m, offset1.data_ptr(), offset2.data_ptr(), b,
+                                     ratio_l.data_ptr(), ratio_r.data_ptr(), cost.data_ptr(), ws.data_ptr(), nbytes,
+                                     _stream())
+    _native.check(rc, "pdae_seg_emd_cost_f32")
+    return cost
+
+
+def segment_emd_cost_grad(grad_cost, xyz1, xyz2, offset1, offset2, ratio_l, ratio_r):
+    """gradient of segment_emd_cost with the match held constant: grad_cost (b,) -> (grad1 (N,3), grad2 (M,3)); points of
+    a segment with an empty side, or past the last segment, get 0."""
+    b = _segment_pair(xyz1, xyz2, offset1, offset2, "segment_emd_cost_grad")
+    n, m = xyz1.size(0), xyz2.size(0)
+    dev = xyz1.device
+    _segment_emd_ratios(ratio_l, ratio_r, n, m, dev)
+    _require_cuda(grad_cost, "segment_emd_cost_grad")
+    _require_f32_contig(grad_cost, "grad_cost")
+    _same_device(dev, grad_cost=grad_cost)
+    if grad_cost.numel() != b:
+        raise RuntimeError("grad_cost must hold one value per segment")
+    L = _native.lib()
+    with _on(dev):
+        grad1 = torch.empty((n, 3), dtype=torch.float32, device=dev)
+        grad2 = torch.empty((m, 3), dtype=torch.float32, device=dev)
+        if b == 0:
+            grad1.zero_(), grad2.zero_()
+            return grad1, grad2
+        nbytes = L.pdae_seg_emd_workspace_bytes(b, n, m)
+        ws = _workspace(nbytes, dev)
+        rc = L.pdae_seg_emd_cost_grad_f32(grad_cost.data_ptr(), xyz1.data_ptr(), n, xyz2.data_ptr(), m, offset1.data_ptr(),
+                                          offset2.data_ptr(), b, ratio_l.data_ptr(), ratio_r.data_ptr(), grad1.data_ptr(),
+                                          grad2.data_ptr(), ws.data_ptr(), nbytes, _stream())
+    _native.check(rc, "pdae_seg_emd_cost_grad_f32")
+    return grad1, grad2
